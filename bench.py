@@ -2,6 +2,7 @@
 """Benchmark of the TriNeRFLet reconstruction hot path on B200 (contract: see the task statement / DESIGN.md section 5).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config small|base_light|large] [--scaling weak|strong]
+    python bench.py ... --dump-outputs DIR                              also write the last timed step's results as .npy
     python bench.py --mode render [--max-steps 4096]                    full-frame 800x800 inference, ray-tile sharded
     python bench.py --impl reference ...                                the reference's CPU path on the host cores
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
@@ -56,7 +57,33 @@ def parse():
                     help="N > 1: gradient exchange by this package's peer-memory kernels (multimem / P2P) or by NCCL (bf16 dirty tiles)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying the captured CUDA graph")
     ap.add_argument("--cpu-budget", type=float, default=25.0, help="seconds of CPU work for the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (train: the loss and "
+                         "every parameter gradient; render: image, depth, weights_sum), float32; a gradient larger than its share "
+                         "of 64 MB is written as a sample at fixed seeded positions")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor.  Writes float32 <name>.npy files, at most DUMP_BYTES in all: a tensor with more elements than
+    its share is flattened and sampled at sorted positions drawn from a generator seeded by its size, so that two runs (or two
+    builds) with the same arguments write the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // max(len(arrays), 1)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if a.numel() > cap:
+            idx = np.unique(np.random.default_rng(a.numel()).integers(0, a.numel(), size=cap))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -413,11 +440,13 @@ def run_render(args, cfg):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        render_frame(*devf[args.warmup + i])
+        o = render_frame(*devf[args.warmup + i])
     e1.record()
     barrier()
     if rank == 0:
         clocks.pause()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: o[k] for k in ("image", "depth", "weights_sum")})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -544,7 +573,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        one_step(devb[args.warmup + i])
+        loss = one_step(devb[args.warmup + i])
     e1.record()
     barrier()
     launches = _lib.launch_count - launches0
@@ -552,6 +581,8 @@ def main():
         launches = ts._graph_kernel_count * args.steps + launches
     if rank == 0:
         clocks.pause()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss, **{"grad." + n: p.grad for n, p in net.named_parameters() if p.grad is not None}})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     counts = net.step_counter[:, 0].float().max().reshape(1)     # samples of the (graph-captured) step slot
     if world > 1:

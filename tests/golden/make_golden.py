@@ -26,10 +26,11 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/reconstruction"
-
+from oracle import reference_path, require_reference  # noqa: E402
 from oracle import wavelet as ow  # noqa: E402
 from oracle import field as of  # noqa: E402
+
+REF = reference_path("reconstruction")
 
 
 def _install_stubs():
@@ -61,7 +62,7 @@ def _install_stubs():
 
 def main():
     _install_stubs()
-    sys.path.insert(0, REF)
+    sys.path.insert(0, require_reference(REF))
     from triplaneencoder.triplane_encoder import TriPlaneVolume
     from nerf.network import NeRFNetwork
 

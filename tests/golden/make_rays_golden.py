@@ -22,7 +22,7 @@ from trinerflet_b200 import scene  # noqa: E402
 
 def main():
     make_golden._install_stubs()
-    sys.path.insert(0, make_golden.REF)
+    sys.path.insert(0, make_golden.require_reference(make_golden.REF))
     from nerf.utils import get_rays, shuffle_data, select_batch
 
     out = {}

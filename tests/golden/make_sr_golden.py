@@ -23,7 +23,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
-REF = "/root/reference/super_resolution/threestudio"
+from oracle import reference_path, require_reference  # noqa: E402
+
+REF = reference_path("super_resolution", "threestudio")
 OUT = os.path.join(HERE, "sr_encoder_fp32.npz")
 
 # one parameter set (C = 8 -- the IDWT kernels take multiples of 8 --, R = 32, two wavelet levels: sides 8 -> 16 -> 32), three pairs of (low_res_scale, high_res_scale):
@@ -42,6 +44,7 @@ def reference_available():
 
 def load_reference_module():
     """-> the reference module threestudio.models.triplaneencoder.triplane_encoder, imported from /root/reference."""
+    require_reference(REF)
     from oracle import wavelet as ow
     if "pytorch_wavelets" not in sys.modules:
         pw = types.ModuleType("pytorch_wavelets")

@@ -1,7 +1,8 @@
 """CPU: the tooling queries of the reconstruction encoder -- TriPlaneVolume.get_planes(max_res / max_scale /
 get_all_resolutions) and get_grid_features (reconstruction/triplaneencoder/triplane_encoder.py:364-416, :485-512; callers
 nerf/utils.py:1649 save_triplane and :500) -- over the host build of the kernels, against the oracle restatement
-(oracle/wavelet.build_planes_limited) and, when /root/reference is present, the reference module itself."""
+(oracle/wavelet.build_planes_limited) and, given a checkout of the original project (TRINERFLET_REFERENCE), the reference
+module itself."""
 import contextlib
 import importlib.util
 import io
@@ -13,11 +14,12 @@ import pytest
 import torch
 
 from oracle import field as of
+from oracle import reference_path
 from oracle import wavelet as ow
 from tests import emu_backend
 from tests.util import rel_l2
 
-REF = "/root/reference/reconstruction"
+REF = reference_path("reconstruction")
 KW = dict(number_of_features=8, plane_resolution=64, init_sigma=0.1, lbound=1.5, inner_multi_res_scale=8)   # 8 -> 16 -> 32 -> 64
 
 
@@ -115,7 +117,7 @@ def _reference_class(monkeypatch):
     return mod.TriPlaneVolume
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original project (TRINERFLET_REFERENCE)")
 def test_queries_against_the_reference_module_live(emu, monkeypatch):
     Ref = _reference_class(monkeypatch)
     with contextlib.redirect_stdout(io.StringIO()):

@@ -3,6 +3,8 @@
   (2) the UNMODIFIED reference kernels compiled from /root/reference (oracle/_ref/_raymarching_ref.so), when present.
 Integer results and fp32 sample positions must be bit-exact; composited floats carry the tolerance written below
 (the GPU uses ex2.approx for __expf, the C oracle expf)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -171,6 +173,46 @@ def test_composite_train_fwd_bwd():
         ref.composite_rays_train_backward(gws, gim, sig.detach(), rgb.detach(), deltas, rays, ws_r, im_r, M, N, 1e-4, gs_r, gc_r)
         assert (gc_r - rgb.grad).abs().max().item() <= COMPOSITE_ATOL_REF
         assert ((gs_r - sig.grad).abs().max() / gs_r.abs().max()).item() <= 1e-5
+
+
+def test_kernels_against_reference_kernel_fixture(golden_dir):
+    """The product kernels on the inputs of tests/golden/raymarch_ref.npz against the outputs the reference's own CUDA kernels
+    gave on them: the same bit-exact / COMPOSITE_ATOL_REF checks as the live comparisons above, without the reference build."""
+    from trinerflet_b200 import _lib
+    from trinerflet_b200 import raymarching as rm
+    g = np.load(os.path.join(golden_dir, "raymarch_ref.npz"))
+    dev = torch.device("cuda")
+    ro, rd = torch.from_numpy(g["rays_o"]).to(dev), torch.from_numpy(g["rays_d"]).to(dev)
+    bf, noises = torch.from_numpy(g["bitfield"]).to(dev), torch.from_numpy(g["noises"]).to(dev)
+    N, M, max_steps, dt_gamma = ro.shape[0], int(g["M"]), int(g["max_steps"]), float(g["dt_gamma"])
+    aabb = torch.tensor([-BOUND] * 3 + [BOUND] * 3, device=dev)
+    nears, fars = rm.near_far_from_aabb(ro, rd, aabb, 0.2)
+    assert np.array_equal(nears.cpu().numpy().view(np.uint32), g["nears"].view(np.uint32))
+    assert np.array_equal(fars.cpu().numpy().view(np.uint32), g["fars"].view(np.uint32))
+    lib = _lib.load()
+    xyzs, dirs, deltas = (torch.zeros(M, k, device=dev) for k in (3, 3, 2))
+    rays = torch.empty(N, 3, dtype=torch.int32, device=dev)
+    counter = torch.zeros(2, dtype=torch.int32, device=dev)
+    ws = torch.empty(lib.tnl_march_rays_train_workspace(N), dtype=torch.uint8, device=dev)
+    _lib.call("tnl_march_rays_train", _lib.ptr(ro), _lib.ptr(rd), _lib.ptr(bf), BOUND, dt_gamma, max_steps, N, CAS, H, M,
+              _lib.ptr(nears), _lib.ptr(fars), _lib.ptr(xyzs), _lib.ptr(dirs), _lib.ptr(deltas), _lib.ptr(rays),
+              _lib.ptr(counter), _lib.ptr(noises), _lib.ptr(ws), ws.numel(), _lib.stream())
+    assert np.array_equal(counter.cpu().numpy(), g["counter"])
+    # the reference kernel's slot order is a race: compare per ray, its rows sorted by ray id
+    rr, mine = g["rays"][np.argsort(g["rays"][:, 0])], rays.cpu().numpy()
+    assert np.array_equal(rr[:, 0], mine[:, 0]) and np.array_equal(rr[:, 2], mine[:, 2])
+    xm, lm = xyzs.cpu().numpy(), deltas.cpu().numpy()
+    for n in range(N):
+        a, b, k = rr[n, 1], mine[n, 1], mine[n, 2]
+        assert np.array_equal(g["xyzs"][a:a + k].view(np.uint32), xm[b:b + k].view(np.uint32))
+        assert np.array_equal(g["deltas"][a:a + k].view(np.uint32), lm[b:b + k].view(np.uint32))
+    w, _, img = rm.composite_rays_train(torch.from_numpy(g["sigmas"]).to(dev), torch.from_numpy(g["rgbs"]).to(dev),
+                                        torch.from_numpy(g["deltas"]).to(dev), torch.from_numpy(g["rays"]).to(dev), 1e-4)
+    assert np.abs(w.detach().cpu().numpy() - g["weights_sum"]).max() <= COMPOSITE_ATOL_REF
+    assert np.abs(img.detach().cpu().numpy() - g["image"]).max() <= COMPOSITE_ATOL_REF
+    packed = rm.packbits(torch.from_numpy(g["grid"]).to(dev), float(g["thresh"]))
+    assert np.array_equal(packed.cpu().numpy(), g["packed"])
+    assert np.array_equal(rm.morton3D(torch.from_numpy(g["coords"]).to(dev)).cpu().numpy(), g["morton"])
 
 
 def _hash_field(x):

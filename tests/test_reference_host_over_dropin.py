@@ -1,6 +1,7 @@
 """Boundary proof (SURVEY.md 8b): the REFERENCE's own host code -- reconstruction/nerf/renderer.py (NeRFRenderer.run_cuda
 train + eval branches, update_extra_state, mark_untrained_grid; :257-381, :383-446, :448-542), nerf/network.py (NeRFNetwork)
-and encoding.py (get_encoder) -- imported UNMODIFIED from /root/reference and run over this package's drop-in modules:
+and encoding.py (get_encoder) -- imported UNMODIFIED from a checkout of the original project and run over this package's
+drop-in modules:
 
     import raymarching                                  ->  trinerflet_b200.raymarching       (renderer.py:9)
     from shencoder import SHEncoder                     ->  trinerflet_b200.shencoder         (encoding.py:61)
@@ -8,8 +9,8 @@ and encoding.py (get_encoder) -- imported UNMODIFIED from /root/reference and ru
 
 i.e. the four-import patch of INTEGRATION.md, then compared with trinerflet_b200.NeRFNetwork / NeRFRenderer on the same
 parameters, rays and RNG seed.  The kernels run as their host build (tests/emu): this is a test of the INTERFACE -- names,
-argument order, return conventions, in-place semantics, RNG call order -- not of device code.  Runs only where
-/root/reference exists (this container); the GPU box does not have it."""
+argument order, return conventions, in-place semantics, RNG call order -- not of device code.  Runs only where the
+environment variable TRINERFLET_REFERENCE names such a checkout."""
 import importlib
 import os
 import sys
@@ -20,10 +21,11 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import reference_path
 from tests import emu_backend
 
-REF = "/root/reference/reconstruction"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not present on this machine")
+REF = reference_path("reconstruction")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original project (TRINERFLET_REFERENCE)")
 
 
 @pytest.fixture

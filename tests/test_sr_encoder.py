@@ -103,7 +103,7 @@ def test_constructor_surface_and_rejections():
         enc(torch.rand(4, 3))
 
 
-@pytest.mark.skipif(not G.reference_available(), reason="/root/reference is only present in the build container")
+@pytest.mark.skipif(not G.reference_available(), reason="needs a checkout of the original project (TRINERFLET_REFERENCE)")
 def test_against_the_reference_module_live(emu):
     """the reference's TriPlaneVolume (its configs' shape: low_res_scale 4, high_res_scale 1) and ours from the same state dict,
     through the application's step sequence; then the reverse direction of the checkpoint: our state dict into the reference"""
