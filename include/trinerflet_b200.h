@@ -238,6 +238,16 @@ int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* f
                      uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb,
                      void* g_feat, float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5,
                      tnl_stream_t stream);
+/* tnl_mlp_backward fused with tnl_sample_planes_backward for the training step (64-wide heads, tcgen05 kernels, fp16 feat,
+ * in_dim = 3C with C in {16, 32}): rows are visited in the order perm [M] (tnl_cell_sort, required), and the input gradient,
+ * rounded to fp16 as tnl_mlp_backward stores it, is scattered straight into g_planes [3][R][R][C] (channels-last, accumulated:
+ * the caller zero-fills every texel the points touch) instead of being written to memory.  feat / dirs / g_sigma / g_rgb /
+ * xyz are indexed by point, as for the two separate calls; R, C, inv_bound, fp16_coords, n_valid as for
+ * tnl_sample_planes_backward.  Same results as the two calls up to the order of the fp32 atomic additions. */
+int tnl_mlp_backward_scatter(const tnl_mlp_dims* dims, const void* packed, const void* feat, const float* dirs, uint32_t M,
+                             const int32_t* n_valid, const int32_t* perm, const float* g_sigma, const float* g_rgb,
+                             const float* xyz, uint32_t R, uint32_t C, float inv_bound, int fp16_coords, float* g_planes,
+                             float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream);
 
 /* Diagnostic: ONE tcgen05.mma product D[M x N] = A B^T with fp16 operands given as plain row-major matrices
  * (A: [a_rows][a_cols] = [M][K] if a_mn == 0, [K][M] if a_mn != 0; B likewise with N), staged in the un-swizzled

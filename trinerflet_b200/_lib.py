@@ -58,6 +58,8 @@ SIGNATURES = {
     "tnl_mlp_pack_weights": (_int, [_DP, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_forward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_backward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "tnl_mlp_backward_scatter": (_int, [_DP, _vp, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _u32, _u32, _f32, _int, _vp, _vp, _vp,
+                                        _vp, _vp, _vp, _vp]),
     "tnl_idwt_level_forward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp]),
     "tnl_idwt_level_backward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _f32, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp]),
     "tnl_tiles_zero": (_int, [_vp, _vp, _vp, _u32, _u32, _u32, _u32, _vp]),

@@ -657,6 +657,11 @@ static bool use_tc(const tnl_mlp_dims* d, int feat_fp16) {
     return !legacy && feat_fp16 && mlp_tc_supported(d->in_dim, d->hidden, d->hidden_c);
 }
 
+namespace tnl {
+size_t mlp_tc_packed_offset(const tnl_mlp_dims* d) { return legacy_packed_bytes(d); }
+bool mlp_tc_selected(const tnl_mlp_dims* d) { return dims_supported(d) && use_tc(d, 1); }
+}  // namespace tnl
+
 #define TNL_MLP_DISPATCH(DIMS, CALL)                                                        \
     do {                                                                                    \
         const uint32_t k_ = (DIMS)->in_dim, h_ = (DIMS)->hidden;                            \

@@ -18,6 +18,7 @@
 #include "mlp_math.cuh"
 #include "mlp_tc.cuh"
 #include "mlp_tc_util.cuh"
+#include "sample_coords.cuh"
 #include "umma.cuh"
 #include <stdlib.h>
 
@@ -236,12 +237,30 @@ __device__ __forceinline__ bool m64_row_of_lane(uint32_t warp, uint32_t lane, ui
 
 constexpr int kBwdStages = 10;
 
-template <int K1>
+// SCATTER variant: tile row i is point perm[i] (the cell order of tnl_cell_sort, rows >= *n_valid last), and the input
+// gradient goes straight into the planes instead of into g_feat: the adjoint of the tri-plane gather (k_sample_bwd4 of
+// sample.cu) applied to the fp16-rounded row, so the [M, K1] gradient stream never leaves the SM.
+struct PlaneScatter {
+    const int32_t* perm;
+    const float* xyz;
+    float* g_planes;      // [3][R][R][C] fp32, accumulated
+    int R;
+    float inv_bound;
+    int fp16_coords;
+};
+
+__device__ __forceinline__ void red_add_v4(float* addr, float4 v, float w) {   // (same instruction as sample.cu's scatter)
+    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};\n" ::"l"(addr), "f"(v.x * w), "f"(v.y * w), "f"(v.z * w),
+                 "f"(v.w * w)
+                 : "memory");
+}
+
+template <int K1, bool SCATTER>
 __global__ void __launch_bounds__(544, 1)
 k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
              const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
              __half* __restrict__ g_feat, float* __restrict__ gW1, float* __restrict__ gW2, float* __restrict__ gW3,
-             float* __restrict__ gW4, float* __restrict__ gW5, unsigned long long* __restrict__ dbg) {
+             float* __restrict__ gW4, float* __restrict__ gW5, unsigned long long* __restrict__ dbg, const PlaneScatter sc) {
     using W = TcW<K1>;
     using S = TcBwdSmem<K1>;
     // TMEM columns: chain accumulators of the two warpgroups | dW1 [64 x K1] | dW4 [64 x 64] | dW3 [64 x 32] | dW2^T, dW5^T [64 x 16]
@@ -367,31 +386,36 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             *q = mask8(pack8<false>(a + 8 * kc), *q);                                                                   \
         }                                                                                                               \
     }
-        // first tile's feature row
+        // first tile's feature row; mx = the point it belongs to (row i of the tile sequence is point i, or perm[i])
         uint4 x[XH];
+        uint32_t mx;
         {
             const uint32_t p0 = (2 * blockIdx.x + g) * 128 + t;
-            const uint4* src = reinterpret_cast<const uint4*>(feat + (size_t)p0 * K1) + hf * XH;
+            const bool v0 = my_pairs > 0 && p0 < nvalid;
+            mx = (SCATTER && v0) ? (uint32_t)__ldg(sc.perm + p0) : p0;
+            const uint4* src = reinterpret_cast<const uint4*>(feat + (size_t)mx * K1) + hf * XH;
 #pragma unroll
-            for (int kc = 0; kc < XH; ++kc) x[kc] = (my_pairs > 0 && p0 < nvalid) ? __ldg(src + kc) : make_uint4(0u, 0u, 0u, 0u);
+            for (int kc = 0; kc < XH; ++kc) x[kc] = v0 ? __ldg(src + kc) : make_uint4(0u, 0u, 0u, 0u);
         }
         for (uint32_t it = 0; it < my_pairs; ++it) {
             const uint32_t tile = 2 * (blockIdx.x + it * gridDim.x) + g;
             const uint32_t p = tile * 128 + t;
             const bool v = p < nvalid;
+            const uint32_t m = mx;
 #pragma unroll
             for (int kc = 0; kc < XH; ++kc) *reinterpret_cast<uint4*>(sub + S::X + ((hf * XH + kc) * 128 + t) * 16) = x[kc];
             float d[3] = {0.f, 0.f, 0.f}, gr[3] = {0.f, 0.f, 0.f}, gs = 0.f;
             if (v && hf == 0) {            // (the 16-column stages are half 0's)
 #pragma unroll
-                for (int j = 0; j < 3; ++j) { d[j] = __ldg(dirs + 3 * (size_t)p + j); gr[j] = __ldg(g_rgb + 3 * (size_t)p + j); }
-                gs = __ldg(g_sigma + p);
+                for (int j = 0; j < 3; ++j) { d[j] = __ldg(dirs + 3 * (size_t)m + j); gr[j] = __ldg(g_rgb + 3 * (size_t)m + j); }
+                gs = __ldg(g_sigma + m);
             }
             TNL_HANDOFF();   // stage 0
             {   // prefetch the next tile's feature row; it is consumed at the top of the next iteration
                 const uint32_t pn = (2 * (blockIdx.x + (it + 1) * gridDim.x) + g) * 128 + t;
-                const uint4* src = reinterpret_cast<const uint4*>(feat + (size_t)pn * K1) + hf * XH;
                 const bool vn = (it + 1 < my_pairs) && pn < nvalid;
+                mx = (SCATTER && vn) ? (uint32_t)__ldg(sc.perm + pn) : pn;
+                const uint4* src = reinterpret_cast<const uint4*>(feat + (size_t)mx * K1) + hf * XH;
 #pragma unroll
                 for (int kc = 0; kc < XH; ++kc) x[kc] = vn ? __ldg(src + kc) : make_uint4(0u, 0u, 0u, 0u);
             }
@@ -441,6 +465,11 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             TNL_HANDOFF();   // stage 6
             TNL_EPI_MASK(S::H3);
             TNL_HANDOFF();   // stage 7
+            float pos[3] = {0.f, 0.f, 0.f};   // the point's position, for the scatter after stage 9 (loaded two stages ahead)
+            if (SCATTER && v) {
+#pragma unroll
+                for (int j = 0; j < 3; ++j) pos[j] = __ldg(sc.xyz + 3 * (size_t)m + j);
+            }
             if (hf == 0) {   // dh2: column 0 <- g_sigma * exp(clamp(logit, -15, 15)) (trunc_exp backward), columns 1..15 <- d(geo)
                 float a[16];
                 tmem_load_row<16>(trow, a);
@@ -454,7 +483,49 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             TNL_HANDOFF();   // stage 8
             TNL_EPI_MASK(S::H1);
             TNL_HANDOFF();   // stage 9
-            {
+            if constexpr (SCATTER) {
+                // 1. the row's input gradient, rounded to fp16 as the g_feat store of the unfused path rounds it, and the point's
+                //    projected coordinates go to a staging area in the H3 | H4 tiles: both are dead from here until the next tile's
+                //    stage-2 epilogue, which no thread reaches before all 256 have handed off that tile's stage 0, i.e. finished below
+                constexpr int C = K1 / 3, CH = KH % 16 == 0 ? 16 : 8, RS = 2 * K1 + 16;   // row stride padded: conflict-free stores
+                static_assert(128 * RS + 128 * 12 <= 2 * tile_bytes(128, 64), "staging area exceeds the H3 | H4 tiles");
+                uint8_t* stg = sub + S::H3;
+                float* su = reinterpret_cast<float*>(stg + 128 * RS);
+#pragma unroll
+                for (int j = 0; j < KH / CH; ++j) {
+                    float a[CH];
+                    tmem_load_row<CH>(trow + hf * KH + j * CH, a);
+#pragma unroll
+                    for (int kc = 0; kc < CH / 8; ++kc)
+                        *reinterpret_cast<uint4*>(stg + t * RS + (hf * KH + j * CH + 8 * kc) * 2) = pack8<false>(a + 8 * kc);
+                }
+                if (hf == 0) {
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) su[3 * t + j] = project_coord(pos[j], sc.inv_bound, sc.fp16_coords);
+                }
+                asm volatile("bar.sync %0, 256;" ::"r"(1u + g) : "memory");   // the sub-tile's two warpgroups
+                // 2. the adjoint of the gather with k_sample_bwd4's mapping: thread <-> (point, plane, 4-channel group), so that
+                //    the C / 4 lanes of one (point, plane) add to one contiguous run of texel channels per corner
+                const uint32_t r = hf * 128 + t;
+                const uint32_t nvt = nvalid - tile * 128 < 128u ? nvalid - tile * 128 : 128u;   // valid rows of this tile
+#pragma unroll 4
+                for (int k = 0; k < K1 / 8; ++k) {       // 128 * K1 / 4 tasks over 256 threads
+                    const uint32_t task = k * 256 + r;
+                    const uint32_t q = task % (C / 4), pl = (task / (C / 4)) % 3, pt = task / (3 * C / 4);
+                    if (pt >= nvt) break;
+                    const float4 gq = unpack4h(*reinterpret_cast<const uint2*>(stg + pt * RS + (pl * C + 4 * q) * 2));
+                    if (gq.x == 0.f && gq.y == 0.f && gq.z == 0.f && gq.w == 0.f) continue;   // adding zeros is a no-op
+                    // plane 0 samples (u_x, u_z), plane 1 (u_x, u_y), plane 2 (u_y, u_z): plane_coords of sample_coords.cuh
+                    const float* u = su + 3 * pt;
+                    const Tap tp = make_tap(pl == 2 ? u[1] : u[0], pl == 1 ? u[1] : u[2], sc.R);
+                    float* base = sc.g_planes + (((size_t)pl * sc.R + tp.y0) * sc.R + tp.x0) * C + 4 * q;
+                    const size_t dx = (size_t)C, dy = (size_t)sc.R * C;
+                    red_add_v4(base, gq, tp.nw);
+                    if (tp.x1ok) red_add_v4(base + dx, gq, tp.ne);
+                    if (tp.y1ok) red_add_v4(base + dy, gq, tp.sw);
+                    if (tp.x1ok && tp.y1ok) red_add_v4(base + dy + dx, gq, tp.se);
+                }
+            } else {
                 float a[KH];
                 tmem_load_row<KH>(trow + hf * KH, a);
                 if (g_feat && p < M) {
@@ -685,22 +756,25 @@ void mlp_tc_forward(uint32_t in_dim, uint32_t hidden, const void* wpk, const voi
 // optional device buffer of 64 cycle counters (tnl_mlp_tc_profile); nullptr in normal operation
 static unsigned long long* g_tc_dbg = nullptr;
 
-template <int K1>
+template <int K1, bool SCATTER>
 static void launch_bwd(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
-                       const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, cudaStream_t s) {
+                       const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, const PlaneScatter& sc,
+                       cudaStream_t s) {
     using S = TcBwdSmem<K1>;
-    cudaFuncSetAttribute(k_mlp_tc_bwd<K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
+    cudaFuncSetAttribute(k_mlp_tc_bwd<K1, SCATTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
     const uint32_t blocks = min(ceil_div(M, 256u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
-    k_mlp_tc_bwd<K1><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M, n_valid,
-                                                   g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4, gW5, g_tc_dbg);
+    k_mlp_tc_bwd<K1, SCATTER><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M,
+                                                            n_valid, g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4,
+                                                            gW5, g_tc_dbg, sc);
 }
 
 void mlp_tc_backward(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
                      const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3,
                      float* gW4, float* gW5, cudaStream_t s) {
     if (hidden == 128) { mlp_tc128_backward(in_dim, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s); return; }
-    if (in_dim == 48) launch_bwd<48>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s);
-    else launch_bwd<96>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s);
+    const PlaneScatter none{};
+    if (in_dim == 48) launch_bwd<48, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, s);
+    else launch_bwd<96, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, s);
 }
 
 }  // namespace tnl
@@ -710,6 +784,27 @@ using namespace tnl;
 extern "C" int tnl_mlp_tc_profile(unsigned long long* counters64) {
     g_tc_dbg = counters64;
     return 0;
+}
+
+extern "C" int tnl_mlp_backward_scatter(const tnl_mlp_dims* dims, const void* packed, const void* feat, const float* dirs, uint32_t M,
+                                        const int32_t* n_valid, const int32_t* perm, const float* g_sigma, const float* g_rgb,
+                                        const float* xyz, uint32_t R, uint32_t C, float inv_bound, int fp16_coords, float* g_planes,
+                                        float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream) {
+    if (M == 0) return 0;
+    if (!dims || !mlp_tc_selected(dims) || dims->hidden != 64 || dims->in_dim != 3 * C) {
+        set_error("mlp_backward_scatter: the 64-wide heads on the tcgen05 kernels (in_dim = 3C in {48, 96}, hidden = hidden_color = 64)");
+        return TNL_ERR_UNSUPPORTED;
+    }
+    TNL_ARG_CHECK(packed && feat && dirs && perm && g_sigma && g_rgb && xyz && g_planes && g_W1 && g_W2 && g_W3 && g_W4 && g_W5,
+                  "null pointer");
+    TNL_ARG_CHECK(R >= 2, "R >= 2");
+    TNL_ARG_CHECK(((uintptr_t)feat & 15) == 0 && ((uintptr_t)g_planes & 15) == 0, "feat/g_planes must be 16-byte aligned");
+    const PlaneScatter sc{perm, xyz, g_planes, (int)R, inv_bound, fp16_coords};
+    const uint8_t* wpk = static_cast<const uint8_t*>(packed) + mlp_tc_packed_offset(dims);
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    if (C == 16) launch_bwd<48, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, s);
+    else launch_bwd<96, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, s);
+    return finish_launch("mlp_backward_scatter(tcgen05)");
 }
 
 extern "C" int tnl_umma_bench(int a_rows, int b_rows, int a_mn, int b_mn, int M, int N, int K, int reps, long long* out2,

@@ -45,11 +45,16 @@ __device__ __forceinline__ Tap make_tap(float gx, float gy, int R) {
     return t;
 }
 
-// projected coordinate of point m on world axis a (0 = x, 1 = y, 2 = z)
-__device__ __forceinline__ float axis_coord(const float* __restrict__ xyz, uint32_t m, int a, float inv_bound, int fp16_coords) {
-    float g = __fmul_rn(__ldg(xyz + 3 * (size_t)m + a), inv_bound);
+// projected coordinate of a world coordinate x
+__device__ __forceinline__ float project_coord(float x, float inv_bound, int fp16_coords) {
+    float g = __fmul_rn(x, inv_bound);
     if (fp16_coords) g = __half2float(__float2half_rn(g));  // autocast rounds the projected coordinates to fp16 (triplane_encoder.py:299)
     return g;
+}
+
+// projected coordinate of point m on world axis a (0 = x, 1 = y, 2 = z)
+__device__ __forceinline__ float axis_coord(const float* __restrict__ xyz, uint32_t m, int a, float inv_bound, int fp16_coords) {
+    return project_coord(__ldg(xyz + 3 * (size_t)m + a), inv_bound, fp16_coords);
 }
 
 __device__ __forceinline__ void plane_coords(const float* __restrict__ xyz, uint32_t m, int p, float inv_bound,

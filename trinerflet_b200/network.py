@@ -20,6 +20,7 @@ from ._lib import MlpDims, call, ptr, stream
 from .activation import trunc_exp
 from .encoding import get_encoder
 from .renderer import NeRFRenderer
+from .triplane_encoder import gather_features, take_grad_buffer
 
 
 def fused_dims_supported(in_dim, hidden, hidden_color):
@@ -56,6 +57,19 @@ def _warn_library_path(net, x):
         _warned_library_path = True
 
 
+def _mlp_forward(feat, dirs, n_valid, W):
+    """tnl_mlp_forward -> (sigma, rgb, fp32 contiguous dirs, packed weights, dims)"""
+    dirs = dirs.detach().contiguous().float()
+    M = feat.shape[0]
+    dims = MlpDims(W[0].shape[1], W[0].shape[0], W[3].shape[0])
+    packed = pack_mlp_weights(dims, W)
+    sigma = torch.empty(M, device=feat.device, dtype=torch.float32)
+    rgb = torch.empty(M, 3, device=feat.device, dtype=torch.float32)
+    call("tnl_mlp_forward", ctypes.byref(dims), ptr(packed), ptr(feat), int(feat.dtype == torch.float16), ptr(dirs), M, ptr(n_valid),
+         ptr(sigma), ptr(rgb), None, stream())
+    return sigma, rgb, dirs, packed, dims
+
+
 class _FieldMLP(Function):
     """(feat [M,3C], dirs [M,3]) -> sigma [M] fp32, rgb [M,3] fp32 (fp16-representable values)."""
 
@@ -67,15 +81,7 @@ class _FieldMLP(Function):
             feat = feat.half()          # 128-wide heads: tcgen05 kernels only, fp16 feature stream (the first Linear's own rounding)
         elif feat.dtype != torch.float16:
             feat = feat.float()
-        fh = int(feat.dtype == torch.float16)
-        dirs = dirs.detach().contiguous().float()
-        M = feat.shape[0]
-        dims = MlpDims(W1.shape[1], W1.shape[0], W4.shape[0])
-        packed = pack_mlp_weights(dims, (W1, W2, W3, W4, W5))
-        sigma = torch.empty(M, device=feat.device, dtype=torch.float32)
-        rgb = torch.empty(M, 3, device=feat.device, dtype=torch.float32)
-        call("tnl_mlp_forward", ctypes.byref(dims), ptr(packed), ptr(feat), fh, ptr(dirs), M, ptr(n_valid), ptr(sigma),
-             ptr(rgb), None, stream())
+        sigma, rgb, dirs, packed, dims = _mlp_forward(feat, dirs, n_valid, (W1, W2, W3, W4, W5))
         ctx.save_for_backward(feat, dirs, packed, n_valid if n_valid is not None else torch.empty(0))
         ctx.dims = (dims.in_dim, dims.hidden, dims.hidden_c, n_valid is not None)
         ctx.wshapes = [tuple(w.shape) for w in (W1, W2, W3, W4, W5)]
@@ -97,6 +103,39 @@ class _FieldMLP(Function):
         if g_feat.dtype != ctx.in_dtype:
             g_feat = g_feat.to(ctx.in_dtype)
         return (g_feat, None, None, *gW)
+
+
+class _Field(Function):
+    """The field of a training step on the fused path (fp16 autocast, 64-wide heads, cell-sorted samples): (planes [3,C,R,R],
+    coords [M,3], dirs [M,3], W1..W5) -> sigma [M], rgb [M,3].  The forward makes the two calls of the unfused path (plane gather
+    in cell order into fp16 features, tnl_mlp_forward), so it computes the same bits; the backward is ONE
+    tnl_mlp_backward_scatter, which scatters the feature gradient into the planes from inside the MLP backward instead of
+    writing it out and reading it back.  Same gradient-buffer contract as _SamplePlanes (grad_buf of prefetch_planes)."""
+
+    @staticmethod
+    def forward(ctx, planes, coords, dirs, bound, n_valid, perm, grad_buf, W1, W2, W3, W4, W5):
+        ctx.grad_buf = grad_buf
+        # fp16 coordinates: the path runs under fp16 autocast, which rounds the projected coordinates (sample_planes)
+        feat, coords, ctx.meta = gather_features(planes, coords, bound, True, n_valid, perm, True)
+        sigma, rgb, dirs, packed, dims = _mlp_forward(feat, dirs, n_valid, (W1, W2, W3, W4, W5))
+        ctx.save_for_backward(feat, coords, dirs, packed, n_valid if n_valid is not None else torch.empty(0), perm)
+        ctx.dims = (dims.in_dim, dims.hidden, dims.hidden_c)
+        ctx.wshapes = [tuple(w.shape) for w in (W1, W2, W3, W4, W5)]
+        return sigma, rgb
+
+    @staticmethod
+    def backward(ctx, g_sigma, g_rgb):
+        feat, coords, dirs, packed, n_valid, perm = ctx.saved_tensors
+        M, R, C, inv, fp16_coords, has_nv, _, _ = ctx.meta
+        dims = MlpDims(*ctx.dims)
+        g_planes, external, plane_hook = take_grad_buffer(ctx, C, R, feat.device)
+        assert plane_hook is None, "the plane-by-plane exchange scatters through _SamplePlanes"
+        g_sigma = g_sigma.contiguous().float()
+        g_rgb = g_rgb.contiguous().float()
+        gW = [torch.zeros(s, device=feat.device, dtype=torch.float32) for s in ctx.wshapes]
+        call("tnl_mlp_backward_scatter", ctypes.byref(dims), ptr(packed), ptr(feat), ptr(dirs), M, ptr(n_valid) if has_nv else None,
+             ptr(perm), ptr(g_sigma), ptr(g_rgb), ptr(coords), R, C, inv, fp16_coords, ptr(g_planes), *[ptr(g) for g in gW], stream())
+        return (None if external else g_planes, None, None, None, None, None, None, *gW)
 
 
 class _DensityMLP(Function):
@@ -168,6 +207,12 @@ class NeRFNetwork(NeRFRenderer):
             from .triplane_encoder import cell_sort
             perm = cell_sort(x, self.bound, n_valid, 64)
         fused = self._fused()
+        if (fused and perm is not None and self.hidden_dim == 64 and self.in_dim in (48, 96)
+                and self.encoder.scatter_plane_hook is None):
+            # training step: one fused MLP-backward + plane scatter (the plane-by-plane exchange of the multi-GPU step scatters
+            # through _SamplePlanes instead)
+            planes, gbuf = self.encoder.planes_and_grad_buffer()
+            return _Field.apply(planes, x, d, self.bound, n_valid, perm, gbuf, *self._weights())
         # fused path: the feature stream between the gather and the MLP kernels is fp16 (the first Linear's own rounding)
         feat = self.encoder(x, bound=self.bound, n_valid=n_valid, perm=perm, half_out=fused)
         if fused:

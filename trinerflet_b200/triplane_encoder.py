@@ -250,22 +250,40 @@ def _inv_bound(bound):
     return float(np.float32(1.0) / np.float32(bound))
 
 
+def gather_features(planes, coords, bound, fp16_coords, n_valid, perm, half_out):
+    """The plane gather (tnl_sample_planes_forward) -> (feat [M, 3C], the fp32 contiguous coords it read, meta tuple of the
+    backward: M, R, C, inv_bound, fp16_coords, has n_valid, has perm, half_out)."""
+    _require_cuda_f32(planes, "planes")
+    planes_cl = to_cl_planes(planes.detach())
+    coords = coords.detach().contiguous().float()
+    M = coords.shape[0]
+    C, R = planes.shape[1], planes.shape[2]
+    feat = torch.empty(M, 3 * C, device=planes.device, dtype=torch.float16 if half_out else torch.float32)
+    inv = _inv_bound(bound)
+    call("tnl_sample_planes_forward", ptr(planes_cl), ptr(coords), M, R, C, inv, int(bool(fp16_coords)),
+         ptr(n_valid), ptr(perm), ptr(feat), int(bool(half_out)), stream())
+    return feat, coords, (M, R, C, inv, int(bool(fp16_coords)), n_valid is not None, perm is not None, bool(half_out))
+
+
+def take_grad_buffer(ctx, C, R, device):
+    """-> (g_planes, external, plane_hook): where a sampling backward scatters.  The buffer of ctx.grad_buf (zero-filled ahead of
+    time on the prefetch stream, TriPlaneVolume.prefetch_planes) is taken once, after the current stream waits for it; without
+    one a zero-filled channels-last buffer.  external: the caller owns the buffer and the backward returns no plane gradient."""
+    if ctx.grad_buf is None:
+        return cl_empty_planes(C, R, device=device, zero=True), False, None
+    g_planes, ready, external, plane_hook = ctx.grad_buf
+    ctx.grad_buf = None
+    torch.cuda.current_stream().wait_event(ready)
+    return g_planes, external, plane_hook
+
+
 class _SamplePlanes(Function):
     @staticmethod
     def forward(ctx, planes, coords, bound, fp16_coords, n_valid, perm=None, half_out=False, grad_buf=None):
-        _require_cuda_f32(planes, "planes")
         ctx.grad_buf = grad_buf
-        planes_cl = to_cl_planes(planes.detach())
-        coords = coords.detach().contiguous().float()
-        M = coords.shape[0]
-        C, R = planes.shape[1], planes.shape[2]
-        feat = torch.empty(M, 3 * C, device=planes.device, dtype=torch.float16 if half_out else torch.float32)
-        inv = _inv_bound(bound)
-        call("tnl_sample_planes_forward", ptr(planes_cl), ptr(coords), M, R, C, inv, int(bool(fp16_coords)),
-             ptr(n_valid), ptr(perm), ptr(feat), int(bool(half_out)), stream())
+        feat, coords, ctx.meta = gather_features(planes, coords, bound, fp16_coords, n_valid, perm, half_out)
         ctx.save_for_backward(coords, n_valid if n_valid is not None else torch.empty(0),
                               perm if perm is not None else torch.empty(0))
-        ctx.meta = (M, R, C, inv, int(bool(fp16_coords)), n_valid is not None, perm is not None, bool(half_out))
         return feat
 
     @staticmethod
@@ -273,14 +291,7 @@ class _SamplePlanes(Function):
         coords, n_valid, perm = ctx.saved_tensors
         M, R, C, inv, fp16_coords, has_nv, has_perm, half = ctx.meta
         g_feat = g_feat.contiguous().half() if half else g_feat.contiguous().float()
-        external = False
-        if ctx.grad_buf is not None:     # zero-filled ahead of time on the prefetch stream (TriPlaneVolume.prefetch_planes)
-            g_planes, ready, external, plane_hook = ctx.grad_buf
-            ctx.grad_buf = None
-            torch.cuda.current_stream().wait_event(ready)
-        else:
-            g_planes = cl_empty_planes(C, R, device=g_feat.device, zero=True)
-            plane_hook = None
+        g_planes, external, plane_hook = take_grad_buffer(ctx, C, R, g_feat.device)
         if plane_hook is not None and C in (16, 32, 48):
             # multi-GPU step: plane by plane, so that the caller can start exchanging plane p while plane p + 1 scatters
             for p in range(3):
@@ -564,13 +575,18 @@ class TriPlaneVolume(nn.Module):
         feats = self.sample_from_planes(grid.reshape(-1, 3), plane_features=plane_features)
         return self.lbound, feats.reshape(*shape[:-1], -1), grid
 
-    def forward(self, coordinates, bound, n_valid=None, perm=None, half_out=False):
-        """coordinates [M,3] in [-bound, bound] -> features [M, 3C] (index p*C + c); fp32 as the reference's
-        grid_sample, or fp16 (half_out) for the fused MLP path, which rounds its input to fp16 anyway."""
+    def planes_and_grad_buffer(self):
+        """-> (planes, the gradient buffer of this step's sampling backward or None): what a sampling call of the step needs."""
         planes = self.get_planes()
         gbuf = self._join_prefetch()
         if gbuf is not None and not torch.is_grad_enabled():
             gbuf = None
+        return planes, gbuf
+
+    def forward(self, coordinates, bound, n_valid=None, perm=None, half_out=False):
+        """coordinates [M,3] in [-bound, bound] -> features [M, 3C] (index p*C + c); fp32 as the reference's
+        grid_sample, or fp16 (half_out) for the fused MLP path, which rounds its input to fp16 anyway."""
+        planes, gbuf = self.planes_and_grad_buffer()
         return sample_planes(planes, coordinates, bound, n_valid=n_valid, perm=perm, half_out=half_out, grad_buf=gbuf)
 
     # -- checkpoints: accept reference (NCHW-contiguous) tensors, keep channels-last storage -------------
