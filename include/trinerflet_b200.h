@@ -131,7 +131,7 @@ int tnl_compact_alive_dev(int32_t* ctrl, uint32_t cap, const int32_t* alive, int
 int tnl_sh_encode_forward(const float* inputs, float* outputs, uint32_t B, uint32_t degree, tnl_stream_t stream);
 
 /* ------------------------------------------------------------------ wavelet planes ----------- */
-/* One level of the inverse 2-D DWT (bior6.8, zero mode) exactly as TriPlaneVolume.build_planes chains
+/* One level of the inverse 2-D DWT (bior6.8, zero mode; other wavelets: the *_wavelet calls below) exactly as TriPlaneVolume.build_planes chains
  * it (triplane_encoder.py:379-394):  out = IDWT(pad4(2*x), pad4(yh)),  n -> 2n.
  * x [3][n][n][C], yh [3][3][n][n][C] (yh[.,0]=high-pass along H, [.,1]=along W, [.,2]=both),
  * out [3][2n][2n][C].  C % 8 == 0, n % 8 == 0. */
@@ -171,6 +171,27 @@ int tnl_idwt_level_backward_sparse(const float* g_out, float* g_x, float* g_yh, 
                                    const float* reg_grad, float reg_coef, const int32_t* active, const int32_t* clean,
                                    const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts,
                                    float* abs_sum, tnl_stream_t stream);
+
+/* The four calls above for a chosen wavelet of the reference's pad table (triplane_encoder.py:174-180); the calls without
+ * the suffix are the TNL_WAVELET_BIOR6_8 case.  Same arguments plus `wavelet`; unknown ids return TNL_ERR_INVALID_ARGUMENT.
+ * Every bank has 4*pad = L - 2 (L = filter length), so a padded level maps n -> 2n and the shapes above hold for all of them. */
+#define TNL_WAVELET_BIOR6_8 0 /* pad 4, L = 18 */
+#define TNL_WAVELET_HAAR 1    /* pad 0, L = 2 */
+#define TNL_WAVELET_BIOR2_2 2 /* pad 1, L = 6 */
+#define TNL_WAVELET_BIOR2_6 3 /* pad 3, L = 14 */
+#define TNL_WAVELET_BIOR4_4 4 /* pad 2, L = 10 */
+int tnl_idwt_level_forward_wavelet(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                                   uint32_t wavelet, tnl_stream_t stream);
+int tnl_idwt_level_backward_wavelet(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                                    const float* reg_grad, float reg_coef, uint32_t plane0, uint32_t nplanes, uint32_t wavelet,
+                                    tnl_stream_t stream);
+int tnl_idwt_level_forward_sparse_wavelet(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                                          const int32_t* active, const int32_t* clean, const int32_t* counts, uint32_t max_active,
+                                          uint32_t max_clean, uint32_t parts, uint32_t wavelet, tnl_stream_t stream);
+int tnl_idwt_level_backward_sparse_wavelet(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                                           const float* reg_grad, float reg_coef, const int32_t* active, const int32_t* clean,
+                                           const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts,
+                                           float* abs_sum, uint32_t wavelet, tnl_stream_t stream);
 
 /* Bilinear tri-plane sampling: replaces F.grid_sample(bilinear, border, align_corners=True) +
  * permute/concat of TriPlaneVolume.forward (triplane_encoder.py:314-332, 523-530).

@@ -62,6 +62,11 @@ SIGNATURES = {
                                         _vp, _vp, _vp, _vp]),
     "tnl_idwt_level_forward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp]),
     "tnl_idwt_level_backward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _f32, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp]),
+    "tnl_idwt_level_forward_wavelet": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _u32, _vp]),
+    "tnl_idwt_level_backward_wavelet": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _f32, _u32, _u32, _u32, _vp]),
+    "tnl_idwt_level_forward_sparse_wavelet": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _u32, _vp]),
+    "tnl_idwt_level_backward_sparse_wavelet": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _f32, _vp, _vp, _vp, _u32, _u32, _u32, _vp,
+                                                      _u32, _vp]),
     "tnl_tiles_zero": (_int, [_vp, _vp, _vp, _u32, _u32, _u32, _u32, _vp]),
     "tnl_mlp_tc_profile": (_int, [_vp]),
     "tnl_umma_bench": (_int, [_int] * 8 + [_vp, _vp]),
@@ -129,7 +134,8 @@ def check(rc, what):
 KERNELS_PER_CALL = {"tnl_march_rays_train": 6, "tnl_composite_rays_train_backward": 2, "tnl_compact_alive": 3, "tnl_compact_alive_dev": 3, "tnl_cell_sort": 5,
                     "tnl_mlp_pack_weights": 2}
 # work-list IDWT calls launch one kernel per requested part (position of the `parts` argument from the end)
-_PARTS_ARG = {"tnl_idwt_level_forward_sparse": -2, "tnl_idwt_level_backward_sparse": -3}
+_PARTS_ARG = {"tnl_idwt_level_forward_sparse": -2, "tnl_idwt_level_backward_sparse": -3,
+              "tnl_idwt_level_forward_sparse_wavelet": -3, "tnl_idwt_level_backward_sparse_wavelet": -4}
 launch_count = 0
 _profile = None  # when enabled: name -> list of (start_event, end_event, scalar_args)
 

@@ -1,4 +1,5 @@
-// Inverse 2-D DWT level (bior6.8, zero mode) and its exact adjoint -- sm_100a, channels-last.
+// Inverse 2-D DWT level (zero mode; bior6.8, haar, bior2.2, bior2.6 or bior4.4) and its exact adjoint -- sm_100a,
+// channels-last.  The wavelet is a template parameter of the kernels (idwt_core.cuh: its taps in the 18-tap frame).
 //
 // The reference spends ~7 full-size passes per level (2 F.pad, 6 conv_transpose2d, 3 adds, see
 // triplane_encoder.py:391-394 + pytorch_wavelets sfb1d); here one kernel per level reads each
@@ -22,9 +23,11 @@
 #include "idwt_core.cuh"
 #include <stdlib.h>
 
+#include <type_traits>
+
 namespace tnl {
 
-template <typename Cfg>
+template <typename Cfg, int W>
 __global__ void __launch_bounds__(Cfg::NT, (768 / Cfg::NT) > 0 ? (768 / Cfg::NT) : 1)
 k_idwt_fwd(const float* __restrict__ x, const float* __restrict__ yh, float* __restrict__ out, int n, int C,
            int rows_per_cta, float* __restrict__ abs_sum, const int4* __restrict__ items, const int* __restrict__ n_items) {
@@ -53,9 +56,9 @@ k_idwt_fwd(const float* __restrict__ x, const float* __restrict__ yh, float* __r
         fwd_issue_stage<Cfg>(g, st, stage0 + ((PH + 2) % 3) * Cfg::STAGE, tid);               \
         cp_async_wait<2>();                                                                   \
         float* mid = mid0 + (ss & 1) * Cfg::MID_F;                                            \
-        fwd_phase_a<Cfg, PH>(g, st, stage0 + PH * Cfg::STAGE, mid, tid, ss);                  \
+        fwd_phase_a<Cfg, PH, W>(g, st, stage0 + PH * Cfg::STAGE, mid, tid, ss);               \
         __syncthreads();                                                                      \
-        fwd_phase_b<Cfg>(g, st, mid, out, ss);                                                \
+        fwd_phase_b<Cfg, W>(g, st, mid, out, ss);                                             \
     }
         TNL_STEP(0) TNL_STEP(1) TNL_STEP(2)
 #undef TNL_STEP
@@ -77,7 +80,7 @@ k_idwt_fwd(const float* __restrict__ x, const float* __restrict__ yh, float* __r
     }
 }
 
-template <typename Cfg>
+template <typename Cfg, int W>
 __global__ void __launch_bounds__(Cfg::NT, (768 / Cfg::NT) > 0 ? (768 / Cfg::NT) : 1)
 k_idwt_bwd(const float* __restrict__ gout, float* __restrict__ g_x, float* __restrict__ g_yh, int n, int C,
            int rows_per_cta, const float* __restrict__ yh, const float* __restrict__ reg_grad, float reg_coef, int plane0,
@@ -109,9 +112,9 @@ k_idwt_bwd(const float* __restrict__ gout, float* __restrict__ g_x, float* __res
         bwd_issue_stage<Cfg>(g, st, stage0 + ((PH + 2) % 3) * Cfg::STAGE, tid);               \
         cp_async_wait<2>();                                                                   \
         float* mid = mid0 + (ss & 1) * Cfg::MID_B;                                            \
-        bwd_phase_a<Cfg, PH>(st, stage0 + PH * Cfg::STAGE, mid, tid);                         \
+        bwd_phase_a<Cfg, PH, W>(st, stage0 + PH * Cfg::STAGE, mid, tid);                      \
         __syncthreads();                                                                      \
-        bwd_phase_b<Cfg>(g, mid, g_x, g_yh, tid, ss, yh_reg, reg);                            \
+        bwd_phase_b<Cfg, W>(g, mid, g_x, g_yh, tid, ss, yh_reg, reg);                         \
     }
         TNL_STEP(0) TNL_STEP(1) TNL_STEP(2)
 #undef TNL_STEP
@@ -203,14 +206,14 @@ k_idwt_clean_bwd(const float* __restrict__ yh, float* __restrict__ g_x, float* _
     }
 }
 
-template <typename Cfg>
+template <typename Cfg, int W>
 static int launch_fwd_sparse(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum, const int32_t* active,
                              const int32_t* clean, const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts,
                              cudaStream_t stream) {
     // (per device, cheap: no process-wide "already set" flag -- a process may drive several devices)
-    cudaFuncSetAttribute(k_idwt_fwd<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_F);
+    cudaFuncSetAttribute(k_idwt_fwd<Cfg, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_F);
     if (max_active > 0 && (parts & 1u))
-        k_idwt_fwd<Cfg><<<max_active * (C / Cfg::CG), Cfg::NT, Cfg::SMEM_F, stream>>>(x, yh, out, (int)n, (int)C, 0, abs_sum,
+        k_idwt_fwd<Cfg, W><<<max_active * (C / Cfg::CG), Cfg::NT, Cfg::SMEM_F, stream>>>(x, yh, out, (int)n, (int)C, 0, abs_sum,
                                                                                      reinterpret_cast<const int4*>(active), counts);
     if (abs_sum != nullptr && max_clean > 0 && (parts & 2u))
         k_idwt_clean_fwd<<<min(max_clean, (uint32_t)kNumSM * 8u), 256, 0, stream>>>(yh, (int)n, (int)C, reinterpret_cast<const int4*>(clean),
@@ -218,14 +221,14 @@ static int launch_fwd_sparse(const float* x, const float* yh, float* out, uint32
     return finish_launch("idwt_level_forward_sparse");
 }
 
-template <typename Cfg>
+template <typename Cfg, int W>
 static int launch_bwd_sparse(const float* g, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh, const float* reg_grad,
                              float reg_coef, const int32_t* active, const int32_t* clean, const int32_t* counts, uint32_t max_active,
                              uint32_t max_clean, uint32_t parts, float* abs_sum, cudaStream_t stream) {
     // (per device, cheap: no process-wide "already set" flag -- a process may drive several devices)
-    cudaFuncSetAttribute(k_idwt_bwd<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_B);
+    cudaFuncSetAttribute(k_idwt_bwd<Cfg, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_B);
     if (max_active > 0 && (parts & 1u))
-        k_idwt_bwd<Cfg><<<max_active * (C / Cfg::CG), Cfg::NT, Cfg::SMEM_B, stream>>>(g, g_x, g_yh, (int)n, (int)C, 0, yh, reg_grad, reg_coef,
+        k_idwt_bwd<Cfg, W><<<max_active * (C / Cfg::CG), Cfg::NT, Cfg::SMEM_B, stream>>>(g, g_x, g_yh, (int)n, (int)C, 0, yh, reg_grad, reg_coef,
                                                                                      0, reinterpret_cast<const int4*>(active), counts);
     if (max_clean > 0 && (parts & 2u))
         k_idwt_clean_bwd<<<min(max_clean, (uint32_t)kNumSM * 8u), 256, 0, stream>>>(yh, g_x, g_yh, (int)n, (int)C,
@@ -234,28 +237,41 @@ static int launch_bwd_sparse(const float* g, float* g_x, float* g_yh, uint32_t n
     return finish_launch("idwt_level_backward_sparse");
 }
 
-template <typename Cfg>
+template <typename Cfg, int W>
 static int launch_fwd(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
                       cudaStream_t stream) {
     // (per device, cheap: no process-wide "already set" flag -- a process may drive several devices)
-    cudaFuncSetAttribute(k_idwt_fwd<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_F);
+    cudaFuncSetAttribute(k_idwt_fwd<Cfg, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_F);
     unsigned gx, gy, gz, rows;
     idwt_grid<Cfg>(n, C, kNumSM, gx, gy, gz, rows);
-    k_idwt_fwd<Cfg><<<dim3(gx, gy, gz), Cfg::NT, Cfg::SMEM_F, stream>>>(x, yh, out, (int)n, (int)C, (int)rows, abs_sum, nullptr, nullptr);
+    k_idwt_fwd<Cfg, W><<<dim3(gx, gy, gz), Cfg::NT, Cfg::SMEM_F, stream>>>(x, yh, out, (int)n, (int)C, (int)rows, abs_sum, nullptr, nullptr);
     return finish_launch("idwt_level_forward");
 }
 
-template <typename Cfg>
+template <typename Cfg, int W>
 static int launch_bwd(const float* g, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
                       const float* reg_grad, float reg_coef, uint32_t plane0, uint32_t nplanes, cudaStream_t stream) {
     // (per device, cheap: no process-wide "already set" flag -- a process may drive several devices)
-    cudaFuncSetAttribute(k_idwt_bwd<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_B);
+    cudaFuncSetAttribute(k_idwt_bwd<Cfg, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_B);
     unsigned gx, gy, gz, rows;
     idwt_grid<Cfg>(n, C, kNumSM, gx, gy, gz, rows);
     gz = nplanes;
-    k_idwt_bwd<Cfg><<<dim3(gx, gy, gz), Cfg::NT, Cfg::SMEM_B, stream>>>(g, g_x, g_yh, (int)n, (int)C, (int)rows, yh, reg_grad,
+    k_idwt_bwd<Cfg, W><<<dim3(gx, gy, gz), Cfg::NT, Cfg::SMEM_B, stream>>>(g, g_x, g_yh, (int)n, (int)C, (int)rows, yh, reg_grad,
                                                                         reg_coef, (int)plane0, nullptr, nullptr);
     return finish_launch("idwt_level_backward");
+}
+
+// runtime wavelet id -> the kernels' template argument
+template <typename Fn>
+static int with_wavelet(uint32_t wavelet, Fn&& fn) {
+    switch (wavelet) {
+        case TNL_WAVELET_BIOR6_8: return fn(std::integral_constant<int, TNL_WAVELET_BIOR6_8>());
+        case TNL_WAVELET_HAAR: return fn(std::integral_constant<int, TNL_WAVELET_HAAR>());
+        case TNL_WAVELET_BIOR2_2: return fn(std::integral_constant<int, TNL_WAVELET_BIOR2_2>());
+        case TNL_WAVELET_BIOR2_6: return fn(std::integral_constant<int, TNL_WAVELET_BIOR2_6>());
+        case TNL_WAVELET_BIOR4_4: return fn(std::integral_constant<int, TNL_WAVELET_BIOR4_4>());
+        default: set_error("idwt: unknown wavelet id %u", wavelet); return TNL_ERR_INVALID_ARGUMENT;
+    }
 }
 
 }  // namespace tnl
@@ -264,58 +280,106 @@ using namespace tnl;
 
 extern "C" {
 
-int tnl_idwt_level_forward(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
-                           tnl_stream_t stream) {
+int tnl_idwt_level_forward_wavelet(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                                   uint32_t wavelet, tnl_stream_t stream) {
     TNL_ARG_CHECK(x && yh && out, "null pointer");
     TNL_ARG_CHECK(n >= 8 && n % 8 == 0 && n <= 16384, "n must be a multiple of 8 in [8, 16384]");
     TNL_ARG_CHECK(C >= 8 && C % 8 == 0, "C must be a multiple of 8");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (C % 32 == 0 && getenv("TNL_IDWT_CG32")) return launch_fwd<IdwtCfg<32, 32>>(x, yh, out, n, C, abs_sum, s);
-    if (C % 24 == 0) return launch_fwd<IdwtCfg<24, 32>>(x, yh, out, n, C, abs_sum, s);
-    if (C % 16 == 0) return launch_fwd<IdwtCfg<16, 32>>(x, yh, out, n, C, abs_sum, s);
-    return launch_fwd<IdwtCfg<8, 32>>(x, yh, out, n, C, abs_sum, s);
+    return with_wavelet(wavelet, [&](auto w) {
+        constexpr int W = decltype(w)::value;
+        if (C % 32 == 0 && getenv("TNL_IDWT_CG32")) return launch_fwd<IdwtCfg<32, 32>, W>(x, yh, out, n, C, abs_sum, s);
+        if (C % 24 == 0) return launch_fwd<IdwtCfg<24, 32>, W>(x, yh, out, n, C, abs_sum, s);
+        if (C % 16 == 0) return launch_fwd<IdwtCfg<16, 32>, W>(x, yh, out, n, C, abs_sum, s);
+        return launch_fwd<IdwtCfg<8, 32>, W>(x, yh, out, n, C, abs_sum, s);
+    });
 }
 
-int tnl_idwt_level_backward(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
-                            const float* reg_grad, float reg_coef, uint32_t plane0, uint32_t nplanes, tnl_stream_t stream) {
+int tnl_idwt_level_backward_wavelet(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                                    const float* reg_grad, float reg_coef, uint32_t plane0, uint32_t nplanes, uint32_t wavelet,
+                                    tnl_stream_t stream) {
     TNL_ARG_CHECK(nplanes >= 1 && plane0 + nplanes <= 3, "plane range must lie in [0, 3)");
     TNL_ARG_CHECK(g_out && g_x && g_yh, "null pointer");
     TNL_ARG_CHECK(n >= 8 && n % 8 == 0 && n <= 16384, "n must be a multiple of 8 in [8, 16384]");
     TNL_ARG_CHECK(C >= 8 && C % 8 == 0, "C must be a multiple of 8");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (C % 32 == 0 && getenv("TNL_IDWT_CG32")) return launch_bwd<IdwtCfg<32, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
-    if (C % 24 == 0) return launch_bwd<IdwtCfg<24, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
-    if (C % 16 == 0) return launch_bwd<IdwtCfg<16, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
-    return launch_bwd<IdwtCfg<8, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
+    return with_wavelet(wavelet, [&](auto w) {
+        constexpr int W = decltype(w)::value;
+        if (C % 32 == 0 && getenv("TNL_IDWT_CG32"))
+            return launch_bwd<IdwtCfg<32, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
+        if (C % 24 == 0) return launch_bwd<IdwtCfg<24, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
+        if (C % 16 == 0) return launch_bwd<IdwtCfg<16, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
+        return launch_bwd<IdwtCfg<8, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, s);
+    });
 }
 
-int tnl_idwt_level_forward_sparse(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
-                                  const int32_t* active, const int32_t* clean, const int32_t* counts, uint32_t max_active,
-                                  uint32_t max_clean, uint32_t parts, tnl_stream_t stream) {
+int tnl_idwt_level_forward_sparse_wavelet(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                                          const int32_t* active, const int32_t* clean, const int32_t* counts, uint32_t max_active,
+                                          uint32_t max_clean, uint32_t parts, uint32_t wavelet, tnl_stream_t stream) {
     TNL_ARG_CHECK(x && yh && out && counts, "null pointer");
     TNL_ARG_CHECK(parts >= 1 && parts <= 3, "parts: bit 0 = active blocks, bit 1 = |yh| sum of the clean blocks");
     TNL_ARG_CHECK((max_active == 0 || active) && (max_clean == 0 || clean), "null work list");
     TNL_ARG_CHECK(n >= 16 && n % 16 == 0 && n <= 16384, "work-list mode: n must be a multiple of 16 in [16, 16384]");
     TNL_ARG_CHECK(C >= 8 && C % 8 == 0, "C must be a multiple of 8");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (C % 24 == 0) return launch_fwd_sparse<IdwtCfg<24, 32>>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
-    if (C % 16 == 0) return launch_fwd_sparse<IdwtCfg<16, 32>>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
-    return launch_fwd_sparse<IdwtCfg<8, 32>>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
+    return with_wavelet(wavelet, [&](auto w) {
+        constexpr int W = decltype(w)::value;
+        if (C % 24 == 0)
+            return launch_fwd_sparse<IdwtCfg<24, 32>, W>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
+        if (C % 16 == 0)
+            return launch_fwd_sparse<IdwtCfg<16, 32>, W>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
+        return launch_fwd_sparse<IdwtCfg<8, 32>, W>(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts, s);
+    });
 }
 
-int tnl_idwt_level_backward_sparse(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
-                                   const float* reg_grad, float reg_coef, const int32_t* active, const int32_t* clean,
-                                   const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts, float* abs_sum,
-                                   tnl_stream_t stream) {
+int tnl_idwt_level_backward_sparse_wavelet(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                                           const float* reg_grad, float reg_coef, const int32_t* active, const int32_t* clean,
+                                           const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts,
+                                           float* abs_sum, uint32_t wavelet, tnl_stream_t stream) {
     TNL_ARG_CHECK((g_out || !(parts & 1u)) && g_x && g_yh && counts, "null pointer");
     TNL_ARG_CHECK(parts >= 1 && parts <= 3, "parts: bit 0 = active blocks, bit 1 = clean blocks");
     TNL_ARG_CHECK((max_active == 0 || active) && (max_clean == 0 || clean), "null work list");
     TNL_ARG_CHECK(n >= 16 && n % 16 == 0 && n <= 16384, "work-list mode: n must be a multiple of 16 in [16, 16384]");
     TNL_ARG_CHECK(C >= 8 && C % 8 == 0, "C must be a multiple of 8");
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (C % 24 == 0) return launch_bwd_sparse<IdwtCfg<24, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active, max_clean, parts, abs_sum, s);
-    if (C % 16 == 0) return launch_bwd_sparse<IdwtCfg<16, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active, max_clean, parts, abs_sum, s);
-    return launch_bwd_sparse<IdwtCfg<8, 32>>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active, max_clean, parts, abs_sum, s);
+    return with_wavelet(wavelet, [&](auto w) {
+        constexpr int W = decltype(w)::value;
+        if (C % 24 == 0)
+            return launch_bwd_sparse<IdwtCfg<24, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active,
+                                                         max_clean, parts, abs_sum, s);
+        if (C % 16 == 0)
+            return launch_bwd_sparse<IdwtCfg<16, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active,
+                                                         max_clean, parts, abs_sum, s);
+        return launch_bwd_sparse<IdwtCfg<8, 32>, W>(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active,
+                                                    max_clean, parts, abs_sum, s);
+    });
+}
+
+// the bior6.8 entry points of ABI version 1
+int tnl_idwt_level_forward(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                           tnl_stream_t stream) {
+    return tnl_idwt_level_forward_wavelet(x, yh, out, n, C, abs_sum, TNL_WAVELET_BIOR6_8, stream);
+}
+
+int tnl_idwt_level_backward(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                            const float* reg_grad, float reg_coef, uint32_t plane0, uint32_t nplanes, tnl_stream_t stream) {
+    return tnl_idwt_level_backward_wavelet(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, plane0, nplanes, TNL_WAVELET_BIOR6_8,
+                                           stream);
+}
+
+int tnl_idwt_level_forward_sparse(const float* x, const float* yh, float* out, uint32_t n, uint32_t C, float* abs_sum,
+                                  const int32_t* active, const int32_t* clean, const int32_t* counts, uint32_t max_active,
+                                  uint32_t max_clean, uint32_t parts, tnl_stream_t stream) {
+    return tnl_idwt_level_forward_sparse_wavelet(x, yh, out, n, C, abs_sum, active, clean, counts, max_active, max_clean, parts,
+                                                 TNL_WAVELET_BIOR6_8, stream);
+}
+
+int tnl_idwt_level_backward_sparse(const float* g_out, float* g_x, float* g_yh, uint32_t n, uint32_t C, const float* yh,
+                                   const float* reg_grad, float reg_coef, const int32_t* active, const int32_t* clean,
+                                   const int32_t* counts, uint32_t max_active, uint32_t max_clean, uint32_t parts, float* abs_sum,
+                                   tnl_stream_t stream) {
+    return tnl_idwt_level_backward_sparse_wavelet(g_out, g_x, g_yh, n, C, yh, reg_grad, reg_coef, active, clean, counts, max_active,
+                                                  max_clean, parts, abs_sum, TNL_WAVELET_BIOR6_8, stream);
 }
 
 }  // extern "C"

@@ -8,9 +8,15 @@
 //     yl = 2*x ; pad yl, yh by 4 ; x' = DWTInverse('bior6.8', mode='zero')((yl, [yh]))
 // per axis   y[i] = sum_m lo[m]*g0[i+8-2m] + hi[m]*g1[i+8-2m]   (0 <= i+8-2m < 18, zero outside),
 // H axis first on (2*LL, yh0) and (yh1, yh2), then W axis (pytorch_wavelets SFB2D order).
+// The other wavelets of the reference's pad table (haar, bior2.2, bior2.6, bior4.4: length L, pad (L-2)/4) use the same
+// closed form: their taps sit in the 18-tap frame at G[k + 9 - L/2] = g[k], and padding by 4 with G gives exactly what
+// padding by their own pad with g gives.  Every tap is a compile-time constant, so the zero taps of the shorter banks cost
+// no instruction.
 #pragma once
 #include <math.h>
 #include <stddef.h>
+
+#include "../../include/trinerflet_b200.h"   // TNL_WAVELET_*
 
 #ifdef __CUDACC__
 #define TNL_HD __host__ __device__ __forceinline__
@@ -20,8 +26,15 @@
 
 namespace tnl {
 
+// synthesis taps g0 = rec_lo, g1 = rec_hi of wavelet W (TNL_WAVELET_*) in the 18-tap frame
+template <int W>
+TNL_HD constexpr float rec_lo(int k);
+template <int W>
+TNL_HD constexpr float rec_hi(int k);
+
 // PyWavelets bior6.8 synthesis taps (rec_lo = g0 has 11 non-zero taps, rec_hi = g1 has 17).
-TNL_HD constexpr float rec_lo(int k) {
+template <>
+TNL_HD constexpr float rec_lo<TNL_WAVELET_BIOR6_8>(int k) {
     switch (k) {
         case 3: return 0.014426282505624435f;
         case 4: return 0.014467504896790148f;
@@ -37,7 +50,8 @@ TNL_HD constexpr float rec_lo(int k) {
         default: return 0.0f;
     }
 }
-TNL_HD constexpr float rec_hi(int k) {
+template <>
+TNL_HD constexpr float rec_hi<TNL_WAVELET_BIOR6_8>(int k) {
     switch (k) {
         case 1: return -0.0019088317364812906f;
         case 2: return -0.0019142861290887667f;
@@ -58,6 +72,114 @@ TNL_HD constexpr float rec_hi(int k) {
         case 17: return -0.0019088317364812906f;
         default: return 0.0f;
     }
+}
+
+// PyWavelets haar, bior2.2, bior2.6, bior4.4 (tests/wavelet_oracle.py), placed in the frame
+template <>
+TNL_HD constexpr float rec_lo<TNL_WAVELET_HAAR>(int k) {
+    switch (k) {
+        case 8: return 0.7071067811865476f;
+        case 9: return 0.7071067811865476f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_hi<TNL_WAVELET_HAAR>(int k) {
+    switch (k) {
+        case 8: return 0.7071067811865476f;
+        case 9: return -0.7071067811865476f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_lo<TNL_WAVELET_BIOR2_2>(int k) {
+    switch (k) {
+        case 7: return 0.3535533905932738f;
+        case 8: return 0.7071067811865476f;
+        case 9: return 0.3535533905932738f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_hi<TNL_WAVELET_BIOR2_2>(int k) {
+    switch (k) {
+        case 7: return 0.1767766952966369f;
+        case 8: return 0.3535533905932738f;
+        case 9: return -1.0606601717798214f;
+        case 10: return 0.3535533905932738f;
+        case 11: return 0.1767766952966369f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_lo<TNL_WAVELET_BIOR2_6>(int k) {
+    switch (k) {
+        case 7: return 0.3535533905932738f;
+        case 8: return 0.7071067811865476f;
+        case 9: return 0.3535533905932738f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_hi<TNL_WAVELET_BIOR2_6>(int k) {
+    switch (k) {
+        case 3: return 0.006905339660024878f;
+        case 4: return 0.013810679320049757f;
+        case 5: return -0.046956309688169176f;
+        case 6: return -0.10772329869638811f;
+        case 7: return 0.16987135563661201f;
+        case 8: return 0.4474660099696121f;
+        case 9: return -0.966747552403483f;
+        case 10: return 0.4474660099696121f;
+        case 11: return 0.16987135563661201f;
+        case 12: return -0.10772329869638811f;
+        case 13: return -0.046956309688169176f;
+        case 14: return 0.013810679320049757f;
+        case 15: return 0.006905339660024878f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_lo<TNL_WAVELET_BIOR4_4>(int k) {
+    switch (k) {
+        case 5: return -0.06453888262869706f;
+        case 6: return -0.04068941760916406f;
+        case 7: return 0.41809227322161724f;
+        case 8: return 0.7884856164055829f;
+        case 9: return 0.41809227322161724f;
+        case 10: return -0.04068941760916406f;
+        case 11: return -0.06453888262869706f;
+        default: return 0.0f;
+    }
+}
+template <>
+TNL_HD constexpr float rec_hi<TNL_WAVELET_BIOR4_4>(int k) {
+    switch (k) {
+        case 5: return -0.03782845550726404f;
+        case 6: return -0.023849465019556843f;
+        case 7: return 0.11062440441843718f;
+        case 8: return 0.37740285561283066f;
+        case 9: return -0.8526986790088938f;
+        case 10: return 0.37740285561283066f;
+        case 11: return 0.11062440441843718f;
+        case 12: return -0.023849465019556843f;
+        case 13: return -0.03782845550726404f;
+        default: return 0.0f;
+    }
+}
+
+// W-axis synthesis (fwd_phase_b): does window element i reach a non-zero tap of g1 (HI) or g0 for one of its two output
+// pairs e (tap index d = i - e)?  Elements that reach none are not loaded.
+template <int W, bool HI>
+TNL_HD constexpr bool wsyn_reaches(int i) {
+    for (int e = 0; e < 2; ++e) {
+        const int d = i - e;
+        if (d < 0 || d > 8) continue;
+        const float ge = HI ? rec_hi<W>(16 - 2 * d) : rec_lo<W>(16 - 2 * d);
+        const float go = HI ? rec_hi<W>(17 - 2 * d) : rec_lo<W>(17 - 2 * d);
+        if (ge != 0.f || go != 0.f) return true;
+    }
+    return false;
 }
 
 // async 4-byte global->shared copy with zero fill; the host emulator provides a synchronous version
@@ -230,16 +352,18 @@ TNL_HD void fwd_issue_stage(const IdwtGeom& g, FwdState& st, float* stage, int t
     st.pH2 += Cfg::RA * row_stride;
 }
 
+// The phase functions take the wavelet as their last template argument; it defaults to bior6.8 for the lock-step emulator
+// (tests/emu/idwt_emu.cpp).
 // H-axis synthesis; newest sample at ring slot SLOT:  W[d] = w[(SLOT + 1 + d) % 9], d = 0 (row m-4) .. 8 (row m+4)
 //   even = sum_d W[d] g[16-2d],  odd = sum_d W[d] g[17-2d];  .x = low band pair (2LL, LH), .y = high band pair (HL, HH)
-template <int SLOT>
+template <int SLOT, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void synth_rows(const f2 (&wL)[9], const f2 (&wH)[9], f2& even, f2& odd) {
     f2 e = mk2(0.f, 0.f), o = mk2(0.f, 0.f);
 #pragma unroll
     for (int d = 0; d < 9; ++d) {
         const f2 l = wL[(SLOT + 1 + d) % 9], h = wH[(SLOT + 1 + d) % 9];
-        const float ge0 = rec_lo(16 - 2 * d), go0 = rec_lo(17 - 2 * d);
-        const float ge1 = rec_hi(16 - 2 * d), go1 = rec_hi(17 - 2 * d);
+        const float ge0 = rec_lo<W>(16 - 2 * d), go0 = rec_lo<W>(17 - 2 * d);
+        const float ge1 = rec_hi<W>(16 - 2 * d), go1 = rec_hi<W>(17 - 2 * d);
         if (ge0 != 0.f) e = fma2(ge0, l, e);
         if (go0 != 0.f) o = fma2(go0, l, o);
         if (ge1 != 0.f) e = fma2(ge1, h, e);
@@ -249,7 +373,7 @@ TNL_HD void synth_rows(const f2 (&wL)[9], const f2 (&wH)[9], f2& even, f2& odd) 
     odd = o;
 }
 
-template <int SLOT>
+template <int SLOT, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void fwd_row(FwdState& st, const float* stage, float* mid, int tid, int rr, int NT, int RB, int RS, bool own) {
     const f2* s = reinterpret_cast<const f2*>(stage + ((size_t)rr * NT + tid) * 4);
     f2 l = s[0];                     // (LL, HL)
@@ -259,7 +383,7 @@ TNL_HD void fwd_row(FwdState& st, const float* stage, float* mid, int tid, int r
     st.wL[SLOT] = l;
     st.wH[SLOT] = h;
     f2 e, o;
-    synth_rows<SLOT>(st.wL, st.wH, e, o);
+    synth_rows<SLOT, W>(st.wL, st.wH, e, o);
     mid[(0 * RB + 2 * rr) * RS + tid] = e.x;
     mid[(0 * RB + 2 * rr + 1) * RS + tid] = o.x;
     mid[(1 * RB + 2 * rr) * RS + tid] = e.y;
@@ -267,18 +391,18 @@ TNL_HD void fwd_row(FwdState& st, const float* stage, float* mid, int tid, int r
 }
 
 // phase A of step phase PH (= step index mod 3): RA rows enter the windows at ring slots 3*PH .. 3*PH+2
-template <typename Cfg, int PH>
+template <typename Cfg, int PH, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void fwd_phase_a(const IdwtGeom& g, FwdState& st, const float* stage, float* mid, int tid, int ss) {
     // a coefficient is "owned" by exactly one CTA: its column lies in the strip proper (not the halo) and its row in the chunk
     const bool col_own = g.col >= 4 && g.col < 4 + Cfg::TM;
     const int j0 = g.begin + ss * Cfg::RA;
-    fwd_row<(PH * 3 + 0) % 9>(st, stage, mid, tid, 0, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 0 >= g.row_lo && j0 + 0 < g.row_hi);
-    fwd_row<(PH * 3 + 1) % 9>(st, stage, mid, tid, 1, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 1 >= g.row_lo && j0 + 1 < g.row_hi);
-    fwd_row<(PH * 3 + 2) % 9>(st, stage, mid, tid, 2, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 2 >= g.row_lo && j0 + 2 < g.row_hi);
+    fwd_row<(PH * 3 + 0) % 9, W>(st, stage, mid, tid, 0, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 0 >= g.row_lo && j0 + 0 < g.row_hi);
+    fwd_row<(PH * 3 + 1) % 9, W>(st, stage, mid, tid, 1, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 1 >= g.row_lo && j0 + 1 < g.row_hi);
+    fwd_row<(PH * 3 + 2) % 9, W>(st, stage, mid, tid, 2, Cfg::NT, Cfg::RB, Cfg::RS_F, col_own && j0 + 2 >= g.row_lo && j0 + 2 < g.row_hi);
 }
 
 // phase B: W-axis synthesis. item = (mid row r, strip sb of 4 output columns, channel pair cp)
-template <typename Cfg>
+template <typename Cfg, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void fwd_phase_b(const IdwtGeom& g, const FwdState& st, const float* mid, float* out, int ss) {
     const int r = st.b_r;
     const int m = g.begin + ss * Cfg::RA + (r >> 1) - 4;  // coarse row whose synthesis produced mid row r
@@ -289,15 +413,15 @@ TNL_HD void fwd_phase_b(const IdwtGeom& g, const FwdState& st, const float* mid,
     f2 ev[2] = {mk2(0.f, 0.f), mk2(0.f, 0.f)}, od[2] = {mk2(0.f, 0.f), mk2(0.f, 0.f)};
 #pragma unroll
     for (int i = 0; i < 10; ++i) {
-        const f2 h = mhi[i * (Cfg::CG / 2)];
-        f2 l = mk2(0.f, 0.f);
-        if (i >= 2 && i <= 8) l = mlo[i * (Cfg::CG / 2)];  // rec_lo only has taps at d = 2..7
+        f2 h = mk2(0.f, 0.f), l = mk2(0.f, 0.f);
+        if (wsyn_reaches<W, true>(i)) h = mhi[i * (Cfg::CG / 2)];
+        if (wsyn_reaches<W, false>(i)) l = mlo[i * (Cfg::CG / 2)];
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
             const int d = i - e;
             if (d < 0 || d > 8) continue;
-            const float ge0 = rec_lo(16 - 2 * d), go0 = rec_lo(17 - 2 * d);
-            const float ge1 = rec_hi(16 - 2 * d), go1 = rec_hi(17 - 2 * d);
+            const float ge0 = rec_lo<W>(16 - 2 * d), go0 = rec_lo<W>(17 - 2 * d);
+            const float ge1 = rec_hi<W>(16 - 2 * d), go1 = rec_hi<W>(17 - 2 * d);
             if (ge0 != 0.f) ev[e] = fma2(ge0, l, ev[e]);
             if (go0 != 0.f) od[e] = fma2(go0, l, od[e]);
             if (ge1 != 0.f) ev[e] = fma2(ge1, h, ev[e]);
@@ -365,13 +489,13 @@ TNL_HD void bwd_issue_stage(const IdwtGeom& g, BwdState& st, float* stage, int t
 }
 
 // newest sample (k = 17) at ring slot SLOT;  U[k] = w[(SLOT + 1 + k) % 18];  .x = column Xa, .y = column Xb
-template <int SLOT>
+template <int SLOT, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void analyse(const f2 (&w)[18], f2& a, f2& b) {
     f2 ra = mk2(0.f, 0.f), rb = mk2(0.f, 0.f);
 #pragma unroll
     for (int k = 0; k < 18; ++k) {
         const f2 u = w[(SLOT + 1 + k) % 18];
-        const float g0 = rec_lo(k), g1 = rec_hi(k);
+        const float g0 = rec_lo<W>(k), g1 = rec_hi<W>(k);
         if (g0 != 0.f) ra = fma2(g0, u, ra);
         if (g1 != 0.f) rb = fma2(g1, u, rb);
     }
@@ -379,31 +503,31 @@ TNL_HD void analyse(const f2 (&w)[18], f2& a, f2& b) {
     b = rb;
 }
 
-template <int SLOT>  // SLOT = ring slot of the second (newest) row of the pair; odd
+template <int SLOT, int W = TNL_WAVELET_BIOR6_8>  // SLOT = ring slot of the second (newest) row of the pair; odd
 TNL_HD void bwd_row(BwdState& st, const float* stage, float* mid, int tid, int rr, int NT, int RS) {
     const f2* s = reinterpret_cast<const f2*>(stage);
     st.w[(SLOT + 17) % 18] = s[(size_t)(2 * rr) * NT + tid];
     st.w[SLOT] = s[(size_t)(2 * rr + 1) * NT + tid];
     f2 a, b;
-    analyse<SLOT>(st.w, a, b);
+    analyse<SLOT, W>(st.w, a, b);
     // mid layout [row rr][fine column 0..2*WIN)[CG] of pairs (a, b); this thread owns columns col and col + WIN
     f2* m2 = reinterpret_cast<f2*>(mid);
     m2[(size_t)rr * RS + tid] = mk2(a.x, b.x);
     m2[(size_t)rr * RS + NT + tid] = mk2(a.y, b.y);
 }
 
-template <typename Cfg, int PH>
+template <typename Cfg, int PH, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void bwd_phase_a(BwdState& st, const float* stage, float* mid, int tid) {
-    bwd_row<(2 * (PH * 3 + 0) + 1) % 18>(st, stage, mid, tid, 0, Cfg::NT, Cfg::RS_B);
-    bwd_row<(2 * (PH * 3 + 1) + 1) % 18>(st, stage, mid, tid, 1, Cfg::NT, Cfg::RS_B);
-    bwd_row<(2 * (PH * 3 + 2) + 1) % 18>(st, stage, mid, tid, 2, Cfg::NT, Cfg::RS_B);
+    bwd_row<(2 * (PH * 3 + 0) + 1) % 18, W>(st, stage, mid, tid, 0, Cfg::NT, Cfg::RS_B);
+    bwd_row<(2 * (PH * 3 + 1) + 1) % 18, W>(st, stage, mid, tid, 1, Cfg::NT, Cfg::RS_B);
+    bwd_row<(2 * (PH * 3 + 2) + 1) % 18, W>(st, stage, mid, tid, 2, Cfg::NT, Cfg::RS_B);
 }
 
 TNL_HD float signf_(float v) { return v > 0.f ? 1.f : (v < 0.f ? -1.f : 0.f); }  // torch.sign
 
 // phase B: W-axis adjoint. item = (row r, pair of coarse columns sb, channel cb).
 // yh / reg: optional fused gradient of the wavelet L1 regulariser, g_yh += reg * sign(yh)  (nerf/utils.py:640-655)
-template <typename Cfg>
+template <typename Cfg, int W = TNL_WAVELET_BIOR6_8>
 TNL_HD void bwd_phase_b(const IdwtGeom& g, const float* mid, float* g_x, float* g_yh, int tid, int ss, const float* yh,
                         float reg) {
     const int cb = tid % Cfg::CG;
@@ -436,7 +560,7 @@ TNL_HD void bwd_phase_b(const IdwtGeom& g, const float* mid, float* g_x, float* 
         for (int e = 0; e < 2; ++e) {
             const int k = i - 2 * e;
             if (k < 0 || k > 17) continue;
-            const float g0 = rec_lo(k), g1 = rec_hi(k);
+            const float g0 = rec_lo<W>(k), g1 = rec_hi<W>(k);
             if (g0 != 0.f) lo[e] = fma2(g0, v, lo[e]);
             if (g1 != 0.f) hi[e] = fma2(g1, v, hi[e]);
         }

@@ -24,6 +24,8 @@ import torch.nn.functional as F
 from ._lib import call, ptr, stream
 
 TILE = 32          # top-level tile edge in plane texels == one block of the top level
+# wavelet name -> TNL_WAVELET_* id (include/trinerflet_b200.h)
+WAVELET_IDS = {'bior6.8': 0, 'haar': 1, 'bior2.2': 2, 'bior2.6': 3, 'bior4.4': 4}
 MAX_ACTIVE_RUN = 6  # blocks per active item (96 rows: halo overhead 8/96)
 MAX_CLEAN_RUN = 8
 
@@ -76,6 +78,16 @@ def level_maps(flags, levels):
         if l > 0:
             g = F.max_pool2d(b, kernel_size=2, stride=2)           # its g_x lands in tile k // 2 of the level below
     return [m[0] > 0 for m in fwd], [m[0] > 0 for m in bwd]
+
+
+def idwt_call(name, wave, *args):
+    """Issue the IDWT entry point `name` (tnl_idwt_level_*, arguments ending with the stream) for wavelet `wave`.  bior6.8
+    goes through the entry points without suffix, whose names and argument positions the benchmark's per-kernel
+    attribution reads; the other wavelets through `name`_wavelet, with the wavelet id before the stream."""
+    if wave == 'bior6.8':
+        call(name, *args)
+    else:
+        call(name + "_wavelet", *args[:-1], WAVELET_IDS[wave], args[-1])
 
 
 class IdwtPlan:
@@ -172,11 +184,11 @@ class IdwtPlan:
         return plan.update(flags)
 
     # ---- per-level launches ------------------------------------------------------------------------------------------
-    def forward_level(self, l, x, yh, out, n, abs_sum, parts=3):
+    def forward_level(self, l, x, yh, out, n, abs_sum, parts=3, wave='bior6.8'):
         """parts: 1 = reconstruct the active blocks, 2 = |yh| sum of the clean blocks, 3 = both."""
         s = self.fwd[l]
-        call("tnl_idwt_level_forward_sparse", ptr(x), ptr(yh), ptr(out), n, self.C, ptr(abs_sum), ptr(s["active"]), ptr(s["clean"]),
-             ptr(s["counts"]), s["cap_active"], s["cap_clean"], int(parts), stream())
+        idwt_call("tnl_idwt_level_forward_sparse", wave, ptr(x), ptr(yh), ptr(out), n, self.C, ptr(abs_sum), ptr(s["active"]),
+                  ptr(s["clean"]), ptr(s["counts"]), s["cap_active"], s["cap_clean"], int(parts), stream())
 
     def forward_gap_abs(self, l, yh, n, abs_sum):
         """abs_sum += sum |yh| over the blocks that are active in the backward but not reconstructed by the forward."""
@@ -184,11 +196,11 @@ class IdwtPlan:
         call("tnl_idwt_level_forward_sparse", ptr(yh), ptr(yh), ptr(yh), n, self.C, ptr(abs_sum), ptr(s["active"]), ptr(s["clean"]),
              ptr(s["counts"]), 0, s["cap_clean"], 2, stream())
 
-    def backward_level(self, l, g, g_x, g_yh, n, yh, reg_grad, reg_coef, parts=3, abs_sum=None):
+    def backward_level(self, l, g, g_x, g_yh, n, yh, reg_grad, reg_coef, parts=3, abs_sum=None, wave='bior6.8'):
         """parts: 1 = active blocks only, 2 = clean blocks only (independent of g), 3 = both.
         abs_sum: the clean part adds sum |yh| of its blocks (see defer_clean_abs)."""
         s = self.bwd[l]
-        call("tnl_idwt_level_backward_sparse", ptr(g) if g is not None else None, ptr(g_x), ptr(g_yh), n, self.C,
-             ptr(yh) if yh is not None else None, ptr(reg_grad) if reg_grad is not None else None, float(reg_coef), ptr(s["active"]),
-             ptr(s["clean"]), ptr(s["counts"]), s["cap_active"], s["cap_clean"], int(parts),
-             ptr(abs_sum) if abs_sum is not None else None, stream())
+        idwt_call("tnl_idwt_level_backward_sparse", wave, ptr(g) if g is not None else None, ptr(g_x), ptr(g_yh), n, self.C,
+                  ptr(yh) if yh is not None else None, ptr(reg_grad) if reg_grad is not None else None, float(reg_coef),
+                  ptr(s["active"]), ptr(s["clean"]), ptr(s["counts"]), s["cap_active"], s["cap_clean"], int(parts),
+                  ptr(abs_sum) if abs_sum is not None else None, stream())

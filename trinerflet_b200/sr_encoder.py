@@ -134,6 +134,9 @@ class TriPlaneVolume(_te.TriPlaneVolume):
         if levels > 0 and wavelet_base_resolution != 0:
             # :141 / :309 stop cropping the analysis / padding the synthesis below this side; no reference config sets it with levels
             raise NotImplementedError("trinerflet_b200.sr_encoder.TriPlaneVolume: wavelet_base_resolution != 0 with wavelet levels")
+        if levels > 0 and wavelet_type != 'bior6.8':
+            # the super-resolution readings keep the reference configuration's bior6.8
+            raise NotImplementedError(f"trinerflet_b200.sr_encoder.TriPlaneVolume: wavelet_type={wavelet_type} with wavelet levels")
         if low_res_scale < high_res_scale:
             raise AssertionError("low_res_scale >= high_res_scale")                     # :73
         if planes_features is None and init_fn is not None and levels == 0:      # :91-96: only the plain planes use init_fn
@@ -148,7 +151,7 @@ class TriPlaneVolume(_te.TriPlaneVolume):
                          # without levels the wavelet is never applied (KPlaneVolume passes 'haar'); any name will do
                          wavelet_type=wavelet_type if levels > 0 else 'bior6.8', wavelet_base_resolution=0)
         self.wavelet_type = wavelet_type
-        self.planes_features_wavelet_pad = {'bior6.8': 4, 'bior2.6': 3, 'bior4.4': 2, 'bior2.2': 1, 'haar': 0}.get(wavelet_type, 0)
+        self.planes_features_wavelet_pad = _te.PAD_DICT.get(wavelet_type, 0)
         self.wavelet_base_resolution = wavelet_base_resolution
         self.input_pts_in_unit_cube = input_pts_in_unit_cube
         self.n_output_dims = 3 * number_of_features

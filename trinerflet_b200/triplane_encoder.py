@@ -1,6 +1,6 @@
 """TriPlaneVolume -- drop-in for reconstruction/triplaneencoder/triplane_encoder.py:26-530 on the path every
-README command uses (wavelet-parameterised planes, bior6.8, all levels learnable, no rotation / dropout /
-auto-scale / upscale).  Same constructor kwargs, attributes, method names and state-dict keys:
+README command uses (wavelet-parameterised planes, all levels learnable, no rotation / dropout / auto-scale / upscale),
+with every wavelet of the reference's pad table (bior6.8, the README's choice, and bior2.6, bior4.4, bior2.2, haar).  Same constructor kwargs, attributes, method names and state-dict keys:
 
     planes_features                    logical [3, C, n0, n0]
     planes_features_wavelet_coefs.{l}  logical [3, C, 3, n0*2^l, n0*2^l]
@@ -24,8 +24,9 @@ import torch.nn as nn
 from torch.autograd import Function
 
 from ._lib import call, ptr, stream
+from .idwt_plan import idwt_call
 
-PAD_DICT = {'bior6.8': 4}  # triplane_encoder.py:174-180; only bior6.8 is used by the reference's configs
+PAD_DICT = {'bior6.8': 4, 'bior2.6': 3, 'bior4.4': 2, 'bior2.2': 1, 'haar': 0}  # triplane_encoder.py:174-180
 
 
 def get_levels(upscale_factor):
@@ -86,13 +87,13 @@ def _require_cuda_f32(t, what):
 # multilevel inverse DWT  (build_planes, triplane_encoder.py:364-405)
 # ----------------------------------------------------------------------------------------------
 class _BuildPlanes(Function):
-    """planes = IDWT_L(...IDWT_1(2*x0, yh_0)..., yh_{L-1}) with zero padding 4 per level, plus abs_sums[l] = sum|yh_l|
+    """planes = IDWT_L(...IDWT_1(2*x0, yh_0)..., yh_{L-1}) with the wavelet's zero padding per level, plus abs_sums[l] = sum|yh_l|
     (the forward value of the wavelet L1 regulariser, a free by-product of the pass that reads yh).  Linear in all
     inputs, so backward needs no saved activations: it is the chain of adjoint level kernels, with the regulariser
     gradient  g_abs[l] * sign(yh_l)  folded into the coefficient-gradient store."""
 
     @staticmethod
-    def forward(ctx, planes_features, plan, *coefs):
+    def forward(ctx, planes_features, plan, wave, *coefs):
         """plan: None = dense (reference semantics); an idwt_plan.IdwtPlan = reconstruct only the blocks the training-step
         sampler reads (the rest of the returned planes is undefined) and restrict the adjoint to where gradient arrives."""
         _require_cuda_f32(planes_features, "planes_features")
@@ -101,7 +102,7 @@ class _BuildPlanes(Function):
         ctx.n0, ctx.C, ctx.levels = n, C, len(coefs)
         if plan is not None and (plan.levels != len(coefs) or plan.n0 != n or plan.C != C):
             raise RuntimeError("IdwtPlan does not match the encoder geometry")
-        ctx.plan = plan
+        ctx.plan, ctx.wave = plan, wave
         ctx.set_materialize_grads(False)   # an unused abs_sums output must not cost a pass over the coefficients
         abs_sums = torch.zeros(max(len(coefs), 1), device=x.device, dtype=torch.float32)
         saved = []
@@ -113,9 +114,9 @@ class _BuildPlanes(Function):
             saved.append(yh)
             out = cl_empty_planes(C, 2 * n, device=x.device)
             if plan is None:
-                call("tnl_idwt_level_forward", ptr(x), ptr(yh), ptr(out), n, C, ptr(abs_sums[l:l + 1]), stream())
+                idwt_call("tnl_idwt_level_forward", wave, ptr(x), ptr(yh), ptr(out), n, C, ptr(abs_sums[l:l + 1]), stream())
             else:
-                plan.forward_level(l, x, yh, out, n, abs_sums[l:l + 1], parts=1)
+                plan.forward_level(l, x, yh, out, n, abs_sums[l:l + 1], parts=1, wave=wave)
             x, n = out, 2 * n
         if plan is not None:
             if plan.on_planes_ready is not None and plan.defer_clean_abs:
@@ -126,7 +127,7 @@ class _BuildPlanes(Function):
                 if plan.defer_clean_abs:             # ... except those the backward's clean part will read anyway
                     plan.forward_gap_abs(l, yh, n, abs_sums[l:l + 1])
                 else:
-                    plan.forward_level(l, saved[l], yh, saved[l], n, abs_sums[l:l + 1], parts=2)   # x / out are not touched
+                    plan.forward_level(l, saved[l], yh, saved[l], n, abs_sums[l:l + 1], parts=2, wave=wave)   # x / out untouched
                 n *= 2
         ctx.save_for_backward(*saved)
         return x, abs_sums
@@ -148,17 +149,17 @@ class _BuildPlanes(Function):
             g_yh = cl_empty_coefs(C, n, device=g.device)
             if ctx.plan is not None:
                 if g_abs is not None:
-                    ctx.plan.backward_level(l, g, g_x, g_yh, n, yhs[l], g_abs[l:l + 1], 1.0)
+                    ctx.plan.backward_level(l, g, g_x, g_yh, n, yhs[l], g_abs[l:l + 1], 1.0, wave=ctx.wave)
                 else:
-                    ctx.plan.backward_level(l, g, g_x, g_yh, n, None, None, 0.0)
+                    ctx.plan.backward_level(l, g, g_x, g_yh, n, None, None, 0.0, wave=ctx.wave)
             elif g_abs is not None:
-                call("tnl_idwt_level_backward", ptr(g), ptr(g_x), ptr(g_yh), n, C, ptr(yhs[l]), ptr(g_abs[l:l + 1]), 1.0,
-                     0, 3, stream())
+                idwt_call("tnl_idwt_level_backward", ctx.wave, ptr(g), ptr(g_x), ptr(g_yh), n, C, ptr(yhs[l]), ptr(g_abs[l:l + 1]),
+                          1.0, 0, 3, stream())
             else:
-                call("tnl_idwt_level_backward", ptr(g), ptr(g_x), ptr(g_yh), n, C, None, None, 0.0, 0, 3, stream())
+                idwt_call("tnl_idwt_level_backward", ctx.wave, ptr(g), ptr(g_x), ptr(g_yh), n, C, None, None, 0.0, 0, 3, stream())
             grads.append(g_yh)
             g = g_x
-        return (g, None, *reversed(grads))
+        return (g, None, None, *reversed(grads))
 
 
 class PlanewiseIdwtBackward:
@@ -182,8 +183,9 @@ class PlanewiseIdwtBackward:
             n = self.n0 * 2 ** l
             yh = self.enc.planes_features_wavelet_coefs[l]
             use_reg = self.reg_scale is not None and self.reg_coef != 0.0
-            call("tnl_idwt_level_backward", ptr(g), ptr(self.g_x[l]), ptr(self.g_yh[l]), n, self.C,
-                 ptr(yh.detach()) if use_reg else None, ptr(self.reg_scale) if use_reg else None, self.reg_coef, plane, 1, stream())
+            idwt_call("tnl_idwt_level_backward", self.enc.wavelet_type, ptr(g), ptr(self.g_x[l]), ptr(self.g_yh[l]), n, self.C,
+                      ptr(yh.detach()) if use_reg else None, ptr(self.reg_scale) if use_reg else None, self.reg_coef, plane, 1,
+                      stream())
             g = self.g_x[l]
 
     def assign(self):
@@ -214,7 +216,7 @@ class SplitIdwtBackward:
         yh = self.enc.planes_features_wavelet_coefs[l].detach()
         abs_sum = self.abs_sums[l:l + 1] if (self.abs_sums is not None and (parts & 2)) else None
         self.plan.backward_level(l, g, self.g_x[l], self.g_yh[l], self.n0 * 2 ** l, yh if use_reg else None,
-                                 self.reg_scale if use_reg else None, self.reg_coef, parts, abs_sum)
+                                 self.reg_scale if use_reg else None, self.reg_coef, parts, abs_sum, wave=self.enc.wavelet_type)
 
     def run_clean(self):
         for l in range(self.levels):
@@ -233,13 +235,13 @@ class SplitIdwtBackward:
             p.grad = g
 
 
-def build_planes_with_abs(planes_features, coefs, plan=None):
+def build_planes_with_abs(planes_features, coefs, plan=None, wave='bior6.8'):
     """-> (planes [3,C,R,R], abs_sums [L] with abs_sums[l] = sum |coefs[l]|), both differentiable."""
-    return _BuildPlanes.apply(planes_features, plan, *coefs)
+    return _BuildPlanes.apply(planes_features, plan, wave, *coefs)
 
 
-def build_planes(planes_features, coefs, plan=None):
-    return _BuildPlanes.apply(planes_features, plan, *coefs)[0]
+def build_planes(planes_features, coefs, plan=None, wave='bior6.8'):
+    return _BuildPlanes.apply(planes_features, plan, wave, *coefs)[0]
 
 
 # ----------------------------------------------------------------------------------------------
@@ -492,7 +494,7 @@ class TriPlaneVolume(nn.Module):
         coefs = list(self.planes_features_wavelet_coefs) if coefs is None else coefs
         if self.inner_wavelet_scale <= 1 or len(coefs) == 0:
             return planes_features
-        planes, abs_sums = build_planes_with_abs(planes_features, coefs, self.idwt_plan)
+        planes, abs_sums = build_planes_with_abs(planes_features, coefs, self.idwt_plan, self.wavelet_type)
         self._last_abs_sums = abs_sums
         return planes
 
@@ -520,7 +522,7 @@ class TriPlaneVolume(nn.Module):
                     all_res.append(x)
                 if (max_res > 0 and min(x.shape[2:]) >= max_res) or (max_scale > 0 and scale >= max_scale):
                     break
-                x = build_planes(x, [yh])
+                x = build_planes(x, [yh], wave=self.wavelet_type)
                 scale *= 2
             if get_all_resolutions:
                 all_res.append(x)
