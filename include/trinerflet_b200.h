@@ -129,6 +129,11 @@ int tnl_compact_alive_dev(int32_t* ctrl, uint32_t cap, const int32_t* alive, int
 /* ------------------------------------------------------------------ SH direction encoder ----- */
 /* replaces sh_encode_forward (shencoder.h:9, shencoder.cu:387-398) for degree <= 4, dy_dx = NULL */
 int tnl_sh_encode_forward(const float* inputs, float* outputs, uint32_t B, uint32_t degree, tnl_stream_t stream);
+/* replaces sh_encode_backward (shencoder.h:10, shencoder.cu kernel_sh_backward): grad_inputs [B][3] (fp32, overwritten) =
+ * sum_ch grad[b][ch] d(outputs[b][ch]) / d(inputs[b]), the analytic Jacobian of tnl_sh_encode_forward's polynomials summed in
+ * channel order.  grad [B][degree^2].  degree outside 1..4 returns TNL_ERR_INVALID_ARGUMENT. */
+int tnl_sh_encode_backward(const float* grad, const float* inputs, uint32_t B, uint32_t degree, float* grad_inputs,
+                           tnl_stream_t stream);
 
 /* ------------------------------------------------------------------ wavelet planes ----------- */
 /* One level of the inverse 2-D DWT (bior6.8, zero mode; other wavelets: the *_wavelet calls below) exactly as TriPlaneVolume.build_planes chains
@@ -223,6 +228,14 @@ int tnl_sample_planes_backward_plane(const void* g_feat, int feat_fp16, const fl
  * require grad (analytic normals, super_resolution/threestudio/models/geometry/implicit_volume.py:218-226). */
 int tnl_sample_planes_backward_coords(const float* g_feat, const float* planes, const float* xyz, uint32_t M, uint32_t R,
                                       uint32_t C, float inv_bound, int fp16_coords, float* g_xyz, tnl_stream_t stream);
+/* Position gradient of the NeRF field's plane gather (TriPlaneVolume.forward with coordinates that require grad):
+ * g_xyz [M][3] fp32 (every row written; rows >= *n_valid get 0) from g_feat [M][3C] (fp16 if feat_fp16, else fp32), with the
+ * n_valid / perm conventions of tnl_sample_planes_backward.  fp16_coords reproduces the reference's fp16-autocast backward:
+ * each plane's grid gradient is rounded to fp16, the per-axis sum of the two planes that read an axis is rounded to fp16 again,
+ * and only then scaled by inv_bound.  planes [3][R][R][C] channels-last, as tnl_sample_planes_forward reads them. */
+int tnl_sample_planes_backward_xyz(const void* g_feat, int feat_fp16, const float* planes, const float* xyz, uint32_t M, uint32_t R,
+                                   uint32_t C, float inv_bound, int fp16_coords, const int32_t* n_valid, const int32_t* perm,
+                                   float* g_xyz, tnl_stream_t stream);
 
 /* Spatial binning of sample points: perm[i] = row of the i-th point in the order of a G^3 Morton grid over
  * [-bound, bound]^3 (rows >= *n_valid last).  Kernels taking `perm` visit points in that order, which makes the
@@ -269,6 +282,14 @@ int tnl_mlp_backward_scatter(const tnl_mlp_dims* dims, const void* packed, const
                              const int32_t* n_valid, const int32_t* perm, const float* g_sigma, const float* g_rgb,
                              const float* xyz, uint32_t R, uint32_t C, float inv_bound, int fp16_coords, float* g_planes,
                              float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream);
+/* tnl_mlp_backward plus the gradient with respect to the view directions: g_dirs [M][3] fp32 (every row written; rows >=
+ * *n_valid get 0).  d(in3) = dh3 W3 is taken over all 32 columns; its SH part is rounded to fp16 (the autocast linear backward),
+ * and the degree-4 SH Jacobian at dirs is applied as tnl_sh_encode_backward does.  Same dims and feature streams as
+ * tnl_mlp_backward; g_feat and the weight gradients are the same. */
+int tnl_mlp_backward_dirs(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
+                          uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb,
+                          void* g_feat, float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, float* g_dirs,
+                          tnl_stream_t stream);
 
 /* Diagnostic: ONE tcgen05.mma product D[M x N] = A B^T with fp16 operands given as plain row-major matrices
  * (A: [a_rows][a_cols] = [M][K] if a_mn == 0, [K][M] if a_mn != 0; B likewise with N), staged in the un-swizzled

@@ -46,18 +46,21 @@ SIGNATURES = {
     "tnl_composite_rays_dev": (_int, [_vp, _u32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tnl_compact_alive_dev": (_int, [_vp, _u32, _vp, _vp, _vp, _sz, _vp]),
     "tnl_sh_encode_forward": (_int, [_vp, _vp, _u32, _u32, _vp]),
+    "tnl_sh_encode_backward": (_int, [_vp, _vp, _u32, _u32, _vp, _vp]),
     "tnl_idwt_level_forward": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "tnl_idwt_level_backward": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _f32, _u32, _u32, _vp]),
     "tnl_sample_planes_forward": (_int, [_vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _int, _vp]),
     "tnl_sample_planes_backward": (_int, [_vp, _int, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _vp]),
     "tnl_sample_planes_backward_plane": (_int, [_vp, _int, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _u32, _vp]),
     "tnl_sample_planes_backward_coords": (_int, [_vp, _vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp]),
+    "tnl_sample_planes_backward_xyz": (_int, [_vp, _int, _vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _vp]),
     "tnl_cell_sort_workspace": (_sz, [_u32, _u32]),
     "tnl_cell_sort": (_int, [_vp, _u32, _vp, _f32, _u32, _vp, _vp, _sz, _vp]),
     "tnl_mlp_packed_bytes": (_sz, [_DP]),
     "tnl_mlp_pack_weights": (_int, [_DP, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_forward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_backward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "tnl_mlp_backward_dirs": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_backward_scatter": (_int, [_DP, _vp, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _u32, _u32, _f32, _int, _vp, _vp, _vp,
                                         _vp, _vp, _vp, _vp]),
     "tnl_idwt_level_forward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp]),

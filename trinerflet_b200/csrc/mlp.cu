@@ -423,12 +423,13 @@ __device__ __forceinline__ void relu_mask(uint32_t (&d)[KS][4], const uint32_t (
         }
 }
 
-template <int K1, int H, int HC, int NW, bool FH>
+// DIRS: also g_dirs [M,3] <- the SH Jacobian applied to the fp16-rounded SH columns of d(in2) (valid rows only)
+template <int K1, int H, int HC, int NW, bool FH, bool DIRS>
 __global__ void __launch_bounds__(NW * 32, NW == 4 ? 2 : 1)
 k_mlp_bwd(const uint32_t* __restrict__ wp, const void* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
           const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
           void* __restrict__ g_feat, float* __restrict__ gW1, float* __restrict__ gW2, float* __restrict__ gW3,
-          float* __restrict__ gW4, float* __restrict__ gW5) {
+          float* __restrict__ gW4, float* __restrict__ gW5, float* __restrict__ g_dirs) {
     static_assert(H == 64 && HC == 64, "backward kernel: weight-gradient register tiling is laid out for 64-wide heads");
     static_assert(NW == 4 || NW == 8, "4 or 8 warps");
     constexpr MlpLayout L = make_layout(K1, H, HC);
@@ -522,11 +523,34 @@ k_mlp_bwd(const uint32_t* __restrict__ wp, const void* __restrict__ feat, const 
             }
         }
         store_frags<HC / 16>(sm + SM::O_D3, SM::P_C, row0, d3, t);
-        // d(in2) = dh3 W3 ; only the geo half (internal columns 16..31) is needed
+        // d(in2) = dh3 W3 ; the geo half (internal columns 16..31) feeds dh2, the SH half (columns 0..15) only g_dirs
         uint32_t d2[1][4];
         {
             float acc[4][4];
             layer_mma<HC / 16, 4>(acc, d3, wp, L.B3, lane);
+            if constexpr (DIRS) {
+                // gather the point's 16 SH columns from the four lanes of its quad (row g: elements 0, 1; row g + 8: 2, 3),
+                // rounded to fp16 as the autocast linear backward returns them; lane t = 0 finishes row r0, t = 1 row r1
+                float sh0[16], sh1[16];
+#pragma unroll
+                for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+                    for (int tt = 0; tt < 4; ++tt) {
+                        const int src = (lane & ~3) | tt;
+                        sh0[nt * 8 + 2 * tt] = r16(__shfl_sync(0xffffffffu, acc[nt][0], src));
+                        sh0[nt * 8 + 2 * tt + 1] = r16(__shfl_sync(0xffffffffu, acc[nt][1], src));
+                        sh1[nt * 8 + 2 * tt] = r16(__shfl_sync(0xffffffffu, acc[nt][2], src));
+                        sh1[nt * 8 + 2 * tt + 1] = r16(__shfl_sync(0xffffffffu, acc[nt][3], src));
+                    }
+                const uint32_t r = t == 0 ? r0 : r1;
+                if (t < 2 && (t == 0 ? v0 : v1)) {
+                    float gd[3];
+                    sh_backward<16>(__ldg(dirs + 3 * (size_t)r), __ldg(dirs + 3 * (size_t)r + 1), __ldg(dirs + 3 * (size_t)r + 2),
+                                    t == 0 ? sh0 : sh1, gd);
+#pragma unroll
+                    for (int a = 0; a < 3; ++a) g_dirs[3 * (size_t)r + a] = gd[a];
+                }
+            }
             // dh2 tiles 0,1 <- d(in2) tiles 2,3 ; column 15 <- g_sigma * exp(clamp(logit, -15, 15)) (trunc_exp backward)
             float c1 = acc[3][1], c3 = acc[3][3];
             if (t == 3) {
@@ -725,9 +749,12 @@ int tnl_mlp_forward(const tnl_mlp_dims* dims, const void* packed, const void* fe
     return finish_launch("mlp_forward");
 }
 
-int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
-                     uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1,
-                     float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream) {
+}  // extern "C"
+
+// tnl_mlp_backward (g_dirs == nullptr) and tnl_mlp_backward_dirs
+static int mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs, uint32_t M,
+                        const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1, float* g_W2,
+                        float* g_W3, float* g_W4, float* g_W5, float* g_dirs, tnl_stream_t stream) {
     if (M == 0) return 0;
     if (!dims_supported(dims) || (dims->hidden != 64 && !use_tc(dims, feat_fp16))) {
         set_error("mlp_backward: the 128-wide heads take the fp16 feature stream (tcgen05 kernels); fp32 features: hidden = hidden_color = 64 only");
@@ -739,26 +766,38 @@ int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* f
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (use_tc(dims, feat_fp16)) {
         TNL_ARG_CHECK(((uintptr_t)feat & 15) == 0 && ((uintptr_t)g_feat & 15) == 0, "feat/g_feat must be 16-byte aligned");
-        mlp_tc_backward(dims->in_dim, dims->hidden, static_cast<const uint8_t*>(packed) + legacy_packed_bytes(dims), feat, dirs, M, n_valid,
-                        g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, s);
-        return finish_launch("mlp_backward(tcgen05)");
+        const uint8_t* wpk = static_cast<const uint8_t*>(packed) + legacy_packed_bytes(dims);
+        if (!g_dirs) {
+            mlp_tc_backward(dims->in_dim, dims->hidden, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, s);
+            return finish_launch("mlp_backward(tcgen05)");
+        }
+#ifdef __CUDACC__   // (host builds of this file have no tcgen05 implementation: use_tc() is false there)
+        mlp_tc_backward_dirs(dims->in_dim, dims->hidden, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5,
+                             g_dirs, s);
+#endif
+        return finish_launch("mlp_backward_dirs(tcgen05)");
     }
     // two independent 4-warp CTAs per SM: while one is in its latency-bound recompute / dX phase the other runs the
     // shared-memory-bound weight-gradient phase (TNL_MLP_BWD_NW=8 selects the single 8-warp CTA variant)
     static const int nw = getenv("TNL_MLP_BWD_NW") ? atoi(getenv("TNL_MLP_BWD_NW")) : 4;
-#define CALLB_FH(K, NW, FHV)                                                                                             \
+#define CALLB_D(K, NW, FHV, DV)                                                                                          \
     do {                                                                                                                \
         using SMB = BwdSmem<K, 64, 64, NW>;                                                                             \
         static bool attr = false;                                                                                       \
         if (!attr) {                                                                                                    \
-            cudaFuncSetAttribute(k_mlp_bwd<K, 64, 64, NW, FHV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMB::BYTES); \
+            cudaFuncSetAttribute(k_mlp_bwd<K, 64, 64, NW, FHV, DV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMB::BYTES); \
             attr = true;                                                                                                \
         }                                                                                                               \
         const uint32_t ntiles = ceil_div(M, (uint32_t)(16 * NW));                                                        \
         const uint32_t blocks = min(ntiles, (uint32_t)(kNumSM * (NW == 4 ? 2 : 1)));                                     \
-        k_mlp_bwd<K, 64, 64, NW, FHV><<<blocks, NW * 32, SMB::BYTES, s>>>(static_cast<const uint32_t*>(packed), feat, dirs, \
+        k_mlp_bwd<K, 64, 64, NW, FHV, DV><<<blocks, NW * 32, SMB::BYTES, s>>>(static_cast<const uint32_t*>(packed), feat, dirs, \
                                                                           M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, \
-                                                                          g_W3, g_W4, g_W5);                             \
+                                                                          g_W3, g_W4, g_W5, g_dirs);                     \
+    } while (0)
+#define CALLB_FH(K, NW, FHV)                        \
+    do {                                            \
+        if (g_dirs) CALLB_D(K, NW, FHV, true);      \
+        else CALLB_D(K, NW, FHV, false);            \
     } while (0)
 #define CALLB_NW(K, NW)                  \
     do {                                 \
@@ -776,7 +815,29 @@ int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* f
 #undef CALLB
 #undef CALLB_NW
 #undef CALLB_FH
-    return finish_launch("mlp_backward");
+#undef CALLB_D
+    return finish_launch(g_dirs ? "mlp_backward_dirs" : "mlp_backward");
 }
+
+extern "C" {
+
+int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
+                     uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1,
+                     float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream) {
+    return mlp_backward(dims, packed, feat, feat_fp16, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, nullptr,
+                        stream);
+}
+
+int tnl_mlp_backward_dirs(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
+                          uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1,
+                          float* g_W2, float* g_W3, float* g_W4, float* g_W5, float* g_dirs, tnl_stream_t stream) {
+    if (M == 0) return 0;
+    TNL_ARG_CHECK(g_dirs, "null pointer");
+    // rows the kernels do not visit (>= *n_valid) keep these zeros
+    cudaMemsetAsync(g_dirs, 0, (size_t)M * 3 * sizeof(float), reinterpret_cast<cudaStream_t>(stream));   // (errors: finish_launch)
+    return mlp_backward(dims, packed, feat, feat_fp16, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, g_dirs,
+                        stream);
+}
+
 
 }  // extern "C"

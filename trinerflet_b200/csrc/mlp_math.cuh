@@ -38,6 +38,42 @@ __device__ __forceinline__ void sh16(float x, float y, float z, float (&o)[16]) 
     o[15] = 0.59004358992664352f * x * (-x2 + 3.0f * y2);
 }
 
+// Jacobian of sh16: J[a][ch] = d o[ch] / d (x, y, z)[a] (the reference's dy_dx, shencoder.cu kernel_sh)
+__device__ __forceinline__ void sh16_jacobian(float x, float y, float z, float (&jx)[16], float (&jy)[16], float (&jz)[16]) {
+    const float xy = x * y, xz = x * z, yz = y * z, x2 = x * x, y2 = y * y, z2 = z * z;
+    jx[0] = 0.f; jy[0] = 0.f; jz[0] = 0.f;
+    jx[1] = 0.f; jy[1] = -0.48860251190291987f; jz[1] = 0.f;
+    jx[2] = 0.f; jy[2] = 0.f; jz[2] = 0.48860251190291987f;
+    jx[3] = -0.48860251190291987f; jy[3] = 0.f; jz[3] = 0.f;
+    jx[4] = 1.0925484305920792f * y; jy[4] = 1.0925484305920792f * x; jz[4] = 0.f;
+    jx[5] = 0.f; jy[5] = -1.0925484305920792f * z; jz[5] = -1.0925484305920792f * y;
+    jx[6] = 0.f; jy[6] = 0.f; jz[6] = 1.89234939151512f * z;
+    jx[7] = -1.0925484305920792f * z; jy[7] = 0.f; jz[7] = -1.0925484305920792f * x;
+    jx[8] = 1.0925484305920792f * x; jy[8] = -1.0925484305920792f * y; jz[8] = 0.f;
+    jx[9] = -3.540261539559861f * xy; jy[9] = 1.7701307697799304f * (-x2 + y2); jz[9] = 0.f;
+    jx[10] = 2.8906114426405538f * yz; jy[10] = 2.8906114426405538f * xz; jz[10] = 2.8906114426405538f * xy;
+    jx[11] = 0.f; jy[11] = 0.45704579946446572f - 2.2852289973223288f * z2; jz[11] = -4.5704579946446575f * yz;
+    jx[12] = 0.f; jy[12] = 0.f; jz[12] = 5.597644988851731f * z2 - 1.1195289977703462f;
+    jx[13] = 0.45704579946446572f - 2.2852289973223288f * z2; jy[13] = 0.f; jz[13] = -4.5704579946446575f * xz;
+    jx[14] = 2.8906114426405538f * xz; jy[14] = -2.8906114426405538f * yz; jz[14] = 1.4453057213202769f * (x2 - y2);
+    jx[15] = 1.7701307697799304f * (-x2 + y2); jy[15] = 3.540261539559861f * xy; jz[15] = 0.f;
+}
+
+// g_d[a] = sum_ch g[ch] J[a][ch] over the first NCH = degree^2 channels, accumulated in channel order as the reference's
+// kernel_sh_backward does
+template <int NCH>
+__device__ __forceinline__ void sh_backward(float x, float y, float z, const float* g, float (&gd)[3]) {
+    float jx[16], jy[16], jz[16];
+    sh16_jacobian(x, y, z, jx, jy, jz);
+    gd[0] = gd[1] = gd[2] = 0.f;
+#pragma unroll
+    for (int ch = 0; ch < NCH; ++ch) {
+        gd[0] = fmaf(g[ch], jx[ch], gd[0]);
+        gd[1] = fmaf(g[ch], jy[ch], gd[1]);
+        gd[2] = fmaf(g[ch], jz[ch], gd[2]);
+    }
+}
+
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
 __device__ __forceinline__ float r16(float v) { return __half2float(__float2half_rn(v)); }
 

@@ -255,12 +255,16 @@ __device__ __forceinline__ void red_add_v4(float* addr, float4 v, float w) {   /
                  : "memory");
 }
 
-template <int K1, bool SCATTER>
+// DIRS variant: stage 7 takes d(in3) over all 32 columns, and the point's thread applies the SH Jacobian at its direction to the
+// fp16-rounded SH columns (0..15) -> g_dirs [M,3] (valid rows only).
+template <int K1, bool SCATTER, bool DIRS>
 __global__ void __launch_bounds__(544, 1)
 k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
              const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
              __half* __restrict__ g_feat, float* __restrict__ gW1, float* __restrict__ gW2, float* __restrict__ gW3,
-             float* __restrict__ gW4, float* __restrict__ gW5, unsigned long long* __restrict__ dbg, const PlaneScatter sc) {
+             float* __restrict__ gW4, float* __restrict__ gW5, unsigned long long* __restrict__ dbg, const PlaneScatter sc,
+             float* __restrict__ g_dirs) {
+    static_assert(!(SCATTER && DIRS), "the direction gradient is not on the training path");
     using W = TcW<K1>;
     using S = TcBwdSmem<K1>;
     // TMEM columns: chain accumulators of the two warpgroups | dW1 [64 x K1] | dW4 [64 x 64] | dW3 [64 x 32] | dW2^T, dW5^T [64 x 16]
@@ -331,8 +335,9 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
                     } else if (st == 6) {   // dh3 = dh4 W4 ;  dW4 += dh4^T h3
                         mma_group<4>(tc, op_kmajor(H44, 128, 0, 0), op_mnmajor(W44, 64, 0, 0), make_idesc(128, 64, false, true), false);
                         mma_group<8>(tmem + TM_W4, op_mnmajor(H44, 128, 0, 0), op_mnmajor(H34, 128, 0, 0), make_idesc(64, 64, true, true), accw);
-                    } else if (st == 7) {   // d(in3)[:, 16:32] = dh3 W3[:, 16:32] ;  dW3 += dh3^T in3
-                        mma_group<4>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 64, 0, 16), make_idesc(128, 16, false, true), false);
+                    } else if (st == 7) {   // d(in3)[:, 16:32] = dh3 W3[:, 16:32] (DIRS: all of d(in3) = dh3 W3) ;  dW3 += dh3^T in3
+                        if (DIRS) mma_group<4>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 64, 0, 0), make_idesc(128, 32, false, true), false);
+                        else mma_group<4>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 64, 0, 16), make_idesc(128, 16, false, true), false);
                         mma_group<8>(tmem + TM_W3, op_mnmajor(H34, 128, 0, 0), op_mnmajor(I34, 128, 0, 0), make_idesc(64, 32, true, true), accw);
                     } else if (st == 8) {   // dh1 = dh2 W2 ;  dW2^T += h1^T dh2
                         mma_group<1>(tc, op_kmajor(I34, 128, 0, 0), op_mnmajor(W24, 16, 0, 0), make_idesc(128, 64, false, true), false);
@@ -472,13 +477,25 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             }
             if (hf == 0) {   // dh2: column 0 <- g_sigma * exp(clamp(logit, -15, 15)) (trunc_exp backward), columns 1..15 <- d(geo)
                 float a[16];
-                tmem_load_row<16>(trow, a);
+                tmem_load_row<16>(trow + (DIRS ? 16u : 0u), a);
                 float dh2[16];
                 dh2[0] = gs * expf(fminf(fmaxf(logit, -15.f), 15.f));
 #pragma unroll
                 for (int j = 0; j < 15; ++j) dh2[1 + j] = a[j];
                 *reinterpret_cast<uint4*>(sub + S::I3 + (0 * 128 + t) * 16) = pack8<false>(dh2);
                 *reinterpret_cast<uint4*>(sub + S::I3 + (1 * 128 + t) * 16) = pack8<false>(dh2 + 8);
+                if constexpr (DIRS) {   // the SH columns, rounded to fp16 as the autocast linear backward returns them
+                    float gsh[16];
+                    tmem_load_row<16>(trow, gsh);
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) gsh[j] = r16(gsh[j]);
+                    if (v) {
+                        float gd[3];
+                        sh_backward<16>(d[0], d[1], d[2], gsh, gd);
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) g_dirs[3 * (size_t)m + j] = gd[j];
+                    }
+                }
             }
             TNL_HANDOFF();   // stage 8
             TNL_EPI_MASK(S::H1);
@@ -756,25 +773,40 @@ void mlp_tc_forward(uint32_t in_dim, uint32_t hidden, const void* wpk, const voi
 // optional device buffer of 64 cycle counters (tnl_mlp_tc_profile); nullptr in normal operation
 static unsigned long long* g_tc_dbg = nullptr;
 
-template <int K1, bool SCATTER>
+template <int K1, bool SCATTER, bool DIRS>
 static void launch_bwd(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
                        const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, const PlaneScatter& sc,
-                       cudaStream_t s) {
+                       float* g_dirs, cudaStream_t s) {
     using S = TcBwdSmem<K1>;
-    cudaFuncSetAttribute(k_mlp_tc_bwd<K1, SCATTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
+    cudaFuncSetAttribute(k_mlp_tc_bwd<K1, SCATTER, DIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
     const uint32_t blocks = min(ceil_div(M, 256u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
-    k_mlp_tc_bwd<K1, SCATTER><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M,
-                                                            n_valid, g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4,
-                                                            gW5, g_tc_dbg, sc);
+    k_mlp_tc_bwd<K1, SCATTER, DIRS><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M,
+                                                                  n_valid, g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4,
+                                                                  gW5, g_tc_dbg, sc, g_dirs);
 }
 
 void mlp_tc_backward(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
                      const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3,
                      float* gW4, float* gW5, cudaStream_t s) {
-    if (hidden == 128) { mlp_tc128_backward(in_dim, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s); return; }
+    if (hidden == 128) {
+        mlp_tc128_backward(in_dim, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, nullptr, s);
+        return;
+    }
     const PlaneScatter none{};
-    if (in_dim == 48) launch_bwd<48, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, s);
-    else launch_bwd<96, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, s);
+    if (in_dim == 48) launch_bwd<48, false, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, nullptr, s);
+    else launch_bwd<96, false, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, nullptr, s);
+}
+
+void mlp_tc_backward_dirs(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
+                          const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2,
+                          float* gW3, float* gW4, float* gW5, float* g_dirs, cudaStream_t s) {
+    if (hidden == 128) {
+        mlp_tc128_backward(in_dim, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
+        return;
+    }
+    const PlaneScatter none{};
+    if (in_dim == 48) launch_bwd<48, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, g_dirs, s);
+    else launch_bwd<96, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, g_dirs, s);
 }
 
 }  // namespace tnl
@@ -802,8 +834,8 @@ extern "C" int tnl_mlp_backward_scatter(const tnl_mlp_dims* dims, const void* pa
     const PlaneScatter sc{perm, xyz, g_planes, (int)R, inv_bound, fp16_coords};
     const uint8_t* wpk = static_cast<const uint8_t*>(packed) + mlp_tc_packed_offset(dims);
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (C == 16) launch_bwd<48, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, s);
-    else launch_bwd<96, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, s);
+    if (C == 16) launch_bwd<48, true, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, nullptr, s);
+    else launch_bwd<96, true, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, nullptr, g_W1, g_W2, g_W3, g_W4, g_W5, sc, nullptr, s);
     return finish_launch("mlp_backward_scatter(tcgen05)");
 }
 

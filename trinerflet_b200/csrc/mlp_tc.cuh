@@ -17,6 +17,10 @@ void mlp_tc_forward(uint32_t in_dim, uint32_t hidden, const void* wpk, const voi
 void mlp_tc_backward(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
                      const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3,
                      float* gW4, float* gW5, cudaStream_t s);
+// the same, also writing the direction gradient g_dirs [M,3] of the valid rows (tnl_mlp_backward_dirs)
+void mlp_tc_backward_dirs(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
+                          const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2,
+                          float* gW3, float* gW4, float* gW5, float* g_dirs, cudaStream_t s);
 // mlp.cu: where the tcgen05 tiles start inside the packed weight block, and whether the tcgen05 kernels serve these dims
 // (fp16 feature stream, not forced off by TNL_MLP_LEGACY)
 size_t mlp_tc_packed_offset(const tnl_mlp_dims* dims);
@@ -25,7 +29,7 @@ bool mlp_tc_selected(const tnl_mlp_dims* dims);
 void mlp_tc128_forward(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
                        float* sigma, float* rgb, float* geo, cudaStream_t s);
 void mlp_tc128_backward(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
-                        const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5,
+                        const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, float* g_dirs,
                         cudaStream_t s);
 
 }  // namespace tnl

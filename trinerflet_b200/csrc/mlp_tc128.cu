@@ -260,12 +260,14 @@ __device__ __forceinline__ void load_x_half_async(uint8_t* xtile, uint32_t t, ui
         asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst + kc * 2048u), "l"(src + kc * 8), "r"(nbytes) : "memory");
 }
 
-template <int K1>
+// DIRS: d(in3) over all 32 columns, and g_dirs [M,3] <- the SH Jacobian at the point's direction applied to the fp16-rounded
+// SH columns 0..15 (valid rows only)
+template <int K1, bool DIRS>
 __global__ void __launch_bounds__(256, 1)
 k_mlp_tc_bwd128(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
                 const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
                 __half* __restrict__ g_feat, float* __restrict__ gW1, float* __restrict__ gW2, float* __restrict__ gW3,
-                float* __restrict__ gW4, float* __restrict__ gW5) {
+                float* __restrict__ gW4, float* __restrict__ gW5, float* __restrict__ g_dirs) {
     using W = TcW128<K1>;
     using S = TcBwd128Smem<K1>;
     // TMEM columns: chain accumulator | dW1 [128 x K1] | dW4 [128 x 128] | dW3 [128 x 32] | dW2^T [128 x 16] | dW5^T [128 x 16]
@@ -393,17 +395,30 @@ k_mlp_tc_bwd128(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat
                    mma_group<8>(tmem + TM_W4, op_mnmajor(H44, 128, 0, 0), op_mnmajor(H34, 128, 0, 0), make_idesc(128, 128, true, true), accw)));  // dW4 += dh4^T h3
         load_x_half_async<K1>(smem + S::XR, t, hf, feat, p, v);   // relu(h4) / dh4 / d5 are dead: bring the feature tile back
         TNL_EPI_MASK(S::H3);
-        TNL_STAGE((mma_group<8>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 128, 0, 16), make_idesc(128, 16, false, true), false),        // d(in3)[:, 16:32]
+        TNL_STAGE((DIRS ? mma_group<8>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 128, 0, 0), make_idesc(128, 32, false, true), false)   // d(in3)
+                        : mma_group<8>(tc, op_kmajor(H34, 128, 0, 0), op_mnmajor(W34, 128, 0, 16), make_idesc(128, 16, false, true), false),  // d(in3)[:, 16:32]
                    mma_group<8>(tmem + TM_W3, op_mnmajor(H34, 128, 0, 0), op_mnmajor(I34, 128, 0, 0), make_idesc(128, 32, true, true), accw)));   // dW3 += dh3^T in3
         if (hf == 0) {   // dh2: column 0 <- g_sigma * exp(clamp(logit, -15, 15)) (trunc_exp backward), columns 1..15 <- d(geo)
             float a[16];
-            tmem_load_row<16>(trow, a);
+            tmem_load_row<16>(trow + (DIRS ? 16u : 0u), a);
             float dh2[16];
             dh2[0] = gs * expf(fminf(fmaxf(logit, -15.f), 15.f));
 #pragma unroll
             for (int j = 0; j < 15; ++j) dh2[1 + j] = a[j];
             *reinterpret_cast<uint4*>(smem + S::I3 + (0 * 128 + t) * 16) = pack8<false>(dh2);
             *reinterpret_cast<uint4*>(smem + S::I3 + (1 * 128 + t) * 16) = pack8<false>(dh2 + 8);
+            if constexpr (DIRS) {   // the SH columns, rounded to fp16 as the autocast linear backward returns them
+                float gsh[16];
+                tmem_load_row<16>(trow, gsh);
+#pragma unroll
+                for (int j = 0; j < 16; ++j) gsh[j] = r16(gsh[j]);
+                if (v) {
+                    float gd[3];
+                    sh_backward<16>(d[0], d[1], d[2], gsh, gd);
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) g_dirs[3 * (size_t)p + j] = gd[j];
+                }
+            }
         }
         TNL_STAGE((mma_group<1>(tc, op_kmajor(I34, 128, 0, 0), op_mnmajor(W24, 16, 0, 0), make_idesc(128, 128, false, true), false),         // dh1 = dh2 W2
                    mma_group<8>(tmem + TM_W2, op_mnmajor(H14, 128, 0, 0), op_mnmajor(I34, 128, 0, 0), make_idesc(128, 16, true, true), accw)));   // dW2^T += h1^T dh2
@@ -508,22 +523,31 @@ void mlp_tc128_forward(uint32_t in_dim, const void* wpk, const void* feat, const
     else launch_fwd128<144>(wpk, feat, dirs, M, n_valid, sigma, rgb, geo, s);
 }
 
+template <int K1, bool DIRS>
+static void launch_bwd128(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
+                          const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, float* g_dirs,
+                          cudaStream_t s) {
+    using S = TcBwd128Smem<K1>;
+    cudaFuncSetAttribute(k_mlp_tc_bwd128<K1, DIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
+    const uint32_t blocks = min(ceil_div(M, 128u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
+    k_mlp_tc_bwd128<K1, DIRS><<<blocks, 256, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M, n_valid,
+                                                            g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4, gW5, g_dirs);
+}
+
 template <int K1>
 static void launch_bwd128(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
-                          const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, cudaStream_t s) {
-    using S = TcBwd128Smem<K1>;
-    cudaFuncSetAttribute(k_mlp_tc_bwd128<K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
-    const uint32_t blocks = min(ceil_div(M, 128u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
-    k_mlp_tc_bwd128<K1><<<blocks, 256, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M, n_valid,
-                                                      g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4, gW5);
+                          const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, float* g_dirs,
+                          cudaStream_t s) {
+    if (g_dirs) launch_bwd128<K1, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
+    else launch_bwd128<K1, false>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, nullptr, s);
 }
 
 void mlp_tc128_backward(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
                         const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5,
-                        cudaStream_t s) {
-    if (in_dim == 48) launch_bwd128<48>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s);
-    else if (in_dim == 96) launch_bwd128<96>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s);
-    else launch_bwd128<144>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, s);
+                        float* g_dirs, cudaStream_t s) {
+    if (in_dim == 48) launch_bwd128<48>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
+    else if (in_dim == 96) launch_bwd128<96>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
+    else launch_bwd128<144>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
 }
 
 }  // namespace tnl

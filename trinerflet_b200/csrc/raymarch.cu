@@ -12,6 +12,7 @@
 //   * stream argument everywhere (the reference launches on the legacy default stream);
 //   * alive-ray compaction runs on the device (kills the per-iteration D2H sync of renderer.py:364).
 #include "common.cuh"
+#include "mlp_math.cuh"
 #include <float.h>
 
 namespace tnl {
@@ -785,6 +786,18 @@ __global__ void k_sh_encode(const float* __restrict__ inputs, float* __restrict_
     o[15] = 0.59004358992664352f * x * (-x2 + 3.0f * y2);
 }
 
+// input gradient of k_sh_encode: grad_inputs[b] = sum_ch grad[b][ch] d o[ch] / d inputs[b] (the reference's kernel_sh_backward)
+template <int NCH>
+__global__ void k_sh_encode_backward(const float* __restrict__ grad, const float* __restrict__ inputs, uint32_t B,
+                                     float* __restrict__ grad_inputs) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    float gd[3];
+    sh_backward<NCH>(inputs[3 * (size_t)b], inputs[3 * (size_t)b + 1], inputs[3 * (size_t)b + 2], grad + (size_t)b * NCH, gd);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) grad_inputs[3 * (size_t)b + a] = gd[a];
+}
+
 }  // namespace tnl
 
 // ================================================================================================
@@ -1005,6 +1018,19 @@ int tnl_sh_encode_forward(const float* inputs, float* outputs, uint32_t B, uint3
     }
     k_sh_encode<<<ceil_div(B, 256u), 256, 0, S(stream)>>>(inputs, outputs, B, degree);
     return finish_launch("sh_encode_forward");
+}
+
+int tnl_sh_encode_backward(const float* grad, const float* inputs, uint32_t B, uint32_t degree, float* grad_inputs,
+                           tnl_stream_t stream) {
+    if (B == 0) return 0;
+    TNL_ARG_CHECK(grad && inputs && grad_inputs, "null pointer");
+    TNL_ARG_CHECK(degree >= 1 && degree <= 4, "sh_encode_backward: degree must be 1..4");
+    const unsigned blocks = ceil_div(B, 256u);
+    if (degree == 1) k_sh_encode_backward<1><<<blocks, 256, 0, S(stream)>>>(grad, inputs, B, grad_inputs);
+    else if (degree == 2) k_sh_encode_backward<4><<<blocks, 256, 0, S(stream)>>>(grad, inputs, B, grad_inputs);
+    else if (degree == 3) k_sh_encode_backward<9><<<blocks, 256, 0, S(stream)>>>(grad, inputs, B, grad_inputs);
+    else k_sh_encode_backward<16><<<blocks, 256, 0, S(stream)>>>(grad, inputs, B, grad_inputs);
+    return finish_launch("sh_encode_backward");
 }
 
 }  // extern "C"

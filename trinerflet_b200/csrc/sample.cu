@@ -286,6 +286,64 @@ k_sample_xyz_grad(const float* __restrict__ g_feat, const float* __restrict__ pl
     }
 }
 
+// The same gradient for the NeRF sampler's streams: g_feat fp16 or fp32 (HALF), rows visited in `perm` order, rows >= *n_valid
+// set to zero, and the fp16-autocast rounding of the reference's backward (fp16_coords): its projection matmul returns the grid
+// gradient of each plane rounded to fp16, sums the two planes that read an axis in fp16 (the broadcast reduction of the matmul
+// backward), and the division by bound scales that in fp32.  A caller that needs the plane gradient too launches
+// tnl_sample_planes_backward separately: folding the scatter into this kernel's pass over the taps was measured slower than the two
+// launches (profiles/README.md).
+template <bool HALF>
+__global__ void __launch_bounds__(3 * XG_PPB)
+k_sample_xyz_grad_nerf(const void* __restrict__ g_feat_, const float* __restrict__ planes, const float* __restrict__ xyz, uint32_t M,
+                       int R, int C, float inv_bound, int fp16_coords, const int32_t* __restrict__ n_valid,
+                       const int32_t* __restrict__ perm, float* __restrict__ g_xyz) {
+    __shared__ float s_uv[XG_PPB][3][2];
+    const int p = threadIdx.x % 3, lp = threadIdx.x / 3;
+    const uint32_t i = blockIdx.x * XG_PPB + lp;
+    const uint32_t m = (i < M && perm) ? (uint32_t)__ldg(perm + i) : i;
+    const bool valid = i < M && !(n_valid && (int32_t)m >= *n_valid);
+    float gu = 0.f, gv = 0.f;
+    if (valid) {
+        float gx, gy, mx, my;
+        plane_coords(xyz, m, p, inv_bound, fp16_coords, gx, gy);
+        const float ix = to_pixel_grad(gx, R, mx), iy = to_pixel_grad(gy, R, my);
+        const float fx = floorf(ix), fy = floorf(iy);
+        const int x0 = (int)fx, y0 = (int)fy;
+        const bool x1ok = x0 + 1 <= R - 1, y1ok = y0 + 1 <= R - 1;
+        const float wx0 = (fx + 1.0f) - ix, wx1 = ix - fx, wy0 = (fy + 1.0f) - iy, wy1 = iy - fy;
+        const int cq_per = C >> 2;
+        const size_t row = (size_t)m * 3 * C + (size_t)p * C;
+        const float4* base = reinterpret_cast<const float4*>(planes + (((size_t)p * R + y0) * R + x0) * C);
+        const size_t dx = (size_t)cq_per, dy = (size_t)R * cq_per;
+        for (int q = 0; q < cq_per; ++q) {
+            const float4 g = HALF ? unpack4h(__ldg(reinterpret_cast<const uint2*>(g_feat_) + row / 4 + q))
+                                  : __ldg(reinterpret_cast<const float4*>(g_feat_) + row / 4 + q);
+            const float nw = dot4(__ldg(base + q), g);
+            const float ne = x1ok ? dot4(__ldg(base + dx + q), g) : 0.f;
+            const float sw = y1ok ? dot4(__ldg(base + dy + q), g) : 0.f;
+            const float se = (x1ok && y1ok) ? dot4(__ldg(base + dy + dx + q), g) : 0.f;
+            gu -= nw * wy0; gv -= nw * wx0;
+            gu += ne * wy0; gv -= ne * wx1;
+            gu -= sw * wy1; gv += sw * wx0;
+            gu += se * wy1; gv += se * wx1;
+        }
+        gu *= mx;
+        gv *= my;
+        if (fp16_coords) { gu = __half2float(__float2half_rn(gu)); gv = __half2float(__float2half_rn(gv)); }
+    }
+    s_uv[lp][p][0] = gu;
+    s_uv[lp][p][1] = gv;
+    __syncthreads();
+    if (i < M) {
+        // axis a = p of this thread: x <- u of planes 0, 1;  y <- v of plane 1, u of plane 2;  z <- v of planes 0, 2
+        float s = (p == 0) ? s_uv[lp][0][0] + s_uv[lp][1][0]
+                : (p == 1) ? s_uv[lp][1][1] + s_uv[lp][2][0]
+                           : s_uv[lp][0][1] + s_uv[lp][2][1];
+        if (fp16_coords) s = __half2float(__float2half_rn(s));
+        g_xyz[3 * (size_t)m + p] = valid ? s * inv_bound : 0.f;
+    }
+}
+
 template <int TPP>
 static void launch_fwd8(const float* planes, const float* xyz, uint32_t M, uint32_t R, float inv_bound, int fp16_coords,
                         const int32_t* n_valid, const int32_t* perm, void* feat, int half, cudaStream_t s) {
@@ -389,6 +447,25 @@ int tnl_sample_planes_backward_coords(const float* g_feat, const float* planes, 
     k_sample_xyz_grad<<<ceil_div(M, (uint32_t)XG_PPB), 3 * XG_PPB, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
         g_feat, planes, xyz, M, (int)R, (int)C, inv_bound, fp16_coords, g_xyz);
     return finish_launch("sample_planes_backward_coords");
+}
+
+int tnl_sample_planes_backward_xyz(const void* g_feat, int feat_fp16, const float* planes, const float* xyz, uint32_t M, uint32_t R,
+                                   uint32_t C, float inv_bound, int fp16_coords, const int32_t* n_valid, const int32_t* perm,
+                                   float* g_xyz, tnl_stream_t stream) {
+    if (M == 0) return 0;
+    TNL_ARG_CHECK(g_feat && planes && xyz && g_xyz, "null pointer");
+    TNL_ARG_CHECK(C >= 4 && C % 4 == 0 && R >= 2, "C must be a multiple of 4, R >= 2");
+    TNL_ARG_CHECK(((uintptr_t)planes & 15) == 0 && ((uintptr_t)g_feat & (feat_fp16 ? 7 : 15)) == 0,
+                  "planes must be 16-byte aligned, g_feat 8 (fp16) or 16 (fp32)");
+    const unsigned blocks = ceil_div(M, (uint32_t)XG_PPB);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (feat_fp16)
+        k_sample_xyz_grad_nerf<true><<<blocks, 3 * XG_PPB, 0, st>>>(g_feat, planes, xyz, M, (int)R, (int)C, inv_bound, fp16_coords, n_valid,
+                                                                   perm, g_xyz);
+    else
+        k_sample_xyz_grad_nerf<false><<<blocks, 3 * XG_PPB, 0, st>>>(g_feat, planes, xyz, M, (int)R, (int)C, inv_bound, fp16_coords, n_valid,
+                                                                    perm, g_xyz);
+    return finish_launch("sample_planes_backward_xyz");
 }
 
 }  // extern "C"

@@ -71,12 +71,14 @@ def _mlp_forward(feat, dirs, n_valid, W):
 
 
 class _FieldMLP(Function):
-    """(feat [M,3C], dirs [M,3]) -> sigma [M] fp32, rgb [M,3] fp32 (fp16-representable values)."""
+    """(feat [M,3C], dirs [M,3]) -> sigma [M] fp32, rgb [M,3] fp32 (fp16-representable values).  When dirs require grad the
+    backward is tnl_mlp_backward_dirs, which also returns their gradient."""
 
     @staticmethod
     def forward(ctx, feat, dirs, n_valid, W1, W2, W3, W4, W5):
         feat = feat.contiguous()
         ctx.in_dtype = feat.dtype
+        ctx.dirs_dtype = dirs.dtype
         if W1.shape[0] != 64:
             feat = feat.half()          # 128-wide heads: tcgen05 kernels only, fp16 feature stream (the first Linear's own rounding)
         elif feat.dtype != torch.float16:
@@ -97,12 +99,19 @@ class _FieldMLP(Function):
         g_rgb = g_rgb.contiguous().float()
         g_feat = torch.empty_like(feat)
         gW = [torch.zeros(s, device=feat.device, dtype=torch.float32) for s in ctx.wshapes]
-        call("tnl_mlp_backward", ctypes.byref(dims), ptr(packed), ptr(feat), int(feat.dtype == torch.float16), ptr(dirs), M,
-             ptr(n_valid) if has_nv else None, ptr(g_sigma), ptr(g_rgb), ptr(g_feat), *[ptr(g) for g in gW], stream())
+        args = (ctypes.byref(dims), ptr(packed), ptr(feat), int(feat.dtype == torch.float16), ptr(dirs), M,
+                ptr(n_valid) if has_nv else None, ptr(g_sigma), ptr(g_rgb), ptr(g_feat), *[ptr(g) for g in gW])
+        g_dirs = None
+        if ctx.needs_input_grad[1]:
+            g_dirs = torch.empty(M, 3, device=feat.device, dtype=torch.float32)
+            call("tnl_mlp_backward_dirs", *args, ptr(g_dirs), stream())
+            g_dirs = g_dirs.to(ctx.dirs_dtype)
+        else:
+            call("tnl_mlp_backward", *args, stream())
         # (rows >= *n_valid of g_feat are never read: the sampling backward skips them with the same counter)
         if g_feat.dtype != ctx.in_dtype:
             g_feat = g_feat.to(ctx.in_dtype)
-        return (g_feat, None, None, *gW)
+        return (g_feat, g_dirs, None, *gW)
 
 
 class _Field(Function):
@@ -208,9 +217,9 @@ class NeRFNetwork(NeRFRenderer):
             perm = cell_sort(x, self.bound, n_valid, 64)
         fused = self._fused()
         if (fused and perm is not None and self.hidden_dim == 64 and self.in_dim in (48, 96)
-                and self.encoder.scatter_plane_hook is None):
+                and self.encoder.scatter_plane_hook is None and not x.requires_grad and not d.requires_grad):
             # training step: one fused MLP-backward + plane scatter (the plane-by-plane exchange of the multi-GPU step scatters
-            # through _SamplePlanes instead)
+            # through _SamplePlanes instead; input gradients go through _SamplePlanes / _FieldMLP)
             planes, gbuf = self.encoder.planes_and_grad_buffer()
             return _Field.apply(planes, x, d, self.bound, n_valid, perm, gbuf, *self._weights())
         # fused path: the feature stream between the gather and the MLP kernels is fp16 (the first Linear's own rounding)

@@ -1,10 +1,12 @@
-"""Drop-in for the reference's `shencoder` package (aux_libs/shencoder/sphere_harmonics.py:14-87).
-Degree <= 4 forward only: on the hot path view directions never require grad (sphere_harmonics.py:84), and
-inside NeRFNetwork the SH evaluation is fused into the MLP kernel; this module serves stand-alone callers."""
+"""Drop-in for the reference's `shencoder` package (aux_libs/shencoder/sphere_harmonics.py:14-87), degree <= 4.
+As in the reference, the input gradient is computed when the inputs require grad (sphere_harmonics.py:84); it is
+once-differentiable.  Inside NeRFNetwork the SH evaluation is fused into the MLP kernels; this module serves stand-alone
+callers and the fp32 library path of the heads."""
 import torch
 import torch.nn as nn
 from torch.autograd import Function
-from torch.amp import custom_fwd
+from torch.autograd.function import once_differentiable
+from torch.amp import custom_bwd, custom_fwd
 
 from ._lib import call, ptr, stream
 
@@ -13,17 +15,25 @@ class _sh_encoder(Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, inputs, degree, calc_grad_inputs=False):
-        if calc_grad_inputs:
-            raise NotImplementedError("SH input gradients are not on the reconstruction hot path (dirs never require grad)")
         inputs = inputs.contiguous()
         B = inputs.shape[0]
         outputs = torch.empty(B, degree ** 2, dtype=inputs.dtype, device=inputs.device)
         call("tnl_sh_encode_forward", ptr(inputs), ptr(outputs), B, int(degree), stream())
+        ctx.save_for_backward(inputs if calc_grad_inputs else None)
+        ctx.degree = int(degree)
         return outputs
 
     @staticmethod
+    @once_differentiable
+    @custom_bwd(device_type="cuda")
     def backward(ctx, grad):
-        return None, None, None
+        (inputs,) = ctx.saved_tensors
+        if inputs is None:
+            return None, None, None
+        grad = grad.contiguous().float()
+        grad_inputs = torch.empty_like(inputs)
+        call("tnl_sh_encode_backward", ptr(grad), ptr(inputs), inputs.shape[0], ctx.degree, ptr(grad_inputs), stream())
+        return grad_inputs, None, None
 
 
 sh_encode = _sh_encoder.apply
@@ -45,5 +55,5 @@ class SHEncoder(nn.Module):
         inputs = inputs / size
         prefix_shape = list(inputs.shape[:-1])
         inputs = inputs.reshape(-1, self.input_dim)
-        outputs = sh_encode(inputs, self.degree, False)
+        outputs = sh_encode(inputs, self.degree, inputs.requires_grad)
         return outputs.reshape(prefix_shape + [self.output_dim])

@@ -284,28 +284,37 @@ class _SamplePlanes(Function):
     def forward(ctx, planes, coords, bound, fp16_coords, n_valid, perm=None, half_out=False, grad_buf=None):
         ctx.grad_buf = grad_buf
         feat, coords, ctx.meta = gather_features(planes, coords, bound, fp16_coords, n_valid, perm, half_out)
+        # the position gradient reads the planes (the gather's channels-last copy: no copy when they are stored that way)
         ctx.save_for_backward(coords, n_valid if n_valid is not None else torch.empty(0),
-                              perm if perm is not None else torch.empty(0))
+                              perm if perm is not None else torch.empty(0),
+                              to_cl_planes(planes.detach()) if ctx.needs_input_grad[1] else None)
         return feat
 
     @staticmethod
     def backward(ctx, g_feat):
-        coords, n_valid, perm = ctx.saved_tensors
+        coords, n_valid, perm, planes_cl = ctx.saved_tensors
         M, R, C, inv, fp16_coords, has_nv, has_perm, half = ctx.meta
         g_feat = g_feat.contiguous().half() if half else g_feat.contiguous().float()
-        g_planes, external, plane_hook = take_grad_buffer(ctx, C, R, g_feat.device)
-        if plane_hook is not None and C in (16, 32, 48):
-            # multi-GPU step: plane by plane, so that the caller can start exchanging plane p while plane p + 1 scatters
-            for p in range(3):
-                call("tnl_sample_planes_backward_plane", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords,
-                     ptr(n_valid) if has_nv else None, ptr(perm) if has_perm else None, ptr(g_planes), p, stream())
-                plane_hook(p)
-        else:
-            call("tnl_sample_planes_backward", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords,
-                 ptr(n_valid) if has_nv else None, ptr(perm) if has_perm else None, ptr(g_planes), stream())
-        if external:      # the caller's persistent (symmetric-memory) buffer holds the result; autograd must not clone 1.6 GB of it
-            return None, None, None, None, None, None, None, None
-        return g_planes, None, None, None, None, None, None, None
+        nv, pm = (ptr(n_valid) if has_nv else None), (ptr(perm) if has_perm else None)
+        g_planes, external = None, False
+        if ctx.needs_input_grad[0]:
+            g_planes, external, plane_hook = take_grad_buffer(ctx, C, R, g_feat.device)
+            if plane_hook is not None and C in (16, 32, 48):
+                # multi-GPU step: plane by plane, so that the caller can start exchanging plane p while plane p + 1 scatters
+                for p in range(3):
+                    call("tnl_sample_planes_backward_plane", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm,
+                         ptr(g_planes), p, stream())
+                    plane_hook(p)
+            else:
+                call("tnl_sample_planes_backward", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm,
+                     ptr(g_planes), stream())
+        g_xyz = None
+        if ctx.needs_input_grad[1]:
+            g_xyz = torch.empty(M, 3, device=g_feat.device, dtype=torch.float32)
+            call("tnl_sample_planes_backward_xyz", ptr(g_feat), int(half), ptr(planes_cl), ptr(coords), M, R, C, inv, fp16_coords, nv, pm,
+                 ptr(g_xyz), stream())
+        # external: the caller's persistent (symmetric-memory) buffer holds the plane gradient; autograd must not clone 1.6 GB of it
+        return None if external else g_planes, g_xyz, None, None, None, None, None, None
 
 
 def cell_sort(coords, bound, n_valid=None, G=64):
