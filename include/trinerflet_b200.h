@@ -219,6 +219,19 @@ int tnl_sample_planes_backward(const void* g_feat, int feat_fp16, const float* x
 int tnl_sample_planes_backward_plane(const void* g_feat, int feat_fp16, const float* xyz, uint32_t M, uint32_t R, uint32_t C,
                                      float inv_bound, int fp16_coords, const int32_t* n_valid, const int32_t* perm,
                                      float* g_planes, uint32_t plane, tnl_stream_t stream);
+/* Deterministic mode (torch.use_deterministic_algorithms): the scatter of tnl_sample_planes_backward with sums that do not depend on
+ * the visiting order (perm) or the thread schedule.  Contributions are added in 64-bit fixed point: m = max |g_feat| over the rows
+ * below *n_valid, 2^e > m, mu = ceil(log2 M), unit = 2^(e + mu - 62); each contribution is rounded to a multiple of the unit (no
+ * partial sum can overflow), and each texel's sum is converted to fp32 once and added to g_planes.  Per texel the result is within
+ * n * unit / 2 (n = its contributions) plus one fp32 rounding of the exact sum.  If a g_feat value below *n_valid is inf or NaN,
+ * every converted g_planes element is NaN.  tile_ids == NULL: the whole planes; else only the listed T x T tiles (tile_ids /
+ * tile_count / tile_capacity as tnl_tiles_zero) are accumulated and converted, contributions elsewhere are dropped (the
+ * work-list IDWT backward reads only those tiles).  workspace: tnl_sample_planes_backward_det_workspace(R, C) bytes (int64 accumulator), 256-byte aligned. */
+size_t tnl_sample_planes_backward_det_workspace(uint32_t R, uint32_t C);
+int tnl_sample_planes_backward_det(const void* g_feat, int feat_fp16, const float* xyz, uint32_t M, uint32_t R, uint32_t C,
+                                   float inv_bound, int fp16_coords, const int32_t* n_valid, const int32_t* perm,
+                                   const int32_t* tile_ids, const int32_t* tile_count, uint32_t tile_capacity, uint32_t T,
+                                   float* g_planes, void* workspace, size_t workspace_bytes, tnl_stream_t stream);
 
 /* Gradient with respect to the sample positions (grid_sampler_2d_backward w.r.t. the grid, chained through u = xyz * inv_bound):
  * g_xyz [M][3] = d(sum g_feat * feat)/d(xyz), written (not accumulated).  The derivative is zero along an axis whose projected
@@ -290,6 +303,17 @@ int tnl_mlp_backward_dirs(const tnl_mlp_dims* dims, const void* packed, const vo
                           uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb,
                           void* g_feat, float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, float* g_dirs,
                           tnl_stream_t stream);
+/* Deterministic mode (torch.use_deterministic_algorithms): tnl_mlp_backward (g_dirs == NULL) or tnl_mlp_backward_dirs with weight
+ * gradients that do not depend on the order in which the CTAs finish.  Each CTA of the same kernels writes its partial sums to its
+ * own slot of `workspace` instead of adding them with fp32 atomics, and a reduction kernel adds the slots in index order to
+ * g_W1..g_W5 (accumulated, as tnl_mlp_backward does).  The tile schedule is static, so the result depends on M, *n_valid and the
+ * inputs only: the same bits on every call.  The workspace (16-byte aligned) holds tnl_mlp_backward_det_workspace(dims,
+ * feat_fp16, M) bytes (0: unsupported dims); g_feat and g_dirs are the same as those of the default entry points. */
+size_t tnl_mlp_backward_det_workspace(const tnl_mlp_dims* dims, int feat_fp16, uint32_t M);
+int tnl_mlp_backward_det(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
+                         uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat,
+                         float* g_W1, float* g_W2, float* g_W3, float* g_W4, float* g_W5, float* g_dirs, void* workspace,
+                         size_t workspace_bytes, tnl_stream_t stream);
 
 /* Diagnostic: ONE tcgen05.mma product D[M x N] = A B^T with fp16 operands given as plain row-major matrices
  * (A: [a_rows][a_cols] = [M][K] if a_mn == 0, [K][M] if a_mn != 0; B likewise with N), staged in the un-swizzled

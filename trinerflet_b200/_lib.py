@@ -52,6 +52,9 @@ SIGNATURES = {
     "tnl_sample_planes_forward": (_int, [_vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _int, _vp]),
     "tnl_sample_planes_backward": (_int, [_vp, _int, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _vp]),
     "tnl_sample_planes_backward_plane": (_int, [_vp, _int, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _u32, _vp]),
+    "tnl_sample_planes_backward_det_workspace": (_sz, [_u32, _u32]),
+    "tnl_sample_planes_backward_det": (_int, [_vp, _int, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _vp, _u32, _u32, _vp, _vp,
+                                              _sz, _vp]),
     "tnl_sample_planes_backward_coords": (_int, [_vp, _vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp]),
     "tnl_sample_planes_backward_xyz": (_int, [_vp, _int, _vp, _vp, _u32, _u32, _u32, _f32, _int, _vp, _vp, _vp, _vp]),
     "tnl_cell_sort_workspace": (_sz, [_u32, _u32]),
@@ -61,6 +64,8 @@ SIGNATURES = {
     "tnl_mlp_forward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_backward": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tnl_mlp_backward_dirs": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "tnl_mlp_backward_det_workspace": (_sz, [_DP, _int, _u32]),
+    "tnl_mlp_backward_det": (_int, [_DP, _vp, _vp, _int, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "tnl_mlp_backward_scatter": (_int, [_DP, _vp, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _u32, _u32, _f32, _int, _vp, _vp, _vp,
                                         _vp, _vp, _vp, _vp]),
     "tnl_idwt_level_forward_sparse": (_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp]),
@@ -118,6 +123,41 @@ def stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def deterministic():
+    """True under torch.use_deterministic_algorithms(True): the package then launches its order-independent kernels (the
+    fixed-point plane-gradient scatter, the slot-ordered MLP weight-gradient reduction) and torch's deterministic reductions
+    instead of fp32 / fp64 atomics, so a single-GPU training step gives the same bits for the same inputs."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def alert_nondeterministic(what):
+    """torch's rule for an operation without a deterministic implementation: in deterministic mode raise, or warn under
+    warn_only=True."""
+    if not deterministic():
+        return
+    msg = f"trinerflet_b200: {what} has no deterministic implementation (torch.use_deterministic_algorithms is on)"
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        import warnings
+        warnings.warn(msg)
+    else:
+        raise RuntimeError(msg)
+
+
+_workspaces = {}
+
+
+def workspace(key, nbytes, device):
+    """A persistent device scratch buffer of at least nbytes (one per key and device), reused by every call: the
+    deterministic kernels need gigabytes at the larger configs, and torch fills fresh allocations in deterministic mode."""
+    k = (key, str(device))
+    buf = _workspaces.get(k)
+    if buf is None or buf.numel() < nbytes:
+        _workspaces[k] = None
+        buf = torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=device)
+        _workspaces[k] = buf
+    return buf
+
+
 def ptr(t):
     """Device pointer of a CUDA tensor (None -> NULL). The tensor must be contiguous in the layout the ABI expects."""
     if t is None:
@@ -134,7 +174,7 @@ def check(rc, what):
 
 
 # number of kernels each ABI call launches (for the launch counter the benchmark reports)
-KERNELS_PER_CALL = {"tnl_march_rays_train": 6, "tnl_composite_rays_train_backward": 2, "tnl_compact_alive": 3, "tnl_compact_alive_dev": 3, "tnl_cell_sort": 5,
+KERNELS_PER_CALL = {"tnl_march_rays_train": 6, "tnl_sample_planes_backward_det": 4, "tnl_mlp_backward_det": 2, "tnl_composite_rays_train_backward": 2, "tnl_compact_alive": 3, "tnl_compact_alive_dev": 3, "tnl_cell_sort": 5,
                     "tnl_mlp_pack_weights": 2}
 # work-list IDWT calls launch one kernel per requested part (position of the `parts` argument from the end)
 _PARTS_ARG = {"tnl_idwt_level_forward_sparse": -2, "tnl_idwt_level_backward_sparse": -3,

@@ -424,7 +424,8 @@ __device__ __forceinline__ void relu_mask(uint32_t (&d)[KS][4], const uint32_t (
 }
 
 // DIRS: also g_dirs [M,3] <- the SH Jacobian applied to the fp16-rounded SH columns of d(in2) (valid rows only)
-template <int K1, int H, int HC, int NW, bool FH, bool DIRS>
+// DET: the weight gradients go to slot blockIdx.x of the workspace gW1 .. gW5 point into (wgrad_add)
+template <int K1, int H, int HC, int NW, bool FH, bool DIRS, bool DET = false>
 __global__ void __launch_bounds__(NW * 32, NW == 4 ? 2 : 1)
 k_mlp_bwd(const uint32_t* __restrict__ wp, const void* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
           const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
@@ -616,29 +617,33 @@ k_mlp_bwd(const uint32_t* __restrict__ wp, const void* __restrict__ feat, const 
     }
     // ------------------------------ flush weight gradients ------------------------------
     {
+        if constexpr (DET) {   // this CTA's slot of the workspace
+            const size_t o = (size_t)blockIdx.x * wgrad_slot(K1, H).size;
+            gW1 += o; gW2 += o; gW3 += o; gW4 += o; gW5 += o;
+        }
         const int nb = warp / SPLIT, hf = warp % SPLIT;
         const int n0 = nb * 16 + g, n1 = n0 + 8;
 #pragma unroll
         for (int q = 0; q < T1; ++q) {
             const int k = (hf * T1 + q) * 8 + 2 * t;
-            atomicAdd(gW1 + (size_t)n0 * K1 + k, acc1[q][0]);
-            atomicAdd(gW1 + (size_t)n0 * K1 + k + 1, acc1[q][1]);
-            atomicAdd(gW1 + (size_t)n1 * K1 + k, acc1[q][2]);
-            atomicAdd(gW1 + (size_t)n1 * K1 + k + 1, acc1[q][3]);
+            wgrad_add<DET>(gW1 + (size_t)n0 * K1 + k, acc1[q][0]);
+            wgrad_add<DET>(gW1 + (size_t)n0 * K1 + k + 1, acc1[q][1]);
+            wgrad_add<DET>(gW1 + (size_t)n1 * K1 + k, acc1[q][2]);
+            wgrad_add<DET>(gW1 + (size_t)n1 * K1 + k + 1, acc1[q][3]);
         }
 #pragma unroll
         for (int q = 0; q < T4; ++q) {
             const int k = (hf * T4 + q) * 8 + 2 * t;
-            atomicAdd(gW4 + (size_t)n0 * HC + k, acc4[q][0]);
-            atomicAdd(gW4 + (size_t)n0 * HC + k + 1, acc4[q][1]);
-            atomicAdd(gW4 + (size_t)n1 * HC + k, acc4[q][2]);
-            atomicAdd(gW4 + (size_t)n1 * HC + k + 1, acc4[q][3]);
+            wgrad_add<DET>(gW4 + (size_t)n0 * HC + k, acc4[q][0]);
+            wgrad_add<DET>(gW4 + (size_t)n0 * HC + k + 1, acc4[q][1]);
+            wgrad_add<DET>(gW4 + (size_t)n1 * HC + k, acc4[q][2]);
+            wgrad_add<DET>(gW4 + (size_t)n1 * HC + k + 1, acc4[q][3]);
         }
 #pragma unroll
         for (int q = 0; q < T3; ++q) {
             const int k = (hf * T3 + q) * 8 + 2 * t;  // internal color_net[0] column: 0..15 SH, 16..30 geo, 31 padding
-            if (k < 31) { atomicAdd(gW3 + (size_t)n0 * 31 + k, acc3[q][0]); atomicAdd(gW3 + (size_t)n1 * 31 + k, acc3[q][2]); }
-            if (k + 1 < 31) { atomicAdd(gW3 + (size_t)n0 * 31 + k + 1, acc3[q][1]); atomicAdd(gW3 + (size_t)n1 * 31 + k + 1, acc3[q][3]); }
+            if (k < 31) { wgrad_add<DET>(gW3 + (size_t)n0 * 31 + k, acc3[q][0]); wgrad_add<DET>(gW3 + (size_t)n1 * 31 + k, acc3[q][2]); }
+            if (k + 1 < 31) { wgrad_add<DET>(gW3 + (size_t)n0 * 31 + k + 1, acc3[q][1]); wgrad_add<DET>(gW3 + (size_t)n1 * 31 + k + 1, acc3[q][3]); }
         }
 #pragma unroll
         for (int q = 0; q < T25; ++q) {
@@ -646,16 +651,28 @@ k_mlp_bwd(const uint32_t* __restrict__ wp, const void* __restrict__ feat, const 
             {   // sigma_net[1]: internal row j < 15 -> reference row j+1, internal 15 -> row 0
                 const int ra = g + 1;                    // internal row g  (< 8)
                 const int rb = (g + 8 < 15) ? g + 9 : 0; // internal row g+8
-                atomicAdd(gW2 + (size_t)ra * H + k, acc2[q][0]);
-                atomicAdd(gW2 + (size_t)ra * H + k + 1, acc2[q][1]);
-                atomicAdd(gW2 + (size_t)rb * H + k, acc2[q][2]);
-                atomicAdd(gW2 + (size_t)rb * H + k + 1, acc2[q][3]);
+                wgrad_add<DET>(gW2 + (size_t)ra * H + k, acc2[q][0]);
+                wgrad_add<DET>(gW2 + (size_t)ra * H + k + 1, acc2[q][1]);
+                wgrad_add<DET>(gW2 + (size_t)rb * H + k, acc2[q][2]);
+                wgrad_add<DET>(gW2 + (size_t)rb * H + k + 1, acc2[q][3]);
             }
             if (g < 3) {  // color_net[2]: rows 0..2 real
-                atomicAdd(gW5 + (size_t)g * HC + k, acc5[q][0]);
-                atomicAdd(gW5 + (size_t)g * HC + k + 1, acc5[q][1]);
+                wgrad_add<DET>(gW5 + (size_t)g * HC + k, acc5[q][0]);
+                wgrad_add<DET>(gW5 + (size_t)g * HC + k + 1, acc5[q][1]);
             }
         }
+    }
+}
+
+// g_W += the sum of the per-CTA slots of a DET backward kernel, in slot order (wgrad_slot layout)
+__global__ void __launch_bounds__(256)
+k_wgrad_reduce(const float* __restrict__ slots, uint32_t nslots, WgradSlot L, float* __restrict__ gW1, float* __restrict__ gW2,
+               float* __restrict__ gW3, float* __restrict__ gW4, float* __restrict__ gW5) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < L.size; i += (size_t)gridDim.x * blockDim.x) {
+        float acc = 0.f;
+        for (uint32_t b = 0; b < nslots; ++b) acc += slots[(size_t)b * L.size + i];
+        float* dst = i < L.o2 ? gW1 + i : i < L.o3 ? gW2 + (i - L.o2) : i < L.o4 ? gW3 + (i - L.o3) : i < L.o5 ? gW4 + (i - L.o4) : gW5 + (i - L.o5);
+        *dst += acc;
     }
 }
 
@@ -751,10 +768,27 @@ int tnl_mlp_forward(const tnl_mlp_dims* dims, const void* packed, const void* fe
 
 }  // extern "C"
 
-// tnl_mlp_backward (g_dirs == nullptr) and tnl_mlp_backward_dirs
+// CTAs of the mma.sync backward kernel: two independent 4-warp CTAs per SM -- while one is in its latency-bound recompute / dX
+// phase the other runs the shared-memory-bound weight-gradient phase (TNL_MLP_BWD_NW=8 selects the single 8-warp CTA variant)
+static int mlp_bwd_warps() {
+    static const int nw = getenv("TNL_MLP_BWD_NW") ? atoi(getenv("TNL_MLP_BWD_NW")) : 4;
+    return nw == 8 ? 8 : 4;
+}
+static uint32_t mlp_bwd_blocks(uint32_t M, int nw) {
+    return min(ceil_div(M, (uint32_t)(16 * nw)), (uint32_t)(kNumSM * (nw == 4 ? 2 : 1)));
+}
+// slots of the deterministic weight-gradient reduction: one per CTA of the kernel mlp_backward launches for these arguments
+static uint32_t mlp_det_slots(const tnl_mlp_dims* d, int feat_fp16, uint32_t M) {
+#ifdef __CUDACC__
+    if (use_tc(d, feat_fp16)) return mlp_tc_backward_blocks(d->hidden, M);
+#endif
+    return mlp_bwd_blocks(M, mlp_bwd_warps());
+}
+
+// tnl_mlp_backward (g_dirs == nullptr), tnl_mlp_backward_dirs, and with det_slots != nullptr tnl_mlp_backward_det
 static int mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs, uint32_t M,
                         const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1, float* g_W2,
-                        float* g_W3, float* g_W4, float* g_W5, float* g_dirs, tnl_stream_t stream) {
+                        float* g_W3, float* g_W4, float* g_W5, float* g_dirs, float* det_slots, tnl_stream_t stream) {
     if (M == 0) return 0;
     if (!dims_supported(dims) || (dims->hidden != 64 && !use_tc(dims, feat_fp16))) {
         set_error("mlp_backward: the 128-wide heads take the fp16 feature stream (tcgen05 kernels); fp32 features: hidden = hidden_color = 64 only");
@@ -767,6 +801,12 @@ static int mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void
     if (use_tc(dims, feat_fp16)) {
         TNL_ARG_CHECK(((uintptr_t)feat & 15) == 0 && ((uintptr_t)g_feat & 15) == 0, "feat/g_feat must be 16-byte aligned");
         const uint8_t* wpk = static_cast<const uint8_t*>(packed) + legacy_packed_bytes(dims);
+#ifdef __CUDACC__
+        if (det_slots) {
+            mlp_tc_backward_det(dims->in_dim, dims->hidden, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, det_slots, g_dirs, s);
+            return finish_launch("mlp_backward_det(tcgen05)");
+        }
+#endif
         if (!g_dirs) {
             mlp_tc_backward(dims->in_dim, dims->hidden, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, s);
             return finish_launch("mlp_backward(tcgen05)");
@@ -777,22 +817,28 @@ static int mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void
 #endif
         return finish_launch("mlp_backward_dirs(tcgen05)");
     }
-    // two independent 4-warp CTAs per SM: while one is in its latency-bound recompute / dX phase the other runs the
-    // shared-memory-bound weight-gradient phase (TNL_MLP_BWD_NW=8 selects the single 8-warp CTA variant)
-    static const int nw = getenv("TNL_MLP_BWD_NW") ? atoi(getenv("TNL_MLP_BWD_NW")) : 4;
-#define CALLB_D(K, NW, FHV, DV)                                                                                          \
+    const int nw = mlp_bwd_warps();
+    const uint32_t blocks = mlp_bwd_blocks(M, nw);
+#define CALLB_DD(K, NW, FHV, DV, DETV, W1, W2, W3, W4, W5)                                                               \
     do {                                                                                                                \
         using SMB = BwdSmem<K, 64, 64, NW>;                                                                             \
         static bool attr = false;                                                                                       \
         if (!attr) {                                                                                                    \
-            cudaFuncSetAttribute(k_mlp_bwd<K, 64, 64, NW, FHV, DV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMB::BYTES); \
+            cudaFuncSetAttribute(k_mlp_bwd<K, 64, 64, NW, FHV, DV, DETV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMB::BYTES); \
             attr = true;                                                                                                \
         }                                                                                                               \
-        const uint32_t ntiles = ceil_div(M, (uint32_t)(16 * NW));                                                        \
-        const uint32_t blocks = min(ntiles, (uint32_t)(kNumSM * (NW == 4 ? 2 : 1)));                                     \
-        k_mlp_bwd<K, 64, 64, NW, FHV, DV><<<blocks, NW * 32, SMB::BYTES, s>>>(static_cast<const uint32_t*>(packed), feat, dirs, \
-                                                                          M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, \
-                                                                          g_W3, g_W4, g_W5, g_dirs);                     \
+        k_mlp_bwd<K, 64, 64, NW, FHV, DV, DETV><<<blocks, NW * 32, SMB::BYTES, s>>>(static_cast<const uint32_t*>(packed), feat, dirs, \
+                                                                                M, n_valid, g_sigma, g_rgb, g_feat, W1, W2, W3, W4, W5, \
+                                                                                g_dirs);                                 \
+    } while (0)
+#define CALLB_D(K, NW, FHV, DV)                                                                                          \
+    do {                                                                                                                \
+        if (det_slots) {                                                                                                \
+            const WgradSlot L = wgrad_slot(K, 64);                                                                      \
+            CALLB_DD(K, NW, FHV, DV, true, det_slots, det_slots + L.o2, det_slots + L.o3, det_slots + L.o4, det_slots + L.o5); \
+        } else {                                                                                                        \
+            CALLB_DD(K, NW, FHV, DV, false, g_W1, g_W2, g_W3, g_W4, g_W5);                                              \
+        }                                                                                                               \
     } while (0)
 #define CALLB_FH(K, NW, FHV)                        \
     do {                                            \
@@ -816,6 +862,7 @@ static int mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void
 #undef CALLB_NW
 #undef CALLB_FH
 #undef CALLB_D
+#undef CALLB_DD
     return finish_launch(g_dirs ? "mlp_backward_dirs" : "mlp_backward");
 }
 
@@ -825,7 +872,7 @@ int tnl_mlp_backward(const tnl_mlp_dims* dims, const void* packed, const void* f
                      uint32_t M, const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1,
                      float* g_W2, float* g_W3, float* g_W4, float* g_W5, tnl_stream_t stream) {
     return mlp_backward(dims, packed, feat, feat_fp16, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, nullptr,
-                        stream);
+                        nullptr, stream);
 }
 
 int tnl_mlp_backward_dirs(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs,
@@ -836,7 +883,33 @@ int tnl_mlp_backward_dirs(const tnl_mlp_dims* dims, const void* packed, const vo
     // rows the kernels do not visit (>= *n_valid) keep these zeros
     cudaMemsetAsync(g_dirs, 0, (size_t)M * 3 * sizeof(float), reinterpret_cast<cudaStream_t>(stream));   // (errors: finish_launch)
     return mlp_backward(dims, packed, feat, feat_fp16, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5, g_dirs,
-                        stream);
+                        nullptr, stream);
+}
+
+size_t tnl_mlp_backward_det_workspace(const tnl_mlp_dims* dims, int feat_fp16, uint32_t M) {
+    if (!dims_supported(dims) || M == 0) return 0;
+    return (size_t)mlp_det_slots(dims, feat_fp16, M) * wgrad_slot(dims->in_dim, dims->hidden).size * sizeof(float);
+}
+
+int tnl_mlp_backward_det(const tnl_mlp_dims* dims, const void* packed, const void* feat, int feat_fp16, const float* dirs, uint32_t M,
+                         const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* g_W1, float* g_W2,
+                         float* g_W3, float* g_W4, float* g_W5, float* g_dirs, void* workspace, size_t workspace_bytes,
+                         tnl_stream_t stream) {
+    if (M == 0) return 0;
+    const size_t need = tnl_mlp_backward_det_workspace(dims, feat_fp16, M);
+    TNL_ARG_CHECK(workspace != nullptr && need > 0 && workspace_bytes >= need && ((uintptr_t)workspace & 15) == 0,
+                  "workspace: tnl_mlp_backward_det_workspace bytes, 16-byte aligned (supported dims)");
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    if (g_dirs) cudaMemsetAsync(g_dirs, 0, (size_t)M * 3 * sizeof(float), s);   // rows the kernels do not visit (>= *n_valid)
+    cudaMemsetAsync(workspace, 0, need, s);   // slots of CTAs without a tile stay zero
+    float* slots = static_cast<float*>(workspace);
+    const int rc = mlp_backward(dims, packed, feat, feat_fp16, dirs, M, n_valid, g_sigma, g_rgb, g_feat, g_W1, g_W2, g_W3, g_W4, g_W5,
+                                g_dirs, slots, stream);
+    if (rc != 0) return rc;
+    const WgradSlot L = wgrad_slot(dims->in_dim, dims->hidden);
+    k_wgrad_reduce<<<(unsigned)min(ceil_div(L.size, (size_t)256), (size_t)kNumSM * 4), 256, 0, s>>>(
+        slots, mlp_det_slots(dims, feat_fp16, M), L, g_W1, g_W2, g_W3, g_W4, g_W5);
+    return finish_launch("mlp_backward_det");
 }
 
 

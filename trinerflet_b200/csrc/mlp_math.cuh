@@ -2,6 +2,7 @@
 // the autocast rounding, SH degree 4 (shencoder.cu:50-68 of the reference), sigmoid.
 #pragma once
 #include <cuda_fp16.h>
+#include <stddef.h>
 #include <stdint.h>
 
 namespace tnl {
@@ -76,5 +77,21 @@ __device__ __forceinline__ void sh_backward(float x, float y, float z, const flo
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
 __device__ __forceinline__ float r16(float v) { return __half2float(__float2half_rn(v)); }
+
+// Weight-gradient flush of the backward kernels.  Default: one fp32 atomicAdd per element per CTA (the sum depends on the CTA
+// order).  DET (tnl_mlp_backward_det): the CTA writes its partial sums to its own slot of a workspace instead, and
+// k_wgrad_reduce adds the slots in index order.  A slot holds g_W1 | g_W2 | g_W3 | g_W4 | g_W5 (fp32, their shapes).
+struct WgradSlot {
+    size_t o2, o3, o4, o5, size;   // offsets of g_W2 .. g_W5 and the slot size, in floats
+};
+__host__ __device__ constexpr WgradSlot wgrad_slot(uint32_t K1, uint32_t H) {
+    return WgradSlot{(size_t)H * K1, (size_t)H * K1 + 16 * H, (size_t)H * K1 + 16 * H + 31 * H, (size_t)H * K1 + 47 * H + (size_t)H * H,
+                     (size_t)H * K1 + 50 * H + (size_t)H * H};
+}
+template <bool DET>
+__device__ __forceinline__ void wgrad_add(float* p, float v) {
+    if constexpr (DET) *p = v;
+    else atomicAdd(p, v);
+}
 
 }  // namespace tnl

@@ -257,7 +257,7 @@ __device__ __forceinline__ void red_add_v4(float* addr, float4 v, float w) {   /
 
 // DIRS variant: stage 7 takes d(in3) over all 32 columns, and the point's thread applies the SH Jacobian at its direction to the
 // fp16-rounded SH columns (0..15) -> g_dirs [M,3] (valid rows only).
-template <int K1, bool SCATTER, bool DIRS>
+template <int K1, bool SCATTER, bool DIRS, bool DET = false>
 __global__ void __launch_bounds__(544, 1)
 k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
              const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
@@ -564,6 +564,10 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
     if (profiling && tid < 64) dbg[tid] += sdbg[tid];
     // ---------------- flush the weight gradients (fp32, one atomicAdd per element per CTA) ----------------
     if (warp < 4 && my_pairs > 0) {
+        if constexpr (DET) {   // this CTA's slot of the workspace (wgrad_add)
+            const size_t o = (size_t)blockIdx.x * wgrad_slot(K1, 64).size;
+            gW1 += o; gW2 += o; gW3 += o; gW4 += o; gW5 += o;
+        }
         const uint32_t tl = tmem + ((warp * 32u) << 16);
         uint32_t row;
         const bool have = m64_row_of_lane(warp, lane, row);
@@ -573,7 +577,7 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             tmem_load_row<16>(tl + TM_W1 + c0, a);
             if (have)
 #pragma unroll
-                for (int k = 0; k < 16; ++k) atomicAdd(gW1 + (size_t)row * K1 + c0 + k, a[k]);
+                for (int k = 0; k < 16; ++k) wgrad_add<DET>(gW1 + (size_t)row * K1 + c0 + k, a[k]);
         }
 #pragma unroll 1
         for (int c0 = 0; c0 < 64; c0 += 16) {
@@ -581,26 +585,26 @@ k_mlp_tc_bwd(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, c
             tmem_load_row<16>(tl + TM_W4 + c0, a);
             if (have)
 #pragma unroll
-                for (int k = 0; k < 16; ++k) atomicAdd(gW4 + (size_t)row * 64 + c0 + k, a[k]);
+                for (int k = 0; k < 16; ++k) wgrad_add<DET>(gW4 + (size_t)row * 64 + c0 + k, a[k]);
         }
         {
             float a[32];
             tmem_load_row<32>(tl + TM_W3, a);
             if (have)
 #pragma unroll
-                for (int k = 0; k < 31; ++k) atomicAdd(gW3 + (size_t)row * 31 + k, a[k]);
+                for (int k = 0; k < 31; ++k) wgrad_add<DET>(gW3 + (size_t)row * 31 + k, a[k]);
         }
         {   // transposed accumulators: lane row = input feature k, column = output row n
             float a[16];
             tmem_load_row<16>(tl + TM_W2, a);
             if (have)
 #pragma unroll
-                for (int n = 0; n < 16; ++n) atomicAdd(gW2 + (size_t)n * 64 + row, a[n]);
+                for (int n = 0; n < 16; ++n) wgrad_add<DET>(gW2 + (size_t)n * 64 + row, a[n]);
             float b[16];
             tmem_load_row<16>(tl + TM_W5, b);
             if (have)
 #pragma unroll
-                for (int n = 0; n < 3; ++n) atomicAdd(gW5 + (size_t)n * 64 + row, b[n]);
+                for (int n = 0; n < 3; ++n) wgrad_add<DET>(gW5 + (size_t)n * 64 + row, b[n]);
         }
     }
     fence_before_sync();
@@ -773,14 +777,19 @@ void mlp_tc_forward(uint32_t in_dim, uint32_t hidden, const void* wpk, const voi
 // optional device buffer of 64 cycle counters (tnl_mlp_tc_profile); nullptr in normal operation
 static unsigned long long* g_tc_dbg = nullptr;
 
-template <int K1, bool SCATTER, bool DIRS>
+uint32_t mlp_tc_backward_blocks(uint32_t hidden, uint32_t M) {
+    // one CTA per SM: it owns all 512 TMEM columns; a CTA of the 64-wide kernel takes two 128-point tiles at a time
+    return min(ceil_div(M, hidden == 128 ? 128u : 256u), (uint32_t)kNumSM);
+}
+
+template <int K1, bool SCATTER, bool DIRS, bool DET = false>
 static void launch_bwd(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
                        const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, const PlaneScatter& sc,
                        float* g_dirs, cudaStream_t s) {
     using S = TcBwdSmem<K1>;
-    cudaFuncSetAttribute(k_mlp_tc_bwd<K1, SCATTER, DIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
-    const uint32_t blocks = min(ceil_div(M, 256u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
-    k_mlp_tc_bwd<K1, SCATTER, DIRS><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M,
+    cudaFuncSetAttribute(k_mlp_tc_bwd<K1, SCATTER, DIRS, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
+    const uint32_t blocks = mlp_tc_backward_blocks(64, M);
+    k_mlp_tc_bwd<K1, SCATTER, DIRS, DET><<<blocks, 544, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M,
                                                                   n_valid, g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4,
                                                                   gW5, g_tc_dbg, sc, g_dirs);
 }
@@ -807,6 +816,25 @@ void mlp_tc_backward_dirs(uint32_t in_dim, uint32_t hidden, const void* wpk, con
     const PlaneScatter none{};
     if (in_dim == 48) launch_bwd<48, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, g_dirs, s);
     else launch_bwd<96, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, none, g_dirs, s);
+}
+
+void mlp_tc_backward_det(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
+                         const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* slots, float* g_dirs,
+                         cudaStream_t s) {
+    if (hidden == 128) {
+        mlp_tc128_backward_det(in_dim, wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, slots, g_dirs, s);
+        return;
+    }
+    const PlaneScatter none{};
+    const WgradSlot L = wgrad_slot(in_dim, 64);
+    float *w1 = slots, *w2 = slots + L.o2, *w3 = slots + L.o3, *w4 = slots + L.o4, *w5 = slots + L.o5;
+    if (in_dim == 48) {
+        if (g_dirs) launch_bwd<48, false, true, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, none, g_dirs, s);
+        else launch_bwd<48, false, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, none, nullptr, s);
+    } else {
+        if (g_dirs) launch_bwd<96, false, true, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, none, g_dirs, s);
+        else launch_bwd<96, false, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, none, nullptr, s);
+    }
 }
 
 }  // namespace tnl

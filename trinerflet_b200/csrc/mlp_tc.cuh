@@ -21,6 +21,13 @@ void mlp_tc_backward(uint32_t in_dim, uint32_t hidden, const void* wpk, const vo
 void mlp_tc_backward_dirs(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
                           const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2,
                           float* gW3, float* gW4, float* gW5, float* g_dirs, cudaStream_t s);
+// the same with the weight gradients written per CTA into `slots` (layout wgrad_slot, one slot per CTA, mlp_tc_backward_blocks
+// of them; tnl_mlp_backward_det reduces them); g_dirs may be nullptr
+void mlp_tc_backward_det(uint32_t in_dim, uint32_t hidden, const void* wpk, const void* feat, const float* dirs, uint32_t M,
+                         const int32_t* n_valid, const float* g_sigma, const float* g_rgb, void* g_feat, float* slots, float* g_dirs,
+                         cudaStream_t s);
+// CTAs of the tcgen05 backward kernels for M points
+uint32_t mlp_tc_backward_blocks(uint32_t hidden, uint32_t M);
 // mlp.cu: where the tcgen05 tiles start inside the packed weight block, and whether the tcgen05 kernels serve these dims
 // (fp16 feature stream, not forced off by TNL_MLP_LEGACY)
 size_t mlp_tc_packed_offset(const tnl_mlp_dims* dims);
@@ -31,5 +38,7 @@ void mlp_tc128_forward(uint32_t in_dim, const void* wpk, const void* feat, const
 void mlp_tc128_backward(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
                         const float* g_sigma, const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, float* g_dirs,
                         cudaStream_t s);
+void mlp_tc128_backward_det(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
+                            const float* g_sigma, const float* g_rgb, void* g_feat, float* slots, float* g_dirs, cudaStream_t s);
 
 }  // namespace tnl

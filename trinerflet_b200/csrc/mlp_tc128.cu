@@ -262,7 +262,7 @@ __device__ __forceinline__ void load_x_half_async(uint8_t* xtile, uint32_t t, ui
 
 // DIRS: d(in3) over all 32 columns, and g_dirs [M,3] <- the SH Jacobian at the point's direction applied to the fp16-rounded
 // SH columns 0..15 (valid rows only)
-template <int K1, bool DIRS>
+template <int K1, bool DIRS, bool DET = false>
 __global__ void __launch_bounds__(256, 1)
 k_mlp_tc_bwd128(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat, const float* __restrict__ dirs, uint32_t M,
                 const int32_t* __restrict__ n_valid_ptr, const float* __restrict__ g_sigma, const float* __restrict__ g_rgb,
@@ -458,35 +458,39 @@ k_mlp_tc_bwd128(const uint8_t* __restrict__ wpk, const __half* __restrict__ feat
     fence_after_sync();
     // ---------------- flush the weight gradients (fp32, one atomicAdd per element per CTA): TMEM lane = row ----------------
     if (my_tiles > 0) {
+        if constexpr (DET) {   // this CTA's slot of the workspace (wgrad_add)
+            const size_t o = (size_t)blockIdx.x * wgrad_slot(K1, 128).size;
+            gW1 += o; gW2 += o; gW3 += o; gW4 += o; gW5 += o;
+        }
         const uint32_t row = t;
         {
             float a[KH];
             tmem_load_row<KH>(tlane + TM_W1 + hf * KH, a);
 #pragma unroll
-            for (int k = 0; k < KH; ++k) atomicAdd(gW1 + (size_t)row * K1 + hf * KH + k, a[k]);
+            for (int k = 0; k < KH; ++k) wgrad_add<DET>(gW1 + (size_t)row * K1 + hf * KH + k, a[k]);
         }
         {
             float a[64];
             tmem_load_row<64>(tlane + TM_W4 + hf * 64u, a);
 #pragma unroll
-            for (int k = 0; k < 64; ++k) atomicAdd(gW4 + (size_t)row * 128 + hf * 64 + k, a[k]);
+            for (int k = 0; k < 64; ++k) wgrad_add<DET>(gW4 + (size_t)row * 128 + hf * 64 + k, a[k]);
         }
         {
             float a[16];
             tmem_load_row<16>(tlane + TM_W3 + hf * 16u, a);
 #pragma unroll
             for (int k = 0; k < 16; ++k)
-                if (hf * 16 + k < 31) atomicAdd(gW3 + (size_t)row * 31 + hf * 16 + k, a[k]);
+                if (hf * 16 + k < 31) wgrad_add<DET>(gW3 + (size_t)row * 31 + hf * 16 + k, a[k]);
         }
         {   // transposed accumulators: lane row = input feature k, column = output row n; half 0 flushes dW2, half 1 dW5
             float a[16];
             tmem_load_row<16>(tlane + (hf == 0 ? TM_W2 : TM_W5), a);
             if (hf == 0) {
 #pragma unroll
-                for (int n = 0; n < 16; ++n) atomicAdd(gW2 + (size_t)n * 128 + row, a[n]);
+                for (int n = 0; n < 16; ++n) wgrad_add<DET>(gW2 + (size_t)n * 128 + row, a[n]);
             } else {
 #pragma unroll
-                for (int n = 0; n < 3; ++n) atomicAdd(gW5 + (size_t)n * 128 + row, a[n]);
+                for (int n = 0; n < 3; ++n) wgrad_add<DET>(gW5 + (size_t)n * 128 + row, a[n]);
             }
         }
     }
@@ -523,14 +527,14 @@ void mlp_tc128_forward(uint32_t in_dim, const void* wpk, const void* feat, const
     else launch_fwd128<144>(wpk, feat, dirs, M, n_valid, sigma, rgb, geo, s);
 }
 
-template <int K1, bool DIRS>
+template <int K1, bool DIRS, bool DET = false>
 static void launch_bwd128(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
                           const float* g_rgb, void* g_feat, float* gW1, float* gW2, float* gW3, float* gW4, float* gW5, float* g_dirs,
                           cudaStream_t s) {
     using S = TcBwd128Smem<K1>;
-    cudaFuncSetAttribute(k_mlp_tc_bwd128<K1, DIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
-    const uint32_t blocks = min(ceil_div(M, 128u), (uint32_t)kNumSM);   // one CTA per SM: it owns all 512 TMEM columns
-    k_mlp_tc_bwd128<K1, DIRS><<<blocks, 256, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M, n_valid,
+    cudaFuncSetAttribute(k_mlp_tc_bwd128<K1, DIRS, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL);
+    const uint32_t blocks = mlp_tc_backward_blocks(128, M);
+    k_mlp_tc_bwd128<K1, DIRS, DET><<<blocks, 256, S::TOTAL, s>>>(static_cast<const uint8_t*>(wpk), static_cast<const __half*>(feat), dirs, M, n_valid,
                                                             g_sigma, g_rgb, static_cast<__half*>(g_feat), gW1, gW2, gW3, gW4, gW5, g_dirs);
 }
 
@@ -548,6 +552,22 @@ void mlp_tc128_backward(uint32_t in_dim, const void* wpk, const void* feat, cons
     if (in_dim == 48) launch_bwd128<48>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
     else if (in_dim == 96) launch_bwd128<96>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
     else launch_bwd128<144>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, gW1, gW2, gW3, gW4, gW5, g_dirs, s);
+}
+
+template <int K1>
+static void launch_bwd128_det(const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid, const float* g_sigma,
+                              const float* g_rgb, void* g_feat, float* slots, float* g_dirs, cudaStream_t s) {
+    const WgradSlot L = wgrad_slot(K1, 128);
+    float *w1 = slots, *w2 = slots + L.o2, *w3 = slots + L.o3, *w4 = slots + L.o4, *w5 = slots + L.o5;
+    if (g_dirs) launch_bwd128<K1, true, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, g_dirs, s);
+    else launch_bwd128<K1, false, true>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, w1, w2, w3, w4, w5, nullptr, s);
+}
+
+void mlp_tc128_backward_det(uint32_t in_dim, const void* wpk, const void* feat, const float* dirs, uint32_t M, const int32_t* n_valid,
+                            const float* g_sigma, const float* g_rgb, void* g_feat, float* slots, float* g_dirs, cudaStream_t s) {
+    if (in_dim == 48) launch_bwd128_det<48>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, slots, g_dirs, s);
+    else if (in_dim == 96) launch_bwd128_det<96>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, slots, g_dirs, s);
+    else launch_bwd128_det<144>(wpk, feat, dirs, M, n_valid, g_sigma, g_rgb, g_feat, slots, g_dirs, s);
 }
 
 }  // namespace tnl

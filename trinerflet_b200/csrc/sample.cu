@@ -344,6 +344,115 @@ k_sample_xyz_grad_nerf(const void* __restrict__ g_feat_, const float* __restrict
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Deterministic scatter (torch.use_deterministic_algorithms): the same contributions c = g * w as k_sample_bwd4, added in
+// 64-bit fixed point.  Integer addition is associative, so the sums do not depend on the visiting order (perm) or on the
+// thread schedule.  Scale: m = max |g_feat| over the rows below *n_valid, 2^e > m, mu = ceil(log2 M), unit = 2^(e + mu - 62).
+// Every bilinear weight is <= 1, so |c| <= m < 2^e, and a texel of one plane receives at most M contributions: no partial sum
+// reaches 2^62 units.  Each contribution is rounded once to a multiple of the unit (error <= unit / 2), the texel's sum is
+// rounded once to fp32.  A non-finite g_feat row turns the whole converted gradient into NaN, so that loss scaling skips the
+// step as it does with the fp32 atomics.
+// ------------------------------------------------------------------------------------------------
+struct DetScale {
+    int state;          // 0: every contribution is zero, 1: finite, 2: some g_feat value is inf or NaN
+    double to_fixed;    // 2^(62 - e - mu)
+    float unit;         // 2^(e + mu - 62)
+};
+
+__device__ __forceinline__ DetScale det_scale(uint32_t absmax_bits, uint32_t M) {
+    DetScale s{0, 0.0, 0.f};
+    if (absmax_bits == 0u) return s;
+    if (absmax_bits >= 0x7f800000u) { s.state = 2; return s; }
+    int e;
+    frexpf(__uint_as_float(absmax_bits), &e);                 // m = f 2^e, f in [0.5, 1): 2^e > m
+    const int mu = M > 1u ? 32 - __clz((int)(M - 1u)) : 0;     // 2^mu >= M
+    s.state = 1;
+    s.to_fixed = ldexp(1.0, 62 - e - mu);
+    s.unit = ldexpf(1.f, e + mu - 62);
+    return s;
+}
+
+// max |g_feat| over rows [0, min(*n_valid, M)) as the bit pattern of a non-negative float (order-free atomicMax; NaN > inf)
+template <bool HALF>
+__global__ void __launch_bounds__(256)
+k_det_absmax(const void* __restrict__ g_feat_, uint32_t M, int C, const int32_t* __restrict__ n_valid, uint32_t* __restrict__ absmax) {
+    uint32_t rows = M;
+    if (n_valid) rows = *n_valid < 0 ? 0u : min((uint32_t)*n_valid, M);
+    const size_t n4 = (size_t)rows * 3 * C / 4;
+    uint32_t mx = 0u;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
+        const float4 g = HALF ? unpack4h(__ldg(reinterpret_cast<const uint2*>(g_feat_) + i)) : __ldg(reinterpret_cast<const float4*>(g_feat_) + i);
+        mx = max(mx, max(max(__float_as_uint(fabsf(g.x)), __float_as_uint(fabsf(g.y))), max(__float_as_uint(fabsf(g.z)), __float_as_uint(fabsf(g.w)))));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    if ((threadIdx.x & 31) == 0 && mx != 0u) atomicMax(absmax, mx);
+}
+
+__device__ __forceinline__ void red_add_fixed(unsigned long long* addr, float4 v, float w, double to_fixed) {
+    atomicAdd(addr, (unsigned long long)llrint((double)(v.x * w) * to_fixed));
+    atomicAdd(addr + 1, (unsigned long long)llrint((double)(v.y * w) * to_fixed));
+    atomicAdd(addr + 2, (unsigned long long)llrint((double)(v.z * w) * to_fixed));
+    atomicAdd(addr + 3, (unsigned long long)llrint((double)(v.w * w) * to_fixed));
+}
+
+// thread <-> (point, plane, 4-channel group) as in k_sample_bwd4; TPP4 = C / 4, or 0 for a run-time C
+template <int TPP4, bool HALF>
+__global__ void __launch_bounds__(256)
+k_sample_bwd_det(const void* __restrict__ g_feat_, const float* __restrict__ xyz, uint32_t M, int R, int C_rt, float inv_bound,
+                 int fp16_coords, const int32_t* __restrict__ n_valid, const int32_t* __restrict__ perm,
+                 const uint32_t* __restrict__ absmax, unsigned long long* __restrict__ acc) {
+    const int C = TPP4 ? 4 * TPP4 : C_rt, cq_per = C >> 2;
+    const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (uint64_t)M * 3 * cq_per) return;
+    const DetScale sc = det_scale(*absmax, M);
+    if (sc.state != 1) return;
+    const int cq = (int)(idx % cq_per);
+    const int p = (int)((idx / cq_per) % 3);
+    uint32_t m = (uint32_t)(idx / ((uint64_t)3 * cq_per));
+    if (perm) m = (uint32_t)__ldg(perm + m);
+    if (n_valid && (int32_t)m >= *n_valid) return;
+    const size_t q4 = ((size_t)m * 3 + p) * cq_per + cq;
+    const float4 g = HALF ? unpack4h(__ldg(reinterpret_cast<const uint2*>(g_feat_) + q4))
+                          : __ldg(reinterpret_cast<const float4*>(g_feat_) + q4);
+    if (g.x == 0.f && g.y == 0.f && g.z == 0.f && g.w == 0.f) return;  // adding zeros is a no-op
+    float gx, gy;
+    plane_coords(xyz, m, p, inv_bound, fp16_coords, gx, gy);
+    const Tap t = make_tap(gx, gy, R);
+    unsigned long long* base = acc + (((size_t)p * R + t.y0) * R + t.x0) * C + 4 * cq;
+    const size_t dx = (size_t)C, dy = (size_t)R * C;
+    red_add_fixed(base, g, t.nw, sc.to_fixed);
+    if (t.x1ok) red_add_fixed(base + dx, g, t.ne, sc.to_fixed);
+    if (t.y1ok) red_add_fixed(base + dy, g, t.sw, sc.to_fixed);
+    if (t.x1ok && t.y1ok) red_add_fixed(base + dy + dx, g, t.se, sc.to_fixed);
+}
+
+// g_planes += acc * unit (one rounding: the int64 -> fp32 conversion; the unit is a power of two) over the listed T x T tiles of
+// [3][R][R][C] (ids / *count as tnl_tiles_zero), or over the whole planes when ids == nullptr
+__global__ void __launch_bounds__(256)
+k_det_convert(const unsigned long long* __restrict__ acc, float* __restrict__ g_planes, const int32_t* __restrict__ ids,
+              const int32_t* __restrict__ count, int R, int C, int T, const uint32_t* __restrict__ absmax, uint32_t M) {
+    const DetScale sc = det_scale(*absmax, M);
+    if (sc.state == 0) return;
+    const float nan = __uint_as_float(0x7fffffffu);
+    if (ids == nullptr) {
+        const size_t n = (size_t)3 * R * R * C;
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+            g_planes[i] = sc.state == 2 ? nan : g_planes[i] + (float)(long long)acc[i] * sc.unit;
+        return;
+    }
+    if ((int)blockIdx.x >= __ldg(count)) return;
+    const int id = __ldg(ids + blockIdx.x), nt = R / T;
+    const int p = id / (nt * nt), ty = (id / nt) % nt, tx = id % nt;
+    const int rows_per_cta = (T + gridDim.y - 1) / gridDim.y;
+    const int row_end = min(T, (int)(blockIdx.y + 1) * rows_per_cta);
+    for (int row = blockIdx.y * rows_per_cta; row < row_end; ++row) {
+        const size_t o = (((size_t)p * R + (size_t)ty * T + row) * R + (size_t)tx * T) * C;
+        for (int i = threadIdx.x; i < T * C; i += blockDim.x)
+            g_planes[o + i] = sc.state == 2 ? nan : g_planes[o + i] + (float)(long long)acc[o + i] * sc.unit;
+    }
+}
+
 template <int TPP>
 static void launch_fwd8(const float* planes, const float* xyz, uint32_t M, uint32_t R, float inv_bound, int fp16_coords,
                         const int32_t* n_valid, const int32_t* perm, void* feat, int half, cudaStream_t s) {
@@ -436,6 +545,59 @@ int tnl_sample_planes_backward_plane(const void* g_feat, int feat_fp16, const fl
     else if (C == 32) launch_bwd4_plane<8>(g_feat, feat_fp16, xyz, M, R, inv_bound, fp16_coords, n_valid, perm, g_planes, (int)plane, st);
     else launch_bwd4_plane<12>(g_feat, feat_fp16, xyz, M, R, inv_bound, fp16_coords, n_valid, perm, g_planes, (int)plane, st);
     return finish_launch("sample_planes_backward_plane");
+}
+
+size_t tnl_sample_planes_backward_det_workspace(uint32_t R, uint32_t C) {
+    return 256 + (size_t)3 * R * R * C * sizeof(unsigned long long);
+}
+
+int tnl_sample_planes_backward_det(const void* g_feat, int feat_fp16, const float* xyz, uint32_t M, uint32_t R, uint32_t C,
+                                   float inv_bound, int fp16_coords, const int32_t* n_valid, const int32_t* perm,
+                                   const int32_t* tile_ids, const int32_t* tile_count, uint32_t tile_capacity, uint32_t T,
+                                   float* g_planes, void* workspace, size_t workspace_bytes, tnl_stream_t stream) {
+    if (M == 0) return 0;
+    TNL_ARG_CHECK(g_feat && xyz && g_planes && workspace, "null pointer");
+    TNL_ARG_CHECK(C >= 4 && C % 4 == 0 && R >= 2, "C must be a multiple of 4, R >= 2");
+    TNL_ARG_CHECK(((uintptr_t)g_planes & 15) == 0 && ((uintptr_t)g_feat & (feat_fp16 ? 7 : 15)) == 0 && ((uintptr_t)workspace & 255) == 0,
+                  "g_planes must be 16-byte aligned, g_feat 8 (fp16) or 16 (fp32), the workspace 256");
+    TNL_ARG_CHECK(workspace_bytes >= tnl_sample_planes_backward_det_workspace(R, C), "workspace too small");
+    TNL_ARG_CHECK(tile_ids == nullptr || (tile_count != nullptr && T > 0 && R % T == 0), "tile list: count and a tile edge dividing R");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    uint32_t* absmax = static_cast<uint32_t*>(workspace);
+    unsigned long long* acc = reinterpret_cast<unsigned long long*>(static_cast<uint8_t*>(workspace) + 256);
+    cudaMemsetAsync(absmax, 0, sizeof(uint32_t), st);
+    if (tile_ids) {
+        // the int64 accumulator viewed as fp32 planes of 2C channels: the same tiles, zeroed by the same kernel
+        if (tile_capacity > 0) {
+            const int rc = tnl_tiles_zero(reinterpret_cast<float*>(acc), tile_ids, tile_count, tile_capacity, R, 2 * C, T, stream);
+            if (rc != 0) return rc;
+        }
+    } else {
+        cudaMemsetAsync(acc, 0, (size_t)3 * R * R * C * sizeof(unsigned long long), st);
+    }
+    const uint32_t absmax_blocks = (uint32_t)min(ceil_div((uint64_t)M * 3 * C / 4, (uint64_t)256), (uint64_t)kNumSM * 8);
+    if (feat_fp16) k_det_absmax<true><<<absmax_blocks, 256, 0, st>>>(g_feat, M, (int)C, n_valid, absmax);
+    else k_det_absmax<false><<<absmax_blocks, 256, 0, st>>>(g_feat, M, (int)C, n_valid, absmax);
+    const unsigned blocks = (unsigned)ceil_div((uint64_t)M * 3 * (C / 4), (uint64_t)256);
+#define TNL_DET_SCATTER(TPP4)                                                                                                       \
+    do {                                                                                                                            \
+        if (feat_fp16) k_sample_bwd_det<TPP4, true><<<blocks, 256, 0, st>>>(g_feat, xyz, M, (int)R, (int)C, inv_bound, fp16_coords, \
+                                                                            n_valid, perm, absmax, acc);                            \
+        else k_sample_bwd_det<TPP4, false><<<blocks, 256, 0, st>>>(g_feat, xyz, M, (int)R, (int)C, inv_bound, fp16_coords, n_valid, \
+                                                                   perm, absmax, acc);                                              \
+    } while (0)
+    if (C == 16) TNL_DET_SCATTER(4);
+    else if (C == 32) TNL_DET_SCATTER(8);
+    else if (C == 48) TNL_DET_SCATTER(12);
+    else TNL_DET_SCATTER(0);
+#undef TNL_DET_SCATTER
+    if (tile_ids) {
+        if (tile_capacity > 0)
+            k_det_convert<<<dim3(tile_capacity, 4), 256, 0, st>>>(acc, g_planes, tile_ids, tile_count, (int)R, (int)C, (int)T, absmax, M);
+    } else {
+        k_det_convert<<<kNumSM * 8, 256, 0, st>>>(acc, g_planes, nullptr, nullptr, (int)R, (int)C, 1, absmax, M);
+    }
+    return finish_launch("sample_planes_backward_det");
 }
 
 int tnl_sample_planes_backward_coords(const float* g_feat, const float* planes, const float* xyz, uint32_t M, uint32_t R,

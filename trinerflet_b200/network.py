@@ -104,10 +104,17 @@ class _FieldMLP(Function):
         g_dirs = None
         if ctx.needs_input_grad[1]:
             g_dirs = torch.empty(M, 3, device=feat.device, dtype=torch.float32)
+        if _lib.deterministic():
+            # the same kernels with the weight gradients reduced over per-CTA slots in a fixed order
+            nbytes = _lib.load().tnl_mlp_backward_det_workspace(ctypes.byref(dims), int(feat.dtype == torch.float16), M)
+            ws = _lib.workspace("mlp_backward_det", nbytes, feat.device)
+            call("tnl_mlp_backward_det", *args, ptr(g_dirs), ptr(ws), ws.numel(), stream())
+        elif g_dirs is not None:
             call("tnl_mlp_backward_dirs", *args, ptr(g_dirs), stream())
-            g_dirs = g_dirs.to(ctx.dirs_dtype)
         else:
             call("tnl_mlp_backward", *args, stream())
+        if g_dirs is not None:
+            g_dirs = g_dirs.to(ctx.dirs_dtype)
         # (rows >= *n_valid of g_feat are never read: the sampling backward skips them with the same counter)
         if g_feat.dtype != ctx.in_dtype:
             g_feat = g_feat.to(ctx.in_dtype)
@@ -217,9 +224,11 @@ class NeRFNetwork(NeRFRenderer):
             perm = cell_sort(x, self.bound, n_valid, 64)
         fused = self._fused()
         if (fused and perm is not None and self.hidden_dim == 64 and self.in_dim in (48, 96)
-                and self.encoder.scatter_plane_hook is None and not x.requires_grad and not d.requires_grad):
+                and self.encoder.scatter_plane_hook is None and not x.requires_grad and not d.requires_grad
+                and not _lib.deterministic()):
             # training step: one fused MLP-backward + plane scatter (the plane-by-plane exchange of the multi-GPU step scatters
-            # through _SamplePlanes instead; input gradients go through _SamplePlanes / _FieldMLP)
+            # through _SamplePlanes instead; input gradients go through _SamplePlanes / _FieldMLP; deterministic mode takes
+            # _SamplePlanes + _FieldMLP, whose results per row do not depend on perm)
             planes, gbuf = self.encoder.planes_and_grad_buffer()
             return _Field.apply(planes, x, d, self.bound, n_valid, perm, gbuf, *self._weights())
         # fused path: the feature stream between the gather and the MLP kernels is fp16 (the first Linear's own rounding)

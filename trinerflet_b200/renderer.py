@@ -12,7 +12,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from . import raymarching
+from . import _lib, raymarching
 from ._lib import call, ptr, stream
 
 
@@ -213,7 +213,12 @@ class NeRFRenderer(nn.Module):
         xyz = torch.empty(n, 3, device=idx32.device, dtype=torch.float32)
         call("tnl_grid_cell_positions", ptr(idx32), n, H, float(bound_c), ptr(noise), ptr(xyz), stream())
         sigmas = self.density(xyz)['sigma'].reshape(-1).detach().float().contiguous()
-        call("tnl_grid_scatter", ptr(idx32), ptr(sigmas), n, float(self.density_scale), ptr(tmp_grid[cas]), stream())
+        if _lib.deterministic():
+            # duplicate cells of the partial sweep: torch's deterministic index_put_, the reference's own statement
+            # (tmp_grid[cas, indices] = sigmas), instead of the kernel where one of the writers wins
+            tmp_grid[cas].index_put_((idx32.long(),), sigmas * float(self.density_scale))
+        else:
+            call("tnl_grid_scatter", ptr(idx32), ptr(sigmas), n, float(self.density_scale), ptr(tmp_grid[cas]), stream())
 
     @property
     def mean_density(self):
@@ -275,6 +280,8 @@ class NeRFRenderer(nn.Module):
         acc = torch.empty(1, dtype=torch.float64, device=dev)
         mean_t = torch.empty(1, dtype=torch.float32, device=dev)
         call("tnl_grid_ema_update_sum", ptr(flat), ptr(tmp_grid.view(-1)), flat.numel(), float(decay), ptr(acc), stream())
+        if _lib.deterministic():   # the kernel's sum adds one double atomic per block: torch's deterministic reduction instead
+            acc.copy_(torch.clamp(flat, min=0).sum(dtype=torch.float64).reshape(1))
         self.iter_density += 1
         call("tnl_packbits_mean", ptr(flat), flat.numel(), ptr(acc), float(self.density_thresh), ptr(mean_t), ptr(self.density_bitfield),
              stream())

@@ -59,7 +59,7 @@ class _SamplePlanesXyz(Function):
         g_planes = g_xyz = None
         if ctx.needs_input_grad[0]:
             g_planes = cl_empty_planes(C, R, device=g_feat.device, zero=True)
-            call("tnl_sample_planes_backward", ptr(g_feat), 0, ptr(xyz), M, R, C, inv, 0, None, None, ptr(g_planes), stream())
+            _te.scatter_planes(g_feat, False, xyz, M, R, C, inv, 0, None, None, g_planes)
         if ctx.needs_input_grad[1]:
             g_xyz = torch.empty(M, 3, device=g_feat.device, dtype=torch.float32)
             call("tnl_sample_planes_backward_coords", ptr(g_feat), ptr(planes_cl), ptr(xyz), M, R, C, inv, 0, ptr(g_xyz), stream())
@@ -95,7 +95,7 @@ class _SampleHighOrderBackward(Function):
         g_planes = g_xyz = None
         if need_planes:
             g_planes = cl_empty_planes(C, R, device=g_feat.device, zero=True)
-            call("tnl_sample_planes_backward", ptr(g_feat), 0, ptr(xyz), M, R, C, inv, 0, None, None, ptr(g_planes), stream())
+            _te.scatter_planes(g_feat, False, xyz, M, R, C, inv, 0, None, None, g_planes)
         if need_xyz:
             g_xyz = torch.empty(M, 3, device=g_feat.device, dtype=torch.float32)
             call("tnl_sample_planes_backward_coords", ptr(g_feat), ptr(planes_cl), ptr(xyz), M, R, C, inv, 0, ptr(g_xyz), stream())

@@ -15,7 +15,7 @@ from types import SimpleNamespace
 
 import torch
 
-from . import parallel
+from . import _lib, parallel
 
 
 def default_opt(**over):
@@ -42,6 +42,8 @@ def wavelet_regulariser(encoder, lam, fused=True):
 class TrainStep:
     def __init__(self, model, opt=None, optimizer=None, world_size=1, sparse_allreduce=True, check_sparse=False,
                  transport=torch.bfloat16, exchange="auto"):
+        if world_size > 1:   # before any distributed call
+            _lib.alert_nondeterministic("a multi-GPU TrainStep (world_size > 1)")
         self.model = model
         self.opt = opt or default_opt()
         self.optimizer = optimizer
@@ -136,7 +138,8 @@ class TrainStep:
         self._split = None
         if will_split:
             self._split = self._make_split(enc, opt)
-            self._split.abs_sums = abs_sums          # completed by the clean part (the forward skipped those blocks)
+            # completed by the clean part (the forward skipped those blocks); deterministic mode: complete already (torch sums)
+            self._split.abs_sums = None if _lib.deterministic() else abs_sums
             # its gradient-independent ("clean") part runs on the side stream: single GPU / NCCL exchange -> right away, under the
             # render; peer exchange -> later, under the exchange (link-bound, few SMs busy), see below
             # (measured at 8 x B200: 6.24 ms with the clean part under the exchange vs 6.33 ms with it under the render;

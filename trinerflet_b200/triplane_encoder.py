@@ -23,6 +23,7 @@ import torch
 import torch.nn as nn
 from torch.autograd import Function
 
+from . import _lib
 from ._lib import call, ptr, stream
 from .idwt_plan import idwt_call
 
@@ -104,6 +105,8 @@ class _BuildPlanes(Function):
             raise RuntimeError("IdwtPlan does not match the encoder geometry")
         ctx.plan, ctx.wave = plan, wave
         ctx.set_materialize_grads(False)   # an unused abs_sums output must not cost a pass over the coefficients
+        # deterministic mode: the kernels' per-CTA atomic |yh| sums are replaced by torch's deterministic reductions (below)
+        det = _lib.deterministic()
         abs_sums = torch.zeros(max(len(coefs), 1), device=x.device, dtype=torch.float32)
         saved = []
         for l, yh in enumerate(coefs):
@@ -113,22 +116,25 @@ class _BuildPlanes(Function):
             yh = to_cl_coefs(yh.detach())
             saved.append(yh)
             out = cl_empty_planes(C, 2 * n, device=x.device)
+            a = None if det else abs_sums[l:l + 1]
             if plan is None:
-                idwt_call("tnl_idwt_level_forward", wave, ptr(x), ptr(yh), ptr(out), n, C, ptr(abs_sums[l:l + 1]), stream())
+                idwt_call("tnl_idwt_level_forward", wave, ptr(x), ptr(yh), ptr(out), n, C, ptr(a), stream())
             else:
-                plan.forward_level(l, x, yh, out, n, abs_sums[l:l + 1], parts=1, wave=wave)
+                plan.forward_level(l, x, yh, out, n, a, parts=1, wave=wave)
             x, n = out, 2 * n
         if plan is not None:
             if plan.on_planes_ready is not None and plan.defer_clean_abs:
                 plan.on_planes_ready()               # the planes are complete and nothing else of this call is awaited
             plan.on_planes_ready = None
             n = ctx.n0
-            for l, yh in enumerate(saved):           # |yh| of the blocks that were not reconstructed (regulariser value)
+            for l, yh in enumerate(saved if not det else []):   # |yh| of the blocks that were not reconstructed (regulariser value)
                 if plan.defer_clean_abs:             # ... except those the backward's clean part will read anyway
                     plan.forward_gap_abs(l, yh, n, abs_sums[l:l + 1])
                 else:
                     plan.forward_level(l, saved[l], yh, saved[l], n, abs_sums[l:l + 1], parts=2, wave=wave)   # x / out untouched
                 n *= 2
+        if det and saved:
+            abs_sums = torch.stack([yh.abs().sum() for yh in saved])
         ctx.save_for_backward(*saved)
         return x, abs_sums
 
@@ -270,13 +276,29 @@ def gather_features(planes, coords, bound, fp16_coords, n_valid, perm, half_out)
 def take_grad_buffer(ctx, C, R, device):
     """-> (g_planes, external, plane_hook): where a sampling backward scatters.  The buffer of ctx.grad_buf (zero-filled ahead of
     time on the prefetch stream, TriPlaneVolume.prefetch_planes) is taken once, after the current stream waits for it; without
-    one a zero-filled channels-last buffer.  external: the caller owns the buffer and the backward returns no plane gradient."""
+    one a zero-filled channels-last buffer.  external: the caller owns the buffer and the backward returns no plane gradient.
+    Sets ctx.grad_tiles: the idwt_plan.IdwtPlan tile list of a buffer zeroed only there, else None."""
+    ctx.grad_tiles = None
     if ctx.grad_buf is None:
         return cl_empty_planes(C, R, device=device, zero=True), False, None
-    g_planes, ready, external, plane_hook = ctx.grad_buf
+    g_planes, ready, external, plane_hook, ctx.grad_tiles = ctx.grad_buf
     ctx.grad_buf = None
     torch.cuda.current_stream().wait_event(ready)
     return g_planes, external, plane_hook
+
+
+def scatter_planes(g_feat, half, coords, M, R, C, inv, fp16_coords, nv, pm, g_planes, tiles=None):
+    """g_planes += the adjoint of the plane gather (tnl_sample_planes_backward).  In deterministic mode the fixed-point scatter
+    tnl_sample_planes_backward_det, restricted to the tiles of `tiles` (an IdwtPlan.zero list) when given."""
+    if not _lib.deterministic():
+        call("tnl_sample_planes_backward", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm, ptr(g_planes), stream())
+        return
+    nbytes = _lib.load().tnl_sample_planes_backward_det_workspace(R, C)
+    ws = _lib.workspace("sample_planes_backward_det", nbytes, g_feat.device)
+    ids, count, cap = (ptr(tiles["ids"]), ptr(tiles["count"]), tiles["cap"]) if tiles is not None else (None, None, 0)
+    from .idwt_plan import TILE
+    call("tnl_sample_planes_backward_det", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm, ids, count, cap, TILE,
+         ptr(g_planes), ptr(ws), ws.numel(), stream())
 
 
 class _SamplePlanes(Function):
@@ -301,13 +323,13 @@ class _SamplePlanes(Function):
             g_planes, external, plane_hook = take_grad_buffer(ctx, C, R, g_feat.device)
             if plane_hook is not None and C in (16, 32, 48):
                 # multi-GPU step: plane by plane, so that the caller can start exchanging plane p while plane p + 1 scatters
+                _lib.alert_nondeterministic("the plane-by-plane scatter of the multi-GPU step (tnl_sample_planes_backward_plane)")
                 for p in range(3):
                     call("tnl_sample_planes_backward_plane", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm,
                          ptr(g_planes), p, stream())
                     plane_hook(p)
             else:
-                call("tnl_sample_planes_backward", ptr(g_feat), int(half), ptr(coords), M, R, C, inv, fp16_coords, nv, pm,
-                     ptr(g_planes), stream())
+                scatter_planes(g_feat, half, coords, M, R, C, inv, fp16_coords, nv, pm, g_planes, ctx.grad_tiles)
         g_xyz = None
         if ctx.needs_input_grad[1]:
             g_xyz = torch.empty(M, 3, device=g_feat.device, dtype=torch.float32)
@@ -484,7 +506,8 @@ class TriPlaneVolume(nn.Module):
                     gbuf = cl_empty_planes(self.number_of_features, self.plane_resolution, device=planes.device, zero=True)
                 gready = torch.cuda.Event()
                 gready.record(side)
-                gbuf = (gbuf, gready, ext is not None, self.scatter_plane_hook if ext is not None else None)
+                gbuf = (gbuf, gready, ext is not None, self.scatter_plane_hook if ext is not None else None,
+                        plan.zero if (plan is not None and partial_zero) else None)
         self._prefetch = (ready, gbuf)
         return planes
 
