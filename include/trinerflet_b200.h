@@ -410,6 +410,29 @@ int tnl_tiles_allreduce(void* multicast, const void* const* peers, const int32_t
 int tnl_flat_allreduce(void* multicast, const void* const* peers, uint32_t n_floats, uint32_t rank, uint32_t world,
                        float scale, tnl_stream_t stream);
 
+/* ------------------------------------------------------------------ mesh extraction ---------- */
+/* Marching cubes (replaces mcubes.marching_cubes in the reference's extract_geometry, nerf/utils.py) over a dense fp32 volume
+ * [nx][ny][nz] (C-contiguous, u[x, y, z]; nx, ny, nz >= 2; +-inf allowed, NaN rejected).  A lattice point is inside iff
+ * u >= threshold.  Case table: csrc/mc_tables.cuh (generated by csrc/gen_mc_tables.py; face-local, so no cracks between cubes).
+ * Outputs, in an order that does not depend on the thread schedule:
+ *   vertices  [V][3] float64, index space: one per lattice edge whose end values straddle the threshold, ordered by (linear
+ *             index of the edge's lower lattice point, axis x < y < z); position p + t e_axis with
+ *             t = (threshold - u_lower) / (u_upper - u_lower) in float64 (t = 1 if u_lower is infinite);
+ *   triangles [T][3] int64 vertex ids, ordered by (linear cube index, table order); normals (v1-v0)x(v2-v0) point from the
+ *             inside region to the outside one.
+ * Two calls on one stream and workspace:
+ *   tnl_mc_count  writes totals[2] (DEVICE int64) = (V, T), or (-1, -1) if the volume contains a NaN;
+ *   tnl_mc_emit   takes the host copy of those totals (the capacities of the caller's outputs) and fills the outputs; negative
+ *                 totals return TNL_ERR_INVALID_ARGUMENT.
+ * Workspace: tnl_mc_workspace bytes, about 2.01 bytes per lattice point (a uint16 per point plus 24 bytes per 2048 points);
+ * 2.0 GiB at 1024^3.  0 if an axis has fewer than 2 points. */
+size_t tnl_mc_workspace(uint32_t nx, uint32_t ny, uint32_t nz);
+int tnl_mc_count(const float* volume, uint32_t nx, uint32_t ny, uint32_t nz, double threshold, void* workspace,
+                 size_t workspace_bytes, int64_t* totals, tnl_stream_t stream);
+int tnl_mc_emit(const float* volume, uint32_t nx, uint32_t ny, uint32_t nz, double threshold, const void* workspace,
+                size_t workspace_bytes, int64_t n_vertices, int64_t n_triangles, double* vertices, int64_t* triangles,
+                tnl_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
