@@ -75,6 +75,23 @@ int tnl_march_rays_train(const float* rays_o, const float* rays_d, const uint8_t
                          const float* nears, const float* fars, float* xyzs, float* dirs, float* deltas,
                          int32_t* rays, int32_t* counter, const float* noises, void* workspace,
                          size_t workspace_bytes, tnl_stream_t stream);
+/* tnl_march_rays_train plus ts [M] (fp32, overwritten): the ray parameter t of every emitted row, so that
+ * xyzs[i] == clamp(fmaf(ts[i], rays_d, rays_o), -bound, bound) bit for bit; rows no ray owns get 0.  Same arguments and
+ * outputs otherwise (bit-identical); ts may be NULL only when M == 0. */
+int tnl_march_rays_train_ts(const float* rays_o, const float* rays_d, const uint8_t* grid, float bound, float dt_gamma,
+                            uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* nears,
+                            const float* fars, float* xyzs, float* dirs, float* deltas, float* ts, int32_t* rays,
+                            int32_t* counter, const float* noises, void* workspace, size_t workspace_bytes,
+                            tnl_stream_t stream);
+/* Ray gradient of the training march with every sample's t held fixed (xyz = clamp(o + t d), dirs = d):
+ *   g_rays_o[n] = sum_k mask_k g_xyz_k,   g_rays_d[n] = sum_k t_k mask_k g_xyz_k + sum_k g_dirs_k
+ * over the rows k of ray n (rays [N][3] and ts [M] from tnl_march_rays_train_ts), mask_k per component: the march's unclamped
+ * coordinate fmaf(t, d, o) lies in [-bound, bound] (borders included, torch.clamp's backward).  g_xyz / g_dirs [M][3] fp32, either
+ * may be NULL (zero).  Rays with no sample or dropped for overflowing M, and rows >= *n_valid (DEVICE int32, NULL = M), contribute
+ * nothing.  g_rays_o / g_rays_d [N][3] are overwritten.  One warp per ray, fixed summation order: the same bits on every run. */
+int tnl_rays_backward(const int32_t* rays, const float* ts, const float* rays_o, const float* rays_d, float bound,
+                      const float* g_xyz, const float* g_dirs, const int32_t* n_valid, uint32_t N, uint32_t M, float* g_rays_o,
+                      float* g_rays_d, tnl_stream_t stream);
 /* replaces composite_rays_train_forward / _backward (raymarching.h:14-15, raymarching.cu:580-693).
  * backward: grad_sigmas / grad_rgbs may be uninitialised; every row is written (zeros past a ray's termination and in rows no
  * kept ray owns -- what the reference leaves untouched in its zero-initialised outputs, raymarching.py:283-284). */
@@ -378,6 +395,15 @@ int tnl_grid_scatter(const int32_t* indices, const float* sigma, uint32_t n, flo
 int tnl_rays_from_ids(const float* poses, uint32_t B, float fx, float fy, float cx, float cy, uint32_t H, uint32_t W,
                       const int64_t* ray_ids, int64_t first_id, uint32_t n, const float* images, uint32_t image_channels,
                       float* rays_o, float* rays_d, float* targets, tnl_stream_t stream);
+/* Pose gradient of tnl_rays_from_ids (same B, intrinsics, H, W, ray_ids / first_id, n; ids clamped as there):
+ *   g_poses[b][r][c] = sum_{rays t of image b} g_rays_d[t][r] dir_t[c]  (c < 3),   g_poses[b][r][3] = sum g_rays_o[t][r],
+ * bottom row 0; an image without rays gets exactly 0.  dir_t is recomputed with the forward's per-pixel arithmetic.  The
+ * gradient does not depend on the pose values, so the poses are not an argument.  g_rays_o / g_rays_d [n][3] fp32 (either may
+ * be NULL: zero); g_poses [B][4][4] fp32 is overwritten.  One CTA per image scans the batch in a fixed order: no atomics, the
+ * same bits on every run. */
+int tnl_rays_from_ids_backward(const float* g_rays_o, const float* g_rays_d, uint32_t B, float fx, float fy, float cx, float cy,
+                               uint32_t H, uint32_t W, const int64_t* ray_ids, int64_t first_id, uint32_t n, float* g_poses,
+                               tnl_stream_t stream);
 
 /* ------------------------------------------------------------------ multi-GPU gradient exchange ---- */
 /* flags [3][R/T][R/T] (uint8): 1 where a tile of T x T texels can receive plane gradient, i.e. lies under the projection

@@ -34,6 +34,9 @@ SIGNATURES = {
     "tnl_march_rays_train_workspace_fast": (_sz, [_u32, _u32]),
     "tnl_march_rays_train": (_int, [_vp, _vp, _vp, _f32, _f32, _u32, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp,
                                     _vp, _vp, _vp, _vp, _sz, _vp]),
+    "tnl_march_rays_train_ts": (_int, [_vp, _vp, _vp, _f32, _f32, _u32, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp,
+                                       _vp, _vp, _vp, _vp, _sz, _vp]),
+    "tnl_rays_backward": (_int, [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp]),
     "tnl_composite_rays_train_forward": (_int, [_vp, _vp, _vp, _vp, _u32, _u32, _f32, _vp, _vp, _vp, _vp]),
     "tnl_composite_rays_train_backward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u32, _u32, _f32, _vp, _vp, _vp]),
     "tnl_march_rays": (_int, [_u32, _u32, _vp, _vp, _vp, _vp, _f32, _f32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp,
@@ -94,6 +97,7 @@ SIGNATURES = {
     "tnl_grid_scatter": (_int, [_vp, _vp, _u32, _f32, _vp, _vp]),
     "tnl_rays_from_ids": (_int, [_vp, _u32, _f32, _f32, _f32, _f32, _u32, _u32, _vp, ctypes.c_int64, _u32, _vp, _u32, _vp, _vp,
                                  _vp, _vp]),
+    "tnl_rays_from_ids_backward": (_int, [_vp, _vp, _u32, _f32, _f32, _f32, _f32, _u32, _u32, _vp, ctypes.c_int64, _u32, _vp, _vp]),
     "tnl_mc_workspace": (_sz, [_u32, _u32, _u32]),
     "tnl_mc_count": (_int, [_vp, _u32, _u32, _u32, _c.c_double, _vp, _sz, _vp, _vp]),
     "tnl_mc_emit": (_int, [_vp, _u32, _u32, _u32, _c.c_double, _vp, _sz, _c.c_int64, _c.c_int64, _vp, _vp, _vp]),
@@ -177,7 +181,7 @@ def check(rc, what):
 
 
 # number of kernels each ABI call launches (for the launch counter the benchmark reports)
-KERNELS_PER_CALL = {"tnl_march_rays_train": 6, "tnl_sample_planes_backward_det": 4, "tnl_mlp_backward_det": 2, "tnl_composite_rays_train_backward": 2, "tnl_compact_alive": 3, "tnl_compact_alive_dev": 3, "tnl_cell_sort": 5,
+KERNELS_PER_CALL = {"tnl_march_rays_train": 6, "tnl_march_rays_train_ts": 7, "tnl_sample_planes_backward_det": 4, "tnl_mlp_backward_det": 2, "tnl_composite_rays_train_backward": 2, "tnl_compact_alive": 3, "tnl_compact_alive_dev": 3, "tnl_cell_sort": 5,
                     "tnl_mlp_pack_weights": 2, "tnl_mc_count": 2}
 # work-list IDWT calls launch one kernel per requested part (position of the `parts` argument from the end)
 _PARTS_ARG = {"tnl_idwt_level_forward_sparse": -2, "tnl_idwt_level_backward_sparse": -3,

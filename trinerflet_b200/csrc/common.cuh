@@ -34,4 +34,11 @@ __host__ __device__ inline T ceil_div(T a, T b) { return (a + b - 1) / b; }
 
 constexpr int kNumSM = 148;  // B200
 
+// sum over the 32 lanes of a warp by a fixed xor tree: every lane gets the same bits, whatever the schedule
+__device__ __forceinline__ float warp_sum(float v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
 }  // namespace tnl

@@ -239,13 +239,14 @@ __global__ void k_march_train_count(const float* __restrict__ rays_o, const floa
     rays[3 * (size_t)n + 2] = (int32_t)num;
 }
 
-// pass 2: re-march and write the samples into [offset, offset+count)
-__global__ void k_march_train_write(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
-                                    const uint8_t* __restrict__ grid, float bound, float dt_gamma, uint32_t max_steps,
-                                    uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears,
-                                    const float* __restrict__ fars, const float* __restrict__ noises,
-                                    const int32_t* __restrict__ rays, float* __restrict__ xyzs,
-                                    float* __restrict__ dirs, float* __restrict__ deltas) {
+// pass 2: re-march and write the samples into [offset, offset+count).  TS: also write each row's ray parameter t to ts_out.
+template <bool TS>
+__device__ __forceinline__ void march_train_write(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
+                                                  const uint8_t* __restrict__ grid, float bound, float dt_gamma, uint32_t max_steps,
+                                                  uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears,
+                                                  const float* __restrict__ fars, const float* __restrict__ noises,
+                                                  const int32_t* __restrict__ rays, float* __restrict__ xyzs,
+                                                  float* __restrict__ dirs, float* __restrict__ deltas, float* __restrict__ ts_out) {
     const uint32_t n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= N) return;
     const uint32_t offset = (uint32_t)rays[3 * (size_t)n + 1];
@@ -260,12 +261,14 @@ __global__ void k_march_train_write(const float* __restrict__ rays_o, const floa
     float* px = xyzs + 3 * (size_t)offset;
     float* pd = dirs + 3 * (size_t)offset;
     float* pl = deltas + 2 * (size_t)offset;
+    float* pt = TS ? ts_out + offset : nullptr;
     uint32_t step = 0;
     float x, y, z, dt;
     while (t < far && step < num) {
         if (march_probe(p, r, t, x, y, z, dt)) {
             px[0] = x; px[1] = y; px[2] = z;
             pd[0] = r.dx; pd[1] = r.dy; pd[2] = r.dz;
+            if (TS) *pt++ = t;
             t = __fadd_rn(t, dt);
             pl[0] = dt;
             pl[1] = __fsub_rn(t, last_t);
@@ -276,14 +279,35 @@ __global__ void k_march_train_write(const float* __restrict__ rays_o, const floa
     }
 }
 
+__global__ void k_march_train_write(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
+                                    const uint8_t* __restrict__ grid, float bound, float dt_gamma, uint32_t max_steps,
+                                    uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears,
+                                    const float* __restrict__ fars, const float* __restrict__ noises,
+                                    const int32_t* __restrict__ rays, float* __restrict__ xyzs,
+                                    float* __restrict__ dirs, float* __restrict__ deltas) {
+    march_train_write<false>(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N, C, H, M, nears, fars, noises, rays, xyzs, dirs,
+                             deltas, nullptr);
+}
+
+__global__ void k_march_train_write_ts(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
+                                       const uint8_t* __restrict__ grid, float bound, float dt_gamma, uint32_t max_steps,
+                                       uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears,
+                                       const float* __restrict__ fars, const float* __restrict__ noises,
+                                       const int32_t* __restrict__ rays, float* __restrict__ xyzs,
+                                       float* __restrict__ dirs, float* __restrict__ deltas, float* __restrict__ ts_out) {
+    march_train_write<true>(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N, C, H, M, nears, fars, noises, rays, xyzs, dirs,
+                            deltas, ts_out);
+}
+
 // pass 2 without a second traversal: pass 1 recorded the parameter t of every sample (ts[n][k]); one warp per ray turns them into
 // positions / directions / deltas with the very operations of the traversal (same roundings => bit-identical rows) and writes
-// the ray's rows coalesced.  The occupancy grid is not touched again.
-__global__ void __launch_bounds__(256)
-k_march_train_emit(const float* __restrict__ rays_o, const float* __restrict__ rays_d, float bound, float dt_gamma, uint32_t max_steps,
-                   uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears, const float* __restrict__ noises,
-                   const int32_t* __restrict__ rays, const float* __restrict__ ts, float* __restrict__ xyzs, float* __restrict__ dirs,
-                   float* __restrict__ deltas) {
+// the ray's rows coalesced.  The occupancy grid is not touched again.  TS: also write each row's t to ts_out.
+template <bool TS>
+__device__ __forceinline__ void march_train_emit(const float* __restrict__ rays_o, const float* __restrict__ rays_d, float bound,
+                                                 float dt_gamma, uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M,
+                                                 const float* __restrict__ nears, const float* __restrict__ noises,
+                                                 const int32_t* __restrict__ rays, const float* __restrict__ ts, float* __restrict__ xyzs,
+                                                 float* __restrict__ dirs, float* __restrict__ deltas, float* __restrict__ ts_out) {
     const uint32_t n = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = threadIdx.x & 31;
     if (n >= N) return;
@@ -310,7 +334,24 @@ k_march_train_emit(const float* __restrict__ rays_o, const float* __restrict__ r
         dirs[3 * i] = r.dx; dirs[3 * i + 1] = r.dy; dirs[3 * i + 2] = r.dz;
         deltas[2 * i] = dt;
         deltas[2 * i + 1] = __fsub_rn(__fadd_rn(t, dt), last_t);
+        if (TS) ts_out[i] = t;
     }
+}
+
+__global__ void __launch_bounds__(256)
+k_march_train_emit(const float* __restrict__ rays_o, const float* __restrict__ rays_d, float bound, float dt_gamma, uint32_t max_steps,
+                   uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears, const float* __restrict__ noises,
+                   const int32_t* __restrict__ rays, const float* __restrict__ ts, float* __restrict__ xyzs, float* __restrict__ dirs,
+                   float* __restrict__ deltas) {
+    march_train_emit<false>(rays_o, rays_d, bound, dt_gamma, max_steps, N, C, H, M, nears, noises, rays, ts, xyzs, dirs, deltas, nullptr);
+}
+
+__global__ void __launch_bounds__(256)
+k_march_train_emit_ts(const float* __restrict__ rays_o, const float* __restrict__ rays_d, float bound, float dt_gamma,
+                      uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* __restrict__ nears,
+                      const float* __restrict__ noises, const int32_t* __restrict__ rays, const float* __restrict__ ts,
+                      float* __restrict__ xyzs, float* __restrict__ dirs, float* __restrict__ deltas, float* __restrict__ ts_out) {
+    march_train_emit<true>(rays_o, rays_d, bound, dt_gamma, max_steps, N, C, H, M, nears, noises, rays, ts, xyzs, dirs, deltas, ts_out);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -426,11 +467,6 @@ __device__ __forceinline__ float warp_scan_add(float v, int lane) {
         const float u = __shfl_up_sync(0xffffffffu, v, o);
         if (lane >= o) v += u;
     }
-    return v;
-}
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 
@@ -757,6 +793,67 @@ __global__ void k_compact_scatter_dev(const int32_t* __restrict__ ctrl, const in
 }
 
 // ------------------------------------------------------------------------------------------------
+// ray gradient of the training march (tnl_rays_backward): with every sample's t held fixed, xyz_k = clamp(o + t_k d) and
+// dirs_k = d, so  g_o = sum_k mask_k g_xyz_k  and  g_d = sum_k t_k mask_k g_xyz_k + sum_k g_dirs_k  (mask: o + t_k d inside
+// [-bound, bound] per component, borders included, as torch.clamp's backward).  One warp per ray: lane l adds the rows
+// l, l + 32, ... in that order, then a fixed xor tree sums the lanes -- no atomics, the same bits on every run.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+k_rays_backward(const int32_t* __restrict__ rays, const float* __restrict__ ts, const float* __restrict__ rays_o,
+                const float* __restrict__ rays_d, float bound, const float* __restrict__ g_xyz, const float* __restrict__ g_dirs,
+                const int32_t* __restrict__ n_valid, uint32_t N, uint32_t M, float* __restrict__ g_rays_o,
+                float* __restrict__ g_rays_d) {
+    const uint32_t n = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint32_t lane = threadIdx.x & 31;
+    if (n >= N) return;
+    const uint32_t index = (uint32_t)rays[3 * (size_t)n];
+    const uint32_t offset = (uint32_t)rays[3 * (size_t)n + 1];
+    const uint32_t num = (uint32_t)rays[3 * (size_t)n + 2];
+    float go[3] = {0.f, 0.f, 0.f}, gd[3] = {0.f, 0.f, 0.f};
+    if (num != 0 && offset + num <= M) {   // dropped rays (overflowing M) contribute nothing
+        uint32_t end = offset + num;
+        if (n_valid) {
+            const int32_t nv = *n_valid;
+            const uint32_t v = nv < 0 ? 0u : (uint32_t)nv;
+            end = end < v ? end : v;
+        }
+        const float o[3] = {rays_o[3 * (size_t)n], rays_o[3 * (size_t)n + 1], rays_o[3 * (size_t)n + 2]};
+        const float d[3] = {rays_d[3 * (size_t)n], rays_d[3 * (size_t)n + 1], rays_d[3 * (size_t)n + 2]};
+        for (uint32_t i = offset + lane; i < end; i += 32) {
+            // all loads first, independent of the mask: one memory round trip per iteration instead of two dependent ones
+            const float t = __ldg(ts + i);
+            float gx[3], gv[3];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                gx[a] = g_xyz ? __ldg(g_xyz + 3 * (size_t)i + a) : 0.f;
+                gv[a] = g_dirs ? __ldg(g_dirs + 3 * (size_t)i + a) : 0.f;
+            }
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const float u = __fmaf_rn(t, d[a], o[a]);          // the march's own unclamped coordinate
+                if (g_xyz && u >= -bound && u <= bound) {
+                    go[a] = __fadd_rn(go[a], gx[a]);
+                    gd[a] = __fmaf_rn(t, gx[a], gd[a]);
+                }
+                if (g_dirs) gd[a] = __fadd_rn(gd[a], gv[a]);
+            }
+        }
+    }
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        go[a] = warp_sum(go[a]);
+        gd[a] = warp_sum(gd[a]);
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            g_rays_o[3 * (size_t)index + a] = go[a];
+            g_rays_d[3 * (size_t)index + a] = gd[a];
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // SH basis, degree <= 4 (shencoder.cu:50-68)
 // ------------------------------------------------------------------------------------------------
 __global__ void k_sh_encode(const float* __restrict__ inputs, float* __restrict__ outputs, uint32_t B, uint32_t degree) {
@@ -857,18 +954,11 @@ size_t tnl_march_rays_train_workspace_fast(uint32_t N, uint32_t max_steps) {
     return march_scan_bytes(N) + sizeof(float) * (size_t)N * max_steps;
 }
 
-int tnl_march_rays_train(const float* rays_o, const float* rays_d, const uint8_t* grid, float bound, float dt_gamma,
-                         uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* nears,
-                         const float* fars, float* xyzs, float* dirs, float* deltas, int32_t* rays, int32_t* counter,
-                         const float* noises, void* workspace, size_t workspace_bytes, tnl_stream_t stream) {
-    if (N == 0) return 0;
-    TNL_ARG_CHECK(rays_o && rays_d && grid && nears && fars && rays && counter && noises, "null pointer");
-    TNL_ARG_CHECK(M == 0 || (xyzs && dirs && deltas), "null output");
-    TNL_ARG_CHECK(C >= 1 && C <= 8 && H >= 2 && H <= 1024 && max_steps >= 1, "unsupported cascade / grid size");
-    if (workspace == nullptr || workspace_bytes < tnl_march_rays_train_workspace(N)) {
-        set_error("march_rays_train: workspace too small");
-        return TNL_ERR_WORKSPACE;
-    }
+// ts_out == nullptr: tnl_march_rays_train; else also the ray parameter of every row (tnl_march_rays_train_ts)
+static int march_rays_train(const float* rays_o, const float* rays_d, const uint8_t* grid, float bound, float dt_gamma,
+                            uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* nears,
+                            const float* fars, float* xyzs, float* dirs, float* deltas, int32_t* rays, int32_t* counter,
+                            const float* noises, void* workspace, size_t workspace_bytes, float* ts_out, tnl_stream_t stream) {
     uint32_t* block_sums = static_cast<uint32_t*>(workspace);
     const uint32_t nb = ceil_div(N, (uint32_t)kScanThreads);
     const bool fast = M > 0 && workspace_bytes >= tnl_march_rays_train_workspace_fast(N, max_steps);
@@ -879,16 +969,65 @@ int tnl_march_rays_train(const float* rays_o, const float* rays_d, const uint8_t
     k_scan_of_sums<<<1, kScanThreads, 0, S(stream)>>>(block_sums, nb, counter, N, nullptr);
     k_scan_offsets<<<nb, kScanThreads, 0, S(stream)>>>(rays + 2, N, 3, block_sums, rays + 1);
     if (M > 0) {
-        if (fast)
+        if (fast && ts_out)
+            k_march_train_emit_ts<<<ceil_div(N, 8u), 256, 0, S(stream)>>>(rays_o, rays_d, bound, dt_gamma, max_steps, N, C, H, M, nears,
+                                                                          noises, rays, ts, xyzs, dirs, deltas, ts_out);
+        else if (fast)
             k_march_train_emit<<<ceil_div(N, 8u), 256, 0, S(stream)>>>(rays_o, rays_d, bound, dt_gamma, max_steps, N, C, H, M, nears, noises,
                                                                        rays, ts, xyzs, dirs, deltas);
+        else if (ts_out)
+            k_march_train_write_ts<<<ceil_div(N, kT), kT, 0, S(stream)>>>(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N, C, H, M,
+                                                                           nears, fars, noises, rays, xyzs, dirs, deltas, ts_out);
         else
             k_march_train_write<<<ceil_div(N, kT), kT, 0, S(stream)>>>(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N,
                                                                         C, H, M, nears, fars, noises, rays, xyzs, dirs, deltas);
         // rows no kept ray owns are zeros, as in the reference's zero-initialised buffers: the caller may pass uninitialised memory
         k_zero_unowned_rows<<<32, 256, 0, S(stream)>>>(rays, N, M, xyzs, 3, dirs, 3, deltas, 2);
+        if (ts_out) k_zero_unowned_rows<<<32, 256, 0, S(stream)>>>(rays, N, M, ts_out, 1, nullptr, 0, nullptr, 0);
     }
-    return finish_launch("march_rays_train");
+    return finish_launch(ts_out ? "march_rays_train_ts" : "march_rays_train");
+}
+
+#define TNL_MARCH_TRAIN_CHECKS(what)                                                                                            \
+    TNL_ARG_CHECK(rays_o && rays_d && grid && nears && fars && rays && counter && noises, "null pointer");                     \
+    TNL_ARG_CHECK(M == 0 || (xyzs && dirs && deltas), "null output");                                                          \
+    TNL_ARG_CHECK(C >= 1 && C <= 8 && H >= 2 && H <= 1024 && max_steps >= 1, "unsupported cascade / grid size");              \
+    if (workspace == nullptr || workspace_bytes < tnl_march_rays_train_workspace(N)) {                                          \
+        set_error(what ": workspace too small");                                                                                \
+        return TNL_ERR_WORKSPACE;                                                                                               \
+    }
+
+int tnl_march_rays_train(const float* rays_o, const float* rays_d, const uint8_t* grid, float bound, float dt_gamma,
+                         uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* nears,
+                         const float* fars, float* xyzs, float* dirs, float* deltas, int32_t* rays, int32_t* counter,
+                         const float* noises, void* workspace, size_t workspace_bytes, tnl_stream_t stream) {
+    if (N == 0) return 0;
+    TNL_MARCH_TRAIN_CHECKS("march_rays_train");
+    return march_rays_train(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N, C, H, M, nears, fars, xyzs, dirs, deltas, rays,
+                            counter, noises, workspace, workspace_bytes, nullptr, stream);
+}
+
+int tnl_march_rays_train_ts(const float* rays_o, const float* rays_d, const uint8_t* grid, float bound, float dt_gamma,
+                            uint32_t max_steps, uint32_t N, uint32_t C, uint32_t H, uint32_t M, const float* nears,
+                            const float* fars, float* xyzs, float* dirs, float* deltas, float* ts, int32_t* rays,
+                            int32_t* counter, const float* noises, void* workspace, size_t workspace_bytes, tnl_stream_t stream) {
+    if (N == 0) return 0;
+    TNL_MARCH_TRAIN_CHECKS("march_rays_train_ts");
+    TNL_ARG_CHECK(M == 0 || ts, "null output");
+    return march_rays_train(rays_o, rays_d, grid, bound, dt_gamma, max_steps, N, C, H, M, nears, fars, xyzs, dirs, deltas, rays,
+                            counter, noises, workspace, workspace_bytes, M > 0 ? ts : nullptr, stream);
+}
+
+int tnl_rays_backward(const int32_t* rays, const float* ts, const float* rays_o, const float* rays_d, float bound,
+                      const float* g_xyz, const float* g_dirs, const int32_t* n_valid, uint32_t N, uint32_t M, float* g_rays_o,
+                      float* g_rays_d, tnl_stream_t stream) {
+    if (N == 0) return 0;
+    TNL_ARG_CHECK(rays && rays_o && rays_d && g_rays_o && g_rays_d, "null pointer");
+    TNL_ARG_CHECK(M == 0 || ts, "null ts");
+    TNL_ARG_CHECK(bound > 0.f, "bound must be positive");
+    k_rays_backward<<<ceil_div(N, 8u), 256, 0, S(stream)>>>(rays, ts, rays_o, rays_d, bound, M ? g_xyz : nullptr,
+                                                             M ? g_dirs : nullptr, n_valid, N, M, g_rays_o, g_rays_d);
+    return finish_launch("rays_backward");
 }
 
 int tnl_composite_rays_train_forward(const float* sigmas, const float* rgbs, const float* deltas, const int32_t* rays,

@@ -41,6 +41,60 @@ __global__ void k_rays_from_ids(const float* __restrict__ poses, RayIntrinsics k
     }
 }
 
+
+// Pose gradient of k_rays_from_ids (rays_d = R dir(pix), rays_o = pose[:3,3]): one CTA per image b scans the batch in a fixed
+// order -- thread j takes the rays j, j + 256, ... (the whole batch for explicit ids, only the image's range for the implicit
+// ones) -- and adds g_d[r] dir[c] into g_pose[b][r][c] and g_o[r] into g_pose[b][r][3]; a fixed shuffle tree and a warp-ordered
+// sum finish the block.  No atomics: the same bits on every run.  The bottom row is 0; an image without rays gets 0.
+constexpr int kPoseThreads = 256;
+
+__global__ void __launch_bounds__(kPoseThreads)
+k_rays_from_ids_backward(const float* __restrict__ g_rays_o, const float* __restrict__ g_rays_d, RayIntrinsics k, uint32_t HW,
+                         uint32_t W, const int64_t* __restrict__ ids, int64_t first_id, int64_t n_total, uint32_t n,
+                         float* __restrict__ g_poses) {
+    __shared__ float part[kPoseThreads / 32][12];
+    const uint32_t b = blockIdx.x;
+    const int64_t lo = (int64_t)b * HW, hi = lo + HW;
+    uint32_t t0 = 0, t1 = n;
+    if (!ids) {     // id = first_id + t, in range (checked on the host): the image's rays are one contiguous slice
+        const int64_t a = lo - first_id, e = hi - first_id;
+        t0 = (uint32_t)(a < 0 ? 0 : (a > (int64_t)n ? (int64_t)n : a));
+        t1 = (uint32_t)(e < 0 ? 0 : (e > (int64_t)n ? (int64_t)n : e));
+    }
+    float acc[12];
+#pragma unroll
+    for (int q = 0; q < 12; ++q) acc[q] = 0.f;
+    for (uint32_t t = t0 + threadIdx.x; t < t1; t += kPoseThreads) {
+        int64_t id = ids ? __ldg(ids + t) : first_id + (int64_t)t;
+        id = id < 0 ? 0 : (id >= n_total ? n_total - 1 : id);   // the forward's clamp
+        if (id < lo || id >= hi) continue;
+        float dir[3];
+        pixel_direction(k, W, (uint32_t)(id - lo), dir);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            const float gd = g_rays_d ? __ldg(g_rays_d + 3 * (size_t)t + r) : 0.f;
+            const float go = g_rays_o ? __ldg(g_rays_o + 3 * (size_t)t + r) : 0.f;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) acc[4 * r + c] = __fmaf_rn(gd, dir[c], acc[4 * r + c]);
+            acc[4 * r + 3] = __fadd_rn(acc[4 * r + 3], go);
+        }
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int q = 0; q < 12; ++q) {
+        const float v = warp_sum(acc[q]);
+        if (lane == 0) part[warp][q] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < 16) {
+        const int q = threadIdx.x;
+        float v = 0.f;
+        if (q < 12)
+            for (int w = 0; w < kPoseThreads / 32; ++w) v = __fadd_rn(v, part[w][q]);
+        g_poses[16 * (size_t)b + q] = v;
+    }
+}
+
 }  // namespace tnl
 
 using namespace tnl;
@@ -71,6 +125,20 @@ int tnl_rays_from_ids(const float* poses, uint32_t B, float fx, float fy, float 
     else
         k_rays_from_ids<4><<<grid, block, 0, s>>>(poses, k, HW, W, ray_ids, first_id, n_total, n, images, rays_o, rays_d, targets);
     return finish_launch("rays_from_ids");
+}
+
+int tnl_rays_from_ids_backward(const float* g_rays_o, const float* g_rays_d, uint32_t B, float fx, float fy, float cx, float cy, uint32_t H, uint32_t W, const int64_t* ray_ids, int64_t first_id, uint32_t n,
+                               float* g_poses, tnl_stream_t stream) {
+    TNL_ARG_CHECK(g_poses, "null pointer");
+    TNL_ARG_CHECK(B >= 1 && H >= 1 && W >= 1 && (uint64_t)H * W <= 0x7fffffffull, "bad image geometry");
+    TNL_ARG_CHECK(fx != 0.f && fy != 0.f, "zero focal length");
+    const uint32_t HW = H * W;
+    const int64_t n_total = (int64_t)B * HW;
+    TNL_ARG_CHECK(ray_ids || (first_id >= 0 && first_id + (int64_t)n <= n_total), "implicit id range outside the ray table");
+    const RayIntrinsics k{fx, fy, cx, cy};
+    k_rays_from_ids_backward<<<B, kPoseThreads, 0, reinterpret_cast<cudaStream_t>(stream)>>>(g_rays_o, g_rays_d, k, HW, W, ray_ids,
+                                                                                              first_id, n_total, n, g_poses);
+    return finish_launch("rays_from_ids_backward");
 }
 
 }  // extern "C"

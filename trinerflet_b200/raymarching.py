@@ -39,6 +39,8 @@ class _near_far_from_aabb(Function):
         fars = torch.empty(N, dtype=rays_o.dtype, device=rays_o.device)
         call("tnl_near_far_from_aabb", ptr(rays_o), ptr(rays_d), ptr(aabb), N, float(min_near), ptr(nears), ptr(fars),
              stream())
+        # piecewise-constant in the rays through the box faces' min / max: no ray gradient flows through nears / fars
+        ctx.mark_non_differentiable(nears, fars)
         return nears, fars
 
 
@@ -118,8 +120,10 @@ class _march_rays_train(Function):
     @staticmethod
     @_fwd32
     def forward(ctx, rays_o, rays_d, bound, density_bitfield, C, H, nears, fars, step_counter=None, mean_count=-1,
-                perturb=False, align=-1, force_all_rays=False, dt_gamma=0, max_steps=1024):
-        """raymarching.py:164-233. Returns xyzs [M,3], dirs [M,3], deltas [M,2], rays [N,3]."""
+                perturb=False, align=-1, force_all_rays=False, dt_gamma=0, max_steps=1024, ray_grad=False):
+        """raymarching.py:164-233. Returns xyzs [M,3], dirs [M,3], deltas [M,2], rays [N,3].
+        ray_grad (set by march_rays_train): record each row's t for the ray backward."""
+        shapes = (rays_o.shape, rays_d.shape)
         rays_o = _cuda_f32(rays_o).view(-1, 3)
         rays_d = _cuda_f32(rays_d).view(-1, 3)
         if not density_bitfield.is_cuda:
@@ -145,7 +149,16 @@ class _march_rays_train(Function):
         need = lib.tnl_march_rays_train_workspace_fast(N, int(max_steps))
         ws = _workspace(need if need <= (1 << 30) else lib.tnl_march_rays_train_workspace(N), dev)
 
+        ts = None
+
         def run(M_, xyzs, dirs, deltas):
+            nonlocal ts
+            if ray_grad:    # the same march, plus the ray parameter of every row for the backward
+                ts = torch.empty(M_, dtype=torch.float32, device=dev) if M_ > 0 else None
+                call("tnl_march_rays_train_ts", ptr(rays_o), ptr(rays_d), ptr(density_bitfield), float(bound), float(dt_gamma),
+                     int(max_steps), N, int(C), int(H), int(M_), ptr(nears), ptr(fars), ptr(xyzs), ptr(dirs), ptr(deltas),
+                     ptr(ts), ptr(rays), ptr(step_counter), ptr(noises), ptr(ws), ws.numel(), stream())
+                return
             call("tnl_march_rays_train", ptr(rays_o), ptr(rays_d), ptr(density_bitfield), float(bound), float(dt_gamma),
                  int(max_steps), N, int(C), int(H), int(M_), ptr(nears), ptr(fars), ptr(xyzs), ptr(dirs), ptr(deltas),
                  ptr(rays), ptr(step_counter), ptr(noises), ptr(ws), ws.numel(), stream())
@@ -172,10 +185,38 @@ class _march_rays_train(Function):
             dirs = torch.empty(M, 3, dtype=rays_o.dtype, device=dev)
             deltas = torch.empty(M, 2, dtype=rays_o.dtype, device=dev)
             run(M, xyzs, dirs, deltas)
+        if ray_grad:
+            ctx.mark_non_differentiable(deltas, rays)
+            ctx.save_for_backward(rays, ts, rays_o, rays_d)
+            ctx.meta = (float(bound), shapes)
         return xyzs, dirs, deltas, rays
 
+    @staticmethod
+    @_bwd
+    def backward(ctx, grad_xyzs, grad_dirs, grad_deltas, grad_rays):
+        rays, ts, rays_o, rays_d = ctx.saved_tensors
+        bound, (shape_o, shape_d) = ctx.meta
+        N, M = rays.shape[0], (ts.shape[0] if ts is not None else 0)
+        g_xyz = grad_xyzs.contiguous().float() if grad_xyzs is not None else None
+        g_dirs = grad_dirs.contiguous().float() if grad_dirs is not None else None
+        g_o = torch.empty_like(rays_o)
+        g_d = torch.empty_like(rays_d)
+        # (rows no ray owns are never read, so the rows past the sample count need no n_valid here)
+        call("tnl_rays_backward", ptr(rays), ptr(ts), ptr(rays_o), ptr(rays_d), bound, ptr(g_xyz), ptr(g_dirs), None, N, M,
+             ptr(g_o), ptr(g_d), stream())
+        return (g_o.view(shape_o) if ctx.needs_input_grad[0] else None, g_d.view(shape_d) if ctx.needs_input_grad[1] else None,
+                *([None] * 14))
 
-march_rays_train = _march_rays_train.apply
+
+def march_rays_train(rays_o, rays_d, bound, density_bitfield, C, H, nears, fars, step_counter=None, mean_count=-1,
+                     perturb=False, align=-1, force_all_rays=False, dt_gamma=0, max_steps=1024):
+    """raymarching.py:164-233 (same positional signature).  When rays_o or rays_d requires grad and grad mode is on, xyzs and
+    dirs are differentiable in the rays with every sample's ray parameter t held fixed: xyz = clamp(o + t d, -bound, bound),
+    dirs = d (tnl_rays_backward); deltas and rays are not.  Otherwise the call and its outputs are exactly those of the plain
+    march.  (Grad mode is read here: inside Function.forward it is always off.)"""
+    ray_grad = torch.is_grad_enabled() and (rays_o.requires_grad or rays_d.requires_grad)
+    return _march_rays_train.apply(rays_o, rays_d, bound, density_bitfield, C, H, nears, fars, step_counter, mean_count, perturb,
+                                   align, force_all_rays, dt_gamma, max_steps, ray_grad)
 
 
 class _composite_rays_train(Function):

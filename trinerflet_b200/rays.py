@@ -29,7 +29,9 @@ def rays_from_ids(poses, intrinsics, H, W, ray_ids=None, first_id=0, n=None, ima
     """poses [B,4,4] fp32 CUDA; ray_ids int64 [n] flat ids into the [B*H*W] table (or None: first_id .. first_id+n-1);
     images [B,H*W,C] / [B,H,W,C] fp32 (optional) -> rays_o [n,3], rays_d [n,3] (, targets [n,C]).
     out = (rays_o, rays_d[, targets]): write into these contiguous fp32 buffers (e.g. the static inputs of a captured
-    CUDA graph) instead of allocating."""
+    CUDA graph) instead of allocating.
+    When the poses require grad (and grad mode is on), rays_o / rays_d are differentiable in them
+    (tnl_rays_from_ids_backward); the targets never are."""
     poses = poses.contiguous().float()
     B = poses.shape[0]
     fx, fy, cx, cy = _intr(intrinsics)
@@ -38,25 +40,65 @@ def rays_from_ids(poses, intrinsics, H, W, ray_ids=None, first_id=0, n=None, ima
         if ray_ids.dtype != torch.int64:
             ray_ids = ray_ids.long()
         n = ray_ids.numel()
+    pose_grad = poses.requires_grad and torch.is_grad_enabled()
     if out is not None:
+        if pose_grad:
+            raise RuntimeError("rays_from_ids: `out` buffers cannot carry a pose gradient (the poses require grad)")
         for t, width in zip(out, (3, 3, images.shape[-1] if images is not None else 0)):
             if t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != n * width:
                 raise RuntimeError("rays_from_ids: `out` buffers must be contiguous fp32 with n rows")
+    if images is not None:
+        if images.dtype != torch.float32 or not images.is_contiguous():
+            raise RuntimeError("rays_from_ids: images must be a contiguous fp32 tensor [B,H*W,C] or [B,H,W,C]")
+        if images.numel() != B * H * W * images.shape[-1]:
+            raise RuntimeError("rays_from_ids: images do not match B*H*W")
+    geom = (B, fx, fy, cx, cy, int(H), int(W), int(first_id), int(n))
+    if pose_grad:
+        return _PoseRays.apply(poses, ray_ids, images, geom)
+    return _rays_from_ids(poses.detach(), ray_ids, images, geom, out)
+
+
+def _rays_from_ids(poses, ray_ids, images, geom, out=None):
+    B, fx, fy, cx, cy, H, W, first_id, n = geom
+    if out is not None:
         rays_o, rays_d = out[0], out[1]
     else:
         rays_o = torch.empty(n, 3, device=poses.device, dtype=torch.float32)
         rays_d = torch.empty(n, 3, device=poses.device, dtype=torch.float32)
     targets, ci = None, 0
     if images is not None:
-        if images.dtype != torch.float32 or not images.is_contiguous():
-            raise RuntimeError("rays_from_ids: images must be a contiguous fp32 tensor [B,H*W,C] or [B,H,W,C]")
         ci = images.shape[-1]
-        if images.numel() != B * H * W * ci:
-            raise RuntimeError("rays_from_ids: images do not match B*H*W")
         targets = out[2] if out is not None else torch.empty(n, ci, device=poses.device, dtype=torch.float32)
-    _lib.call("tnl_rays_from_ids", _lib.ptr(poses), B, fx, fy, cx, cy, H, W, _lib.ptr(ray_ids), int(first_id), n,
+    _lib.call("tnl_rays_from_ids", _lib.ptr(poses), B, fx, fy, cx, cy, H, W, _lib.ptr(ray_ids), first_id, n,
               _lib.ptr(images), ci, _lib.ptr(rays_o), _lib.ptr(rays_d), _lib.ptr(targets), _lib.stream())
     return (rays_o, rays_d) if images is None else (rays_o, rays_d, targets)
+
+
+class _PoseRays(torch.autograd.Function):
+    """rays_from_ids as a function of the poses: rays_d = R dir(pix), rays_o = pose[:3,3], so
+    g_pose[b][r][c] = sum over the rays of image b of g_d[r] dir[c] (c < 3), g_pose[b][r][3] = sum g_o[r], bottom row 0."""
+
+    @staticmethod
+    def forward(ctx, poses, ray_ids, images, geom):
+        res = _rays_from_ids(poses, ray_ids, images, geom)
+        if images is not None:
+            ctx.mark_non_differentiable(res[2])
+        ctx.save_for_backward(ray_ids)
+        ctx.geom = geom
+        return res
+
+    @staticmethod
+    def backward(ctx, g_o, *rest):
+        g_d = rest[0]
+        (ray_ids,) = ctx.saved_tensors
+        B, fx, fy, cx, cy, H, W, first_id, n = ctx.geom
+        g_o = g_o.contiguous().float() if g_o is not None else None
+        g_d = g_d.contiguous().float() if g_d is not None else None
+        dev = (g_o if g_o is not None else g_d).device
+        g_poses = torch.empty(B, 4, 4, device=dev, dtype=torch.float32)
+        _lib.call("tnl_rays_from_ids_backward", _lib.ptr(g_o), _lib.ptr(g_d), B, fx, fy, cx, cy, H, W, _lib.ptr(ray_ids),
+                  first_id, n, _lib.ptr(g_poses), _lib.stream())
+        return g_poses, None, None, None
 
 
 @torch.amp.autocast("cuda", enabled=False)
@@ -152,9 +194,14 @@ class RayFeeder:
             ids = ids[lo:hi]
         return ids
 
-    def select_batch(self, batch_idx, batch_size, out=None):
+    def select_batch(self, batch_idx, batch_size, out=None, poses=None):
+        """poses: [B,4,4] to draw the rays from instead of the feeder's own (e.g. poses.CameraPoses()(): refined poses that
+        require grad, so the batch's rays carry the pose gradient; the targets do not)"""
         ids = self.batch_ids(batch_idx, batch_size)
-        out = rays_from_ids(self.poses, self.intrinsics, self.H, self.W, ray_ids=ids, images=self.images, out=out)
+        if poses is not None and tuple(poses.shape) != (self.B, 4, 4):
+            raise RuntimeError(f"select_batch: poses must be [{self.B},4,4], got {list(poses.shape)}")
+        out = rays_from_ids(self.poses if poses is None else poses, self.intrinsics, self.H, self.W, ray_ids=ids,
+                            images=self.images, out=out)
         res = {'rays_o': out[0].unsqueeze(0), 'rays_d': out[1].unsqueeze(0)}
         if self.images is not None:
             res['images'] = out[2].unsqueeze(0)

@@ -99,7 +99,12 @@ class TrainStep:
             return self.criterion(pred, images).mean(-1).mean()
 
     def forward_backward(self, rays_o, rays_d, images, update_grid=None):
-        """rays_o/rays_d/images: [N,3] device tensors (this rank's shard). Returns the detached loss tensor."""
+        """rays_o/rays_d/images: [N,3] device tensors (this rank's shard). Returns the detached loss tensor.
+        Rays that require grad (e.g. drawn from poses.CameraPoses through RayFeeder.select_batch(poses=...)) pass their
+        gradient on: the backward of this step also fills the .grad of whatever the rays were computed from."""
+        if self.world_size > 1 and (rays_o.requires_grad or rays_d.requires_grad):
+            raise RuntimeError("TrainStep: rays that require grad (camera pose refinement) are supported on one GPU only: "
+                               "the multi-GPU step does not reduce the pose gradient across ranks")
         model, opt = self.model, self.opt
         enc = model.encoder
         model.train()
@@ -362,6 +367,9 @@ class TrainStep:
         Inputs are copied into static buffers before each replay; parameter gradients live in the graph's memory pool
         and are overwritten by every replay (equivalent to zero_grad(set_to_none=True) + backward).  The step counter
         ring slot is the one current at capture time."""
+        if rays_o.requires_grad or rays_d.requires_grad:
+            raise RuntimeError("TrainStep.capture: rays that require grad (camera pose refinement) cannot be captured: the "
+                               "graph's static inputs are plain buffers; run the step eagerly with forward_backward()")
         assert self.model.mean_count > 0, "capture needs the steady state (mean_count > 0): run a few eager steps first"
         self._static = tuple(t.clone() for t in (rays_o, rays_d, images))
         if self.reducer is not None:
